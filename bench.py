@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- 1080p warped frames/s of the pixel-wise warp hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--min-seconds S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
-One "step" = `inner_repeat` passes of the hot path over one resident batch of synthetic frames; a pass = forward warp +
-backward warp (gradients to BOTH the frame and the map) of FRAMES 1080p fp32 RGB frames per GPU, through the C ABI of
-libpwswarp.so.  `inner_repeat` is chosen after the warm-up so that the K timed steps last at least --min-seconds
-(default 1 s: the clocks and the power state are then the sustained ones, not those of a 13 ms burst); it is reported.
+One "step" = one pass of the hot path over one resident batch of synthetic frames: forward warp + backward warp
+(gradients to BOTH the frame and the map) of FRAMES 1080p fp32 RGB frames per GPU, through the C ABI of libpwswarp.so.
+The timed region is exactly K steps.  For the sustained clocks and power state rather than those of a short burst, give
+a K for which the region (`timed_region_s`) lasts a second or more.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0): output, grad_input and grad_grid as
+DIR/<name>.npy, float32, each a sample of DUMP_ELEMS elements at flat indices drawn by torch.randint with a fixed seed.
+The inputs depend only on the seeds, so two builds can be compared output for output.
 
   value        frames/s, whole job, inputs resident in HBM (inputs are 0.9 GB per GPU,
                larger than the 126 MB L2, so every pass streams from DRAM)
@@ -37,6 +41,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -45,6 +50,7 @@ import torch
 
 H, W, C = 1080, 1920, 3
 FRAMES = 16                      # frames per GPU per step
+DUMP_ELEMS = 1 << 22             # per dumped array: 3 x 16 MiB of float32
 FWD_BYTES_PX, BWD_BYTES_PX = 32, 52   # algorithmic bytes per output pixel, fp32 C=3 (DESIGN.md section 4)
 WORKLOAD = ("1080p (1920x1080) fp32 RGB bilinear warp, forward + backward (grad to frame and map), "
             f"{FRAMES} frames/GPU/pass, zeros padding, align_corners=False, NCHW frames, planar-stored map "
@@ -73,6 +79,16 @@ def make_inputs(n_frames, seed, device):
     if device is not None:
         frames, gout, planar = frames.to(device), gout.to(device), planar.to(device)
     return frames, planar.permute(0, 2, 3, 1), gout       # map view: strides (2HW, W, 1, HW)
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy: float32 values of each array (in its logical index order) at DUMP_ELEMS flat indices drawn with a
+    fixed seed, so the same arguments always sample the same elements."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.detach().reshape(-1)
+        idx = torch.randint(flat.numel(), (min(DUMP_ELEMS, flat.numel()),), generator=torch.Generator().manual_seed(0))
+        np.save(os.path.join(path, name + ".npy"), flat[idx.to(flat.device)].float().cpu().numpy())
 
 
 class ClockSampler:
@@ -236,12 +252,15 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="lower bound of the device-timed region")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--config", default="headline", choices=["headline", "train", "clip"],
                     help="headline: the BASELINE metric (default); train: BASELINE config 3 (netG training step, DDP); "
                          "clip: BASELINE config 4 (300-frame 1080p clip inference, frame-sharded)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the last timed step's output, grad_input and grad_grid to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.config != "headline" or args.impl != "ours"):
+        ap.error("--dump-outputs records the headline workload of --impl ours")
     if args.config != "headline":
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         if args.config == "train":
@@ -285,22 +304,10 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    # ---------------- warm-up (same allocation pattern as the timed loop) + calibration of the inner repeat
+    # ---------------- warm-up (same allocation pattern as the timed loop)
     for _ in range(warmup):
         out, gin, ggrid = one_pass()
     barrier()
-    c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    c0.record()
-    for _ in range(10):
-        out, gin, ggrid = one_pass()
-    c1.record()
-    torch.cuda.synchronize()
-    pass_ms = c0.elapsed_time(c1) / 10
-    inner = max(1, int(np.ceil(args.min_seconds * 1e3 / (steps * pass_ms))))
-    if world > 1:   # every rank runs the same number of passes
-        t = torch.tensor([inner], device=dev, dtype=torch.int64)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        inner = int(t.item())
 
     # ---------------- a burst, for comparison with round 1's 13 ms measurement: 20 passes after the GPU has idled
     time.sleep(0.5)
@@ -321,14 +328,13 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     time.sleep(0.25)
-    n_pass = steps * inner
-    ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(n_pass)]
+    ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(steps)]
     l0 = _lib.launch_count()
     barrier()
     t_wall0 = time.time()
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     start.record()
-    for k in range(n_pass):
+    for k in range(steps):
         ev[k][0].record()
         out = pw.warp2d_forward(frames, grid, 0, False)
         ev[k][1].record()
@@ -343,6 +349,8 @@ def main():
     fwd_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in ev]))
     bwd_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in ev]))
     del ev
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"output": out, "grad_input": gin, "grad_grid": ggrid})
 
     # ---------------- what the reference executes on a GPU box: ATen's CUDA kernels on the same tensors (a few passes)
     aten = None
@@ -423,15 +431,15 @@ def main():
 
     if rank == 0:
         peak, peak_src = peaks()
-        value = world * FRAMES * n_pass / (elapsed_ms * 1e-3)
+        value = world * FRAMES * steps / (elapsed_ms * 1e-3)
         bwd_gbs = BWD_BYTES_PX * px / (bwd_ms * 1e-3) / 1e9
         fwd_gbs = FWD_BYTES_PX * px / (fwd_ms * 1e-3) / 1e9
-        step_gbs = (FWD_BYTES_PX + BWD_BYTES_PX) * px * n_pass / (elapsed_ms * 1e-3) / 1e9
+        step_gbs = (FWD_BYTES_PX + BWD_BYTES_PX) * px * steps / (elapsed_ms * 1e-3) / 1e9
         traffic, traffic_src = recorded_traffic()
         line = {
             "metric": "1080p warped frames/s (forward+backward)", "value": value, "unit": "frames/s",
             "n_gpus": world, "steps": steps, "warmup": warmup, "ms_per_step": elapsed_ms / steps,
-            "inner_repeat": inner, "ms_per_pass": elapsed_ms / n_pass, "timed_region_s": elapsed_ms * 1e-3,
+            "ms_per_pass": elapsed_ms / steps, "timed_region_s": elapsed_ms * 1e-3,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": shared_config(world),
             "clocks": clocks,

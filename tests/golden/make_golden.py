@@ -25,10 +25,64 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF = "/root/reference"
+sys.path.insert(0, os.path.dirname(HERE))
+import synth  # noqa: E402
 
 
 def sha(a: np.ndarray) -> str:
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def config1_vectors(frame, gout, maps_planar, drift3_planar, genmaps_planar):
+    """config1_netg.npz from netG's outputs: maps_planar (3,2,256,256), drift3_planar / genmaps_planar (1,2,256,256),
+    frame / gout (1,3,256,256) float32.  A full map is 512 KiB and does not compress, so to keep the file under 1 MB
+    stages 1 and 2 keep every 8th row (each output pixel and its grad_grid depend on its own map row only) and stage 3
+    is stored as drift3 + plane + ulp offsets (tests/synth.py:config1_netg_maps).  Every case is then torch's CPU
+    grid_sample fwd + bwd on the map the tests rebuild."""
+    import torch
+    import torch.nn.functional as F
+
+    d3 = drift3_planar[0]
+    g = synth.identity_map(1, 256, 256, False, np.float64)[0].reshape(-1, 2)
+    a = np.concatenate([g, np.ones((g.shape[0], 1))], 1)
+    resid = maps_planar[2].astype(np.float64) - d3.astype(np.float64)
+    theta = np.stack([np.linalg.lstsq(a, resid[c].ravel(), rcond=None)[0] for c in range(2)])
+    ulps = maps_planar[2].view(np.int32).astype(np.int64) - synth.drift_plus_plane(d3, theta).view(np.int32)
+    assert np.abs(ulps).max() < 2 ** 15
+    out = {
+        "frame_sha": sha(frame),
+        "map_rows8": np.ascontiguousarray(maps_planar[:2, :, ::8, :]),
+        "map2_theta": theta,
+        "map2_ulps": ulps.astype(np.int16),
+        "drift3_planar": drift3_planar,
+        "genmaps_sha": sha(genmaps_planar),
+        "genmaps_sub": genmaps_planar[:, :, ::8, ::8].copy(),
+    }
+    maps = synth.config1_netg_maps(out)
+    assert np.array_equal(maps[2], maps_planar[2])
+    sub = (slice(None), slice(None), slice(None, None, 8), slice(None, None, 8))
+    # the three cascade maps (align_corners unset -> False on torch>=1.3) and the
+    # generate_maps map under both conventions (torch 0.4 behaved as True)
+    cases = [("m0", maps[0], False), ("m1", maps[1], False), ("m2", maps[2], False),
+             ("gm_f", genmaps_planar[0], False), ("gm_t", genmaps_planar[0], True)]
+    for name, planar, align in cases:
+        # planar storage (N,2,H,W): what the reference really hands to grid_sample
+        m = torch.from_numpy(planar[None]).permute(0, 2, 3, 1)
+        go = torch.from_numpy(np.ascontiguousarray(gout[:, :, ::gout.shape[2] // planar.shape[1]]))  # the map's rows
+        for pad in ("zeros", "border"):
+            fi = torch.from_numpy(frame).requires_grad_(True)
+            mi = m.clone().requires_grad_(True)
+            o = F.grid_sample(fi, mi, mode="bilinear", padding_mode=pad, align_corners=align)
+            o.backward(go)
+            key = f"{name}_{pad}"
+            out[key + "_out_sha"] = sha(o.detach().numpy())
+            out[key + "_out_sub"] = o.detach().numpy()[sub].copy()
+            out[key + "_gin_sub"] = fi.grad.numpy()[sub].copy()
+            out[key + "_gin_sum"] = np.float64(fi.grad.double().sum().item())
+            gg = mi.grad.contiguous().numpy()  # (1,H,256,2)
+            out[key + "_ggrid_sub"] = gg[:, ::8, ::8, :].copy()
+            out[key + "_ggrid_abssum"] = np.float64(np.abs(gg.astype(np.float64)).sum())
+    return out
 
 
 def main():
@@ -64,33 +118,9 @@ def main():
     finally:
         torch.Tensor.cuda = orig_cuda
 
-    out = {
-        "frame_sha": sha(frame.numpy()),
-        # planar storage (N,2,H,W): what the reference really hands to grid_sample
-        "map_planar": np.stack([m.permute(0, 3, 1, 2).contiguous().numpy()[0] for m in maps]),
-        "drift3_planar": drifts[2].permute(0, 3, 1, 2).contiguous().numpy(),
-        "genmaps_sha": sha(gm.numpy()),
-        "genmaps_sub": gm.numpy()[:, :, ::8, ::8].copy(),
-    }
-    sub = (slice(None), slice(None), slice(None, None, 8), slice(None, None, 8))
-    # the three cascade maps (align_corners unset -> False on torch>=1.3) and the
-    # generate_maps map under both conventions (torch 0.4 behaved as True)
-    cases = [("m0", maps[0], False), ("m1", maps[1], False), ("m2", maps[2], False),
-             ("gm_f", gm.permute(0, 2, 3, 1), False), ("gm_t", gm.permute(0, 2, 3, 1), True)]
-    for name, m, align in cases:
-        for pad in ("zeros", "border"):
-            fi = frame.clone().requires_grad_(True)
-            mi = m.clone().requires_grad_(True)
-            o = F.grid_sample(fi, mi, mode="bilinear", padding_mode=pad, align_corners=align)
-            o.backward(gout)
-            key = f"{name}_{pad}"
-            out[key + "_out_sha"] = sha(o.detach().numpy())
-            out[key + "_out_sub"] = o.detach().numpy()[sub].copy()
-            out[key + "_gin_sub"] = fi.grad.numpy()[sub].copy()
-            out[key + "_gin_sum"] = np.float64(fi.grad.double().sum().item())
-            gg = mi.grad.contiguous().numpy()  # (1,256,256,2)
-            out[key + "_ggrid_sub"] = gg[:, ::8, ::8, :].copy()
-            out[key + "_ggrid_abssum"] = np.float64(np.abs(gg.astype(np.float64)).sum())
+    out = config1_vectors(frame.numpy(), gout.numpy(),
+                          np.stack([m.permute(0, 3, 1, 2).contiguous().numpy()[0] for m in maps]),
+                          drifts[2].permute(0, 3, 1, 2).contiguous().numpy(), gm.contiguous().numpy())
     if not only_inference:
         np.savez_compressed(os.path.join(HERE, "config1_netg.npz"), **out)
 

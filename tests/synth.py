@@ -48,6 +48,23 @@ def make_map(kind, N, H, W, align_corners, seed=0):
     raise ValueError(kind)
 
 
+def drift_plus_plane(drift, theta):
+    """float32(drift + theta[c] . (x, y, 1)) for a planar drift (2,H,W) and a (2,3) float64 plane, x / y at the pixel
+    centres (align_corners=False); evaluated in float64 and rounded once, so it is the same on every host."""
+    g = identity_map(1, drift.shape[1], drift.shape[2], False, np.float64)[0]
+    plane = theta[:, 0, None, None] * g[None, ..., 0] + theta[:, 1, None, None] * g[None, ..., 1] + theta[:, 2, None, None]
+    return (drift.astype(np.float64) + plane).astype(np.float32)
+
+
+def config1_netg_maps(z):
+    """The reference netG's three cascade maps stored in tests/golden/config1_netg.npz, planar (2,H,W): stages 1 and 2
+    as every 8th row (map_rows8), stage 3 in full.  Stage 3 is drift3 + F.affine_grid(theta) in netG, so it is stored
+    as drift3, the least-squares plane of map - drift3 and each element's offset in ulps from drift_plus_plane: exact."""
+    pred = drift_plus_plane(z["drift3_planar"][0], z["map2_theta"])
+    m2 = (pred.view(np.int32) + z["map2_ulps"].astype(np.int32)).view(np.float32)
+    return [z["map_rows8"][0], z["map_rows8"][1], m2]
+
+
 def make_frames(N, C, H, W, seed=0):
     rng = np.random.default_rng(seed + 1000)
     return (rng.random((N, C, H, W), dtype=np.float32) * 255).astype(np.float32)

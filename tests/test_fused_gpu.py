@@ -223,7 +223,7 @@ def test_inference_site_golden_uint8_through_the_fused_kernel(pw):
     cfg = np.load(os.path.join(gold, "config1_netg.npz"))
     ih, iw = 144, 256
     hwc = torch.from_numpy(np.random.default_rng(716).integers(0, 256, (1, ih, iw, 3), dtype=np.uint8)).cuda()
-    m2 = dev(cfg["map_planar"][2][None])                       # (1,2,256,256) planar, as netG stores it
+    m2 = dev(synth.config1_netg_maps(cfg)[2][None])            # (1,2,256,256) planar, as netG stores it
     theta = dev(np.array([[[1, 0, 0], [0, 1, 0]]], np.float32))
     for name, kw in (("netg", dict(base="none")), ("netg_plus_identity", dict(base="affine", theta=theta))):
         out = pw.warp_fused(hwc.permute(0, 3, 1, 2), drift=m2.permute(0, 2, 3, 1), upsample="aligned", out_size=(ih, iw),

@@ -7,6 +7,7 @@ import os
 import numpy as np
 import pytest
 
+import synth
 from oracle import oracle
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -41,9 +42,10 @@ def test_config1_reference_netg_maps(cfg1, name, stage, align, pad):
         planar = oracle.generate_maps(z["drift3_planar"])[0]
         assert sha(planar[None]) == str(z["genmaps_sha"])  # generate_maps restated bit-exactly
     else:
-        planar = z["map_planar"][stage]
+        planar = synth.config1_netg_maps(z)[stage]
     grid = _planar_view(planar)
     assert grid.strides[3] > grid.strides[2]  # the non-contiguous view the reference passes
+    gout = np.ascontiguousarray(gout[:, :, ::gout.shape[2] // planar.shape[1]])  # the map's rows (every 8th: m0, m1)
     key = f"{name}_{pad}"
     out = oracle.forward(frame, grid, pad, align)
     # forward: bit-exact against torch CPU (same fma chain)
@@ -142,7 +144,7 @@ def test_inference_site_golden_from_the_reference_flow():
     hwc = np.random.default_rng(716).integers(0, 256, (ih, iw, 3), dtype=np.uint8)
     assert hashlib.sha256(np.ascontiguousarray(hwc).tobytes()).hexdigest() == str(site["frame_sha"])
     frame = np.ascontiguousarray(hwc.astype(np.float32).transpose(2, 0, 1)[None])
-    m2 = cfg["map_planar"][2][None]                                   # (1,2,256,256), as netG stores it
+    m2 = synth.config1_netg_maps(cfg)[2][None]                        # (1,2,256,256), as netG stores it
     ident = oracle.affine_map(np.array([[[1, 0, 0], [0, 1, 0]]], np.float32), 256, 256, None, False).transpose(0, 3, 1, 2)
     for name, lattice in (("netg", m2), ("netg_plus_identity", m2 + ident)):
         up = oracle.upsample_map(lattice, ih, iw, align_corners=True)             # (1,2,H,W)

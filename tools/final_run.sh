@@ -11,7 +11,7 @@ for s in $STEPS; do
     bench)  timeout 600 python bench.py 2>$O/bench$TAG.err | tail -1 | tee $O/bench$TAG.json | cut -c1-600
             timeout 600 python bench.py --impl reference --steps 20 --warmup 5 2>>$O/bench$TAG.err | tail -1 | tee $O/bench_reference$TAG.json | cut -c1-300 ;;
     launches) timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/launches_bench$TAG.csv \
-                python bench.py --steps 2 --warmup 3 --min-seconds 0.01 --no-cpu-baseline > $O/bench_under_ncu$TAG.log 2>&1 ;;
+                python bench.py --steps 2 --warmup 3 --no-cpu-baseline > $O/bench_under_ncu$TAG.log 2>&1 ;;
     ncu)    PROF_N=16 timeout 600 ncu --set full --clock-control none --import-source on -k regex:bwd_tma -c 1 -f -o $O/prof_bwd$TAG python tools/prof_driver.py 2>&1 | tail -1
             PROF_N=16 timeout 600 ncu --set full --clock-control none --import-source on -k regex:fwd_tma -c 1 -f -o $O/prof_fwd$TAG python tools/prof_driver.py 2>&1 | tail -1 ;;
     tables) timeout 600 python tools/config_table.py 2>&1 | tee $O/config_table$TAG.log | tail -30
