@@ -149,23 +149,6 @@ __device__ __forceinline__ void st_zero_v4_hint(float4 *p, uint64_t pol)
 {
     asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %1, %1, %1}, %2;" ::"l"(p), "f"(0.0f), "l"(pol) : "memory");
 }
-__device__ __forceinline__ void red_add_f32_hint(float *p, float v, uint64_t pol)
-{
-    asm volatile("red.relaxed.gpu.global.add.L2::cache_hint.f32 [%0], %1, %2;" ::"l"(p), "f"(v), "l"(pol));
-}
-
-// pull a box into L2 only (no shared-memory destination, no completion tracking): shortens the latency of the
-// real load that follows a few tiles later
-__device__ __forceinline__ void prefetch_l2_4d(const CUtensorMap *tm, int c0, int c1, int c2, int c3)
-{
-    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void prefetch_l2_3d(const CUtensorMap *tm, int c0, int c1, int c2)
-{
-    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
 
 // shared -> global box store / f32 add-reduction (out-of-range elements are dropped); bulk-group completion
 __device__ __forceinline__ void store_3d(const CUtensorMap *tm, const void *src, int c0, int c1, int c2)

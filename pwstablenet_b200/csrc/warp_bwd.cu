@@ -213,6 +213,21 @@ int64_t chunk_bytes()
     return (int64_t)4096 << 20;
 }
 
+// The whole backward through the persistent TMA kernel, backward_tma_max_frames() frames per launch; the kernel
+// zero-fills grad_input itself, a few bands ahead of its scatter: no memset pass.  false: the kernel cannot take the
+// problem or refused a launch (stream capture, a context too small for the cooperative launch); the caller's fallback
+// then redoes every frame.
+bool backward_tma(const Problem &pb, cudaStream_t st)
+{
+    BwdTmaPlan *plan = backward_tma_plan(pb);
+    if (!plan) return false;
+    const int step = backward_tma_max_frames();
+    bool ok = true;
+    for (int n0 = 0; ok && n0 < pb.g.N; n0 += step) ok = launch_backward_tma(plan, pb, n0, pb.g.N - n0 < step ? pb.g.N - n0 : step, st);
+    backward_tma_free(plan);
+    return ok;
+}
+
 template <typename T>
 int launch_typed(const Problem &pb, cudaStream_t st)
 {
@@ -226,17 +241,8 @@ int launch_typed(const Problem &pb, cudaStream_t st)
         if (per_chunk > g.N) per_chunk = g.N;
     }
     const bool lean = sizeof(T) == 4 && !force_generic() && backward_lean_eligible(pb);
-    BwdTmaPlan *plan = (sizeof(T) == 4 && !force_generic() && !(lean && small_problem(pb))) ? backward_tma_plan(pb) : nullptr;
-    struct PlanGuard { BwdTmaPlan *p; ~PlanGuard() { if (p) backward_tma_free(p); } } plan_guard{plan};
+    if (sizeof(T) == 4 && !force_generic() && !(lean && small_problem(pb)) && backward_tma(pb, st)) return PWS_OK;
     const int cs = (g.C == 3) ? 3 : (g.C % 4 == 0) ? 4 : (g.C % 2 == 0) ? 2 : 1;
-    if (plan) {
-        // the TMA kernel zero-fills grad_input itself (two frames ahead of its scatter): no memset pass
-        const int step = backward_tma_max_frames();
-        bool ok = true;
-        for (int n0 = 0; ok && n0 < g.N; n0 += step) ok = launch_backward_tma(plan, pb, n0, g.N - n0 < step ? g.N - n0 : step, st);
-        if (ok) return PWS_OK;
-        plan = nullptr;  // (only fails before anything was launched: attribute setup)
-    }
     for (int n0 = 0; n0 < g.N; n0 += per_chunk) {
         const int nn = (g.N - n0 < per_chunk) ? g.N - n0 : per_chunk;
         if (pb.want_gin) {
@@ -265,16 +271,7 @@ int launch_typed(const Problem &pb, cudaStream_t st)
 int launch_16bit(const Problem &pb, cudaStream_t st)
 {
     // above the small-problem threshold: the persistent TMA kernel with 16-bit grad_output tiles and frame boxes (RGB only)
-    if (!force_generic() && !small_problem(pb)) {
-        BwdTmaPlan *plan = backward_tma_plan(pb);
-        struct PlanGuard { BwdTmaPlan *p; ~PlanGuard() { if (p) backward_tma_free(p); } } plan_guard{plan};
-        if (plan) {
-            const int step = backward_tma_max_frames();
-            bool ok = true;
-            for (int n0 = 0; ok && n0 < pb.g.N; n0 += step) ok = launch_backward_tma(plan, pb, n0, pb.g.N - n0 < step ? pb.g.N - n0 : step, st);
-            if (ok) return PWS_OK;
-        }
-    }
+    if (!force_generic() && !small_problem(pb) && backward_tma(pb, st)) return PWS_OK;
     if (!backward_lean_eligible(pb)) {
         set_error("backward: 16-bit frames need W-contiguous frames / grad_output, C in {1,3} and an fp32 map");
         return PWS_EUNSUPPORTED;

@@ -2,12 +2,14 @@
 //
 // Autograd of R/main_new.py:106,116 (grad -> map) and :197 (grad -> frame), triggered at :214.
 //
-// Same pipeline as warp_fwd_tma.cu: one persistent CTA per SM walks 64x16 tiles of OUTPUT pixels;
-//   warp 0      producer   streams the tile's warp map and grad_output into shared memory (TMA);
-//   warps 1-2   scouts     (alternate tiles) reduce the map tile to the bounding box of its source taps and
-//                          load that box of the frame -- only when grad_grid is wanted, it is its one use;
-//   warps 3-10  consumers  two groups of warps, each group owning every other tile; inside a tile a
-//                          warp owns a 32-pixel-wide strip of 2*16/warps-per-group rows and marches down it.
+// One persistent CTA per SM walks 64x16 tiles of OUTPUT pixels, handed out dynamically.  Its 20 warps:
+//   2 scouts     one per consumer group, alternate tiles: TMA-load the map of the next tile, reduce this tile's map
+//                to the bounding box of its source taps, TMA-load its grad_output and that box of the frame (only when
+//                grad_grid is wanted, it is its one use), and hold the tile back until the bands of grad_input its taps
+//                can reach are zero-filled by every CTA;
+//   16 consumers two groups of 8 warps, each group owning every other tile; inside a tile a warp owns a 32-pixel-wide
+//                strip of 4 rows and marches down it;
+//   2 zero-fill  zero-fill grad_input band by band, kZeroAhead bands ahead of the scouts.
 // The scatter into grad_input is the marching scheme of warp_bwd_lean.cu: a lane whose right neighbour
 // samples the next source pixel hands its east taps over by shuffle, the south taps ride down the strip
 // in registers, and what is left is ~1 RED.ADD.F32 per source pixel and channel on consecutive addresses.
@@ -30,76 +32,36 @@ using namespace pipe;
 
 namespace {
 
-// explicit fire-and-forget reduction: with a fence elsewhere in the kernel nvcc turns atomicAdd into the
-// returning ATOMG form, whose round trip to L2 the scatter would then wait for
-#ifndef PWS_KO   // development, TIMING ONLY (results are wrong): knock out one path to see what it costs beyond its issue slots
-#define PWS_KO 0 // 1: zero-fill stores, 2: REDs, 4: grad_grid stores, 8: the scouts' wait for zero-filled bands, 16: tap loads,
-#endif           // 32: the scatter's shuffles, 64: the whole interior strip, 128: the straggler queue (tools/map_bench.py, DESIGN 3.3)
-#if PWS_KO & 2
-#define PWS_RED(p, v) do { const float v_ = (v); if (__float_as_int(v_) == 0x7fc12345) tma::red_add_f32((p), v_); } while (0)
-#else
-#define PWS_RED(p, v) tma::red_add_f32((p), (v))
-#endif
-
-// Scatter refinements of the interior body (development builds may switch them off to measure their share):
-//   east carry    an east-bottom tap nobody takes over is parked like the south-west sum and merges into the lane's own
-//                 east tap of the next row (one queue entry per broken horizontal chain instead of two);
-//   vertical dup  a row that samples the SAME source row as the one above adds the parked sum to its own bottom sum
-//                 instead of flushing it.
-#ifndef PWS_BWD_ECARRY
-#define PWS_BWD_ECARRY 1
-#endif
-#ifndef PWS_BWD_VDUP
-#define PWS_BWD_VDUP 1
-#endif
-#ifndef PWS_BWD_SIDEWAYS   // broken parked sums find a home with the left neighbour / the own north-west tap instead of the queue
-#define PWS_BWD_SIDEWAYS 0
-#endif
-#ifndef PWS_BWD_GGRID_EXACT   // 1: grad_grid of interior tiles in ATen's statement order (bit-identical to it); 0: factored form --
-#define PWS_BWD_GGRID_EXACT 1 // 22 operations per pixel instead of 48, and not one microsecond faster (DESIGN 3.3): not the product
-#endif
-#ifndef PWS_BWD_GROUPS   // consumer groups of 8 warps, one scout each (2; 1 for the scaling experiment of DESIGN 3.3)
-#define PWS_BWD_GROUPS 2
-#endif
-constexpr int kScouts = PWS_BWD_GROUPS, kGroups = PWS_BWD_GROUPS, kGroupWarps = 8, kConsumers = kGroups * kGroupWarps;
+// Tunables (measured on a B200; DESIGN 3.3 has the record of the alternatives).
+constexpr int kGroups = 2, kGroupWarps = 8;     // consumer groups of 8 warps
+constexpr int kScouts = kGroups;                // scout w feeds consumer group w (and tells it when the tiles have run out)
+constexpr int kConsumers = kGroups * kGroupWarps;
 // The zero-fill of grad_input paces the whole kernel when ONE warp does it: a band costs that warp its stores plus a
 // gpu-scope fence (~2 us while the REDs keep the memory system busy), 128 bands of a 16-frame launch = the kernel's 0.46 ms
 // (ncu: the zero-fill warp never sleeps, half of its samples sit on the fence).  kZeroWarps warps take the bands round-robin.
-// interior strip form: 0 = two phases (grad_grid of all rows, then the scatter), 1 = fused rows with a run-time box pitch,
-// 2 = fused rows, one copy of the body per box shape (compile-time pitch)
-#ifndef PWS_BWD_STRIP
-#define PWS_BWD_STRIP 1
-#endif
+constexpr int kZeroWarps = 2;
+// how far the zero-fill runs ahead of the scatter, in bands: the best look-ahead is 3-4 bands (0.593 / 0.482 / 0.469 /
+// 0.468 ms at 1 / 2 / 3 / 4)
+constexpr int kZeroAhead = 4;
 // pause of a zero-fill warp between two looks at the scouts' progress (a band lasts ~5 us; at 256 ns the polls were 7 % of
 // the kernel's instructions)
-#ifndef PWS_BWD_ZERO_POLL_NS
-#define PWS_BWD_ZERO_POLL_NS 1000
-#endif
-#ifndef PWS_BWD_STATIC_TILES
-#define PWS_BWD_STATIC_TILES 0
-#endif
-#ifndef PWS_BWD_L2PF
-#define PWS_BWD_L2PF 0   // measured: 0.434 -> 0.442 ms with it (the loads are not what the consumers wait for)
-#endif
-#ifndef PWS_BWD_ZERO_WARPS
-#define PWS_BWD_ZERO_WARPS 2
-#endif
-constexpr int kZeroWarps = PWS_BWD_ZERO_WARPS;
+constexpr int kZeroPollNs = 1000;
+// grad_input bytes per band (see below)
+constexpr int64_t kBandBytes = (int64_t)4 << 20;
+// main-ring depth of the fp32 kernel with frame boxes (without boxes, or with 16-bit boxes, the ring is 6 deep: Smem)
+constexpr int kBoxStages = 4;
+
 constexpr int kThreads = (kScouts + kConsumers + kZeroWarps) * 32;  // scouts, consumers, the warps that zero-fill grad_input
 constexpr int kZeroWarp = kScouts + kConsumers;                      // first of them
-static_assert(kScouts == kGroups, "scout w feeds consumer group w (and tells it when the tiles have run out)");
 constexpr int kInfoStop = 1 << 11;  // info.z: no more tiles for this consumer group
 
-// grad_input is zero-filled INSIDE the kernel, one frame at a time, two frames ahead of the scatter: the
-// zeroed lines are still in L2 when the REDs land and no separate memset pass runs ahead of the kernel.
-// A launch owns one slot of per-frame completion counters; the last CTA to leave resets the slot.
+// grad_input is zero-filled INSIDE the kernel, kZeroAhead bands ahead of the scatter: the zeroed lines are still in L2
+// when the REDs land and no separate memset pass runs ahead of the kernel.  Band b of a frame split into B bands is rows
+// [ceil(b*H/B), ceil((b+1)*H/B)) of every channel plane; a tile only waits for the bands its taps can reach.  Every band
+// costs its CTA's zero-fill warp a fence, an atomic and a poll (~1 us): a launch of many SMALL frames must not pay many of
+// them per frame, so B follows the frame size (about kBandBytes of grad_input per band, 1..kMaxBands).
+// A launch owns one slot of per-band completion counters; the last CTA to leave resets the slot.
 constexpr int kSyncSlots = kLaunchSlots, kSyncFrames = 256;
-// The zero-fill is tracked in bands of 1/8 frame (rows [ceil(b*H/8), ceil((b+1)*H/8)) of every channel plane): a tile
-// only needs the bands its taps can reach.  (Measured: with band tracking the best look-ahead is still 3-4 bands --
-// 0.593 / 0.482 / 0.469 / 0.468 ms at 1 / 2 / 3 / 4 -- so the finer grain buys robustness, not speed.)
-// Every band costs its CTA's zero-fill warp a fence, an atomic and a poll (~1 us): a launch of many SMALL frames must not pay
-// eight of them per frame, so the number of bands per frame follows the frame size (about 4 MB of grad_input per band,
-// 1..kMaxBands).
 constexpr int kMaxBands = 32;   // (a 4K fp32 grad_input frame is 25 bands of 4 MB)
 __device__ unsigned int g_zero_done[kSyncSlots][kSyncFrames * kMaxBands];
 __device__ unsigned int g_exit_count[kSyncSlots];
@@ -108,11 +70,6 @@ __device__ unsigned int g_exit_count[kSyncSlots];
 // with the fast CTAs waiting at the zero-fill counter of the next frame for the slow ones.
 __device__ unsigned int g_tile_next[kSyncSlots];
 // (slots are leased per device and reused only after their previous launch has finished: pws_launch.cuh)
-// how far the zero-fill runs ahead of the scatter, in bands
-#ifndef PWS_BWD_ZERO_AHEAD
-#define PWS_BWD_ZERO_AHEAD 4
-#endif
-constexpr int kZeroAhead = PWS_BWD_ZERO_AHEAD;
 
 // the scouts' progress words: a flag polled by the zero-fill warp, not data
 #ifdef PWS_BWD_ATOMIC_PROGRESS   // shared-memory atomics: silences compute-sanitizer's racecheck (used for the sanitizer runs)
@@ -131,25 +88,16 @@ __device__ __forceinline__ unsigned int ld_acquire(const unsigned int *p)
 constexpr int kStripRows = 2 * kTH / kGroupWarps;  // a warp owns a 32-column strip of this many rows
 constexpr int kQueueCap = 64;  // entries per consumer warp: 31 left over + one class of stragglers from 32 lanes
 
-// ring depth and the largest box shape a ring slot holds (tiles that need a larger box gather from global memory)
-#ifndef PWS_BWD_STAGES
-#define PWS_BWD_STAGES 4
-#endif
-#ifndef PWS_BWD_SLOT_SHAPE
-#define PWS_BWD_SLOT_SHAPE 2
-#endif
-constexpr int kSlotShape = PWS_BWD_SLOT_SHAPE;
-
-// Two rings.  A stage of the main ring holds a tile's grad_output, its frame box and its info words behind one `full`
-// and one `empty` mbarrier.  The map tiles live in a ring of their own that is two slots deeper: a scout loads the
-// map of its NEXT tile while it dispatches the current one, so that the bounding box of a tile is known before the
-// tile's stage frees up and the grad_output and box loads leave the moment it does.
+// Two rings.  A stage of the main ring holds a tile's grad_output, its frame box (room for the largest box shape) and its
+// info words behind one `full` and one `empty` mbarrier.  The map tiles live in a ring of their own that is two slots
+// deeper: a scout loads the map of its NEXT tile while it dispatches the current one, so that the bounding box of a tile
+// is known before the tile's stage frees up and the grad_output and box loads leave the moment it does.
 // kElem: bytes per frame / grad_output element (4, or 2 for f16 / bf16 frames: the smaller stages buy a deeper ring)
 template <int CS, bool kGgrid, int kElem = 4> struct Smem {
-    static constexpr int kStages = kGgrid ? (kElem == 2 ? 6 : PWS_BWD_STAGES) : 6;
+    static constexpr int kStages = kGgrid ? (kElem == 2 ? 6 : kBoxStages) : 6;
     static constexpr int kMapStages = kStages + kScouts;
     static constexpr int kGoutBytes = CS * kTW * kTH * kElem;
-    static constexpr int kBoxBytes = kGgrid ? (box_w(kSlotShape) * box_h(kSlotShape) * CS * kElem + 127) / 128 * 128 : 0;
+    static constexpr int kBoxBytes = kGgrid ? (box_w(kNumShapes - 1) * box_h(kNumShapes - 1) * CS * kElem + 127) / 128 * 128 : 0;
     static constexpr int kMapOff = 0;
     static constexpr int kGoutOff = kMapStages * kMapTileBytes;
     static constexpr int kBoxOff = kGoutOff + kStages * kGoutBytes;
@@ -201,18 +149,20 @@ __device__ __forceinline__ float *at(float *base, int off)
     return p;
 }
 
-// gp[k]: this frame's grad_input plane of channel k (one 64-bit base per plane; an entry's offset is 32-bit)
+// gp[k]: this frame's grad_input plane of channel k (one 64-bit base per plane; an entry's offset is 32-bit).
+// grad_input's adds are tma::red_add_f32, an explicit fire-and-forget reduction: with a fence elsewhere in the kernel nvcc
+// turns atomicAdd into the returning ATOMG form, whose round trip to L2 the scatter would then wait for.
 template <int CS>
 __device__ __forceinline__ void queue_pop_red(const Queue<CS> &q, int pos, float *const (&gp)[CS])
 {
     if (CS == 3) {
         const int4 e = *reinterpret_cast<const int4 *>(q.buf + pos);
-        PWS_RED(at(gp[0], e.x), __int_as_float(e.y));
-        PWS_RED(at(gp[CS > 1 ? 1 : 0], e.x), __int_as_float(e.z));
-        PWS_RED(at(gp[CS > 2 ? 2 : 0], e.x), __int_as_float(e.w));
+        tma::red_add_f32(at(gp[0], e.x), __int_as_float(e.y));
+        tma::red_add_f32(at(gp[CS > 1 ? 1 : 0], e.x), __int_as_float(e.z));
+        tma::red_add_f32(at(gp[CS > 2 ? 2 : 0], e.x), __int_as_float(e.w));
     } else {
         const int2 e = *reinterpret_cast<const int2 *>(q.buf + pos);
-        PWS_RED(at(gp[0], e.x), __int_as_float(e.y));
+        tma::red_add_f32(at(gp[0], e.x), __int_as_float(e.y));
     }
 }
 // one dense 32-lane RED per channel once a warp's worth of entries is queued (a push adds at most 32 entries to fewer
@@ -304,7 +254,7 @@ __device__ __forceinline__ void masked_row(
             if (take) { top += ptop; bot += pbot; }
             brk[k] = cy.v[k];
             if (chain) top += cy.v[k];
-            if (mask & 1u) PWS_RED(at(gp[k], o_nw), top);
+            if (mask & 1u) tma::red_add_f32(at(gp[k], o_nw), top);
             cy.v[k] = bot;
         }
         const unsigned b1 = __ballot_sync(0xffffffffu, p_e1), b2 = __ballot_sync(0xffffffffu, p_e2), b3 = __ballot_sync(0xffffffffu, p_f);
@@ -367,7 +317,7 @@ __device__ __forceinline__ void masked_strip(
     if (kGin && cy.live) {
         const int o_cy = cy.y * g.W + cy.x;
 #pragma unroll
-        for (int k = 0; k < CS; ++k) PWS_RED(at(gp[k], o_cy), cy.v[k]);
+        for (int k = 0; k < CS; ++k) tma::red_add_f32(at(gp[k], o_cy), cy.v[k]);
     }
 }
 
@@ -384,169 +334,29 @@ __device__ __forceinline__ void queue_push(Queue<CS> &q, const bool p, const int
     }
 }
 
-// two entries per flagged lane (the untaken north-east and south-east taps): one vote serves both
-template <int CS>
-__device__ __forceinline__ void queue_push2(Queue<CS> &q, const bool p, const int off_a, const float (&a)[CS], const int off_b,
-                                            const float (&b)[CS], const unsigned lt, float *const (&gp)[CS], const int lane)
-{
-    const unsigned m = __ballot_sync(0xffffffffu, p);
-    if (m) {
-        const int n = __popc(m), rank = __popc(m & lt);
-        if (p) queue_put<CS>(q, q.count + rank, off_a, a);
-        q.count += n;
-        if (q.count >= 32) queue_drain<CS>(q, gp, lane);
-        if (p) queue_put<CS>(q, q.count + rank, off_b, b);
-        q.count += n;
-        if (q.count >= 32) queue_drain<CS>(q, gp, lane);
-    }
-}
-
 // A strip (32 pixels x kStripRows rows) of an INTERIOR tile: the tile is full and every tap of every pixel lies inside
 // the frame, so there are no masks, the floor is one round-down add, and a source pixel is identified by its linear
-// offset alone.
-// The strip runs in TWO PHASES.  ncu showed the fused row body bound by latency, not by issue slots (45 % issue-active;
-// the top stalls inside the body were fixed-latency dependencies, LDS latency and instruction fetch): a row's grad_grid
-// is one dependent chain of 12 FMA pairs behind its tap loads, the scatter of the same row is a chain of shuffles, votes
-// and branches, and with four consumer warps per scheduler there is nobody to hide either.  Phase 1 computes grad_grid
-// of all the strip's rows -- no branches, fully unrolled: four independent chains for the scheduler to interleave;
-// phase 2 re-reads the map and grad_output from shared memory (15 cheap instructions per row) and runs the scatter.
+// offset alone.  grad_grid and the scatter of a row run in one body: one pass over the map and grad_output in shared memory.
 // Coordinates run on fp32 PAIRS (pws_f32x2.cuh); grad_grid accumulates (giy, gix) as one pair: per tap and channel one
 // FMUL2 (tap value x the pair of fraction weights, ATen's sign folded into the weights: -(v*d) == v*(-d) exactly) and one
 // FFMA2 with grad_output -- ATen's statements, operation for operation, so the result is bit-identical.
 // dw = 1 - de instead of (x0 + 1) - ix: de = ix - x0 is exact, so both are the rounding of the same real number.
-template <bool kAlign, bool kInter>
-__device__ __forceinline__ void strip_coords(const float *__restrict__ mq, const int r, const float2 size2,
-                                             int &x0, int &y0, float2 &es, float2 &wn)
-{
-    float2 gxy;
-    if (kInter) gxy = *reinterpret_cast<const float2 *>(mq + r * (2 * kTW));
-    else { gxy.x = mq[r * kTW]; gxy.y = mq[kTW * kTH + r * kTW]; }
-    // unnormalise (ATen's operation order), floor, fractions
-    const float2 t = x2::add(gxy, x2::bc(1.0f));
-    const float2 ixy = kAlign ? x2::mul(x2::mul(t, x2::bc(0.5f)), size2) : x2::mul(x2::fma(t, size2, x2::bc(-1.0f)), x2::bc(0.5f));
-    const float2 fl = x2::add_rm(ixy, x2::bc(12582912.0f));              // 1.5 * 2^23: the integer part lands in the mantissa
-    x0 = __float_as_int(fl.x) - 0x4B400000; y0 = __float_as_int(fl.y) - 0x4B400000;
-    es = x2::sub(ixy, x2::add(fl, x2::bc(-12582912.0f)));                // (de, ds) = (ix - x0, iy - y0)
-    wn = x2::sub(x2::bc(1.0f), es);                                      // (dw, dn)
-}
-
-template <int CS, bool kAlign, bool kInter, bool kGin, bool kGgrid>
+// Two refinements of the scatter trade ~16 issue slots per row for a quarter fewer queue entries (0.383 -> 0.367 ms / 16
+// 1080p frames with grad_input only, 0.426 -> 0.409 with grad_grid too):
+//   east carry    an east-bottom tap nobody takes over is parked like the south-west sum and merges into the lane's own
+//                 east tap of the next row (one queue entry per broken horizontal chain instead of two);
+//   vertical dup  a row that samples the SAME source row as the one above adds the parked sum to its own bottom sum
+//                 instead of flushing it.
+template <typename T, int CS, bool kAlign, bool kInter, bool kGin, bool kGgrid>
 __device__ __forceinline__ void interior_strip(
     const int lane, const float *__restrict__ mq /* this lane's map element(s) in the strip's first row */,
-    const float *__restrict__ gop, const float *__restrict__ bp /* box base, origin folded in */, const int pitch, const int plane,
+    const T *__restrict__ gop, const T *__restrict__ bp, const int pitch, const int plane,
     const float2 size2 /* (W, H) as floats; (W-1, H-1) when kAlign */, const int W, const float2 gmul2 /* (gym, gxm) */,
     float *const (&gp)[CS], float *__restrict__ ggq, const int gg_s1, const int gg_s3, Queue<CS> &q, const uint64_t pol_first)
 {
-    // The two scatter refinements trade ~16 issue slots per row for a quarter fewer queue entries.
-    constexpr bool kEcarry = PWS_BWD_ECARRY, kVdup = PWS_BWD_VDUP;
-
-    if (kGgrid) {
-        // the two grad_grid stores of a pixel: running byte pointers, one 64-bit add each per row
-        char *gq_x = reinterpret_cast<char *>(ggq), *gq_y = reinterpret_cast<char *>(ggq + gg_s3);
-        const int64_t gq_step = (int64_t)gg_s1 * 4;
-#pragma unroll
-        for (int r = 0; r < kStripRows; ++r) {
-            int x0, y0; float2 es, wn;
-            strip_coords<kAlign, kInter>(mq, r, size2, x0, y0, es, wn);
-            const float de = es.x, ds = es.y, dw = wn.x, dn = wn.y;
-            const float *__restrict__ p0 = bp + (y0 * pitch + x0);
-            const float *__restrict__ p1 = p0 + pitch;
-            // per tap the weights of (giy, gix) with ATen's signs: nw (-dw, -dn), ne (-de, +dn), sw (+dw, -ds), se (+de, +ds)
-            const float2 c_nw = make_float2(-dw, -dn), c_ne = make_float2(-de, dn), c_sw = make_float2(dw, -ds), c_se = es;
-            float2 acc = make_float2(0.f, 0.f);
-#pragma unroll
-            for (int k = 0; k < CS; ++k) {
-                const float v0 = p0[k * plane], v1 = p0[k * plane + 1], v2 = p1[k * plane], v3 = p1[k * plane + 1];
-                const float2 g2 = x2::bc(gop[k * (kTW * kTH) + r * kTW]);
-                acc = x2::fma(x2::mul(x2::bc(v0), c_nw), g2, acc);
-                acc = x2::fma(x2::mul(x2::bc(v1), c_ne), g2, acc);
-                acc = x2::fma(x2::mul(x2::bc(v2), c_sw), g2, acc);
-                acc = x2::fma(x2::mul(x2::bc(v3), c_se), g2, acc);
-            }
-            acc = x2::mul(gmul2, acc);
-            tma::st_f32_hint(reinterpret_cast<float *>(gq_x), acc.y, pol_first); tma::st_f32_hint(reinterpret_cast<float *>(gq_y), acc.x, pol_first);
-            // (volatile: the unrolled rows otherwise recompute base + r * step with twice the 64-bit adds)
-            asm volatile("add.s64 %0, %0, %1;" : "+l"(gq_x) : "l"(gq_step));
-            asm volatile("add.s64 %0, %0, %1;" : "+l"(gq_y) : "l"(gq_step));
-        }
-    }
-
-    if (kGin) {
-        const unsigned lt = (1u << lane) - 1u;
-        int co = -1, eo = -1;        // linear offsets of the parked south-west / south-east sums' targets; -1: nothing parked
-        float cv[CS], ev[CS];
-#pragma unroll
-        for (int k = 0; k < CS; ++k) { cv[k] = 0.f; ev[k] = 0.f; }
-#pragma unroll 2
-        for (int r = 0; r < kStripRows; ++r) {
-            int x0, y0; float2 es, wn;
-            strip_coords<kAlign, kInter>(mq, r, size2, x0, y0, es, wn);
-            const float de = es.x, ds = es.y, dw = wn.x, dn = wn.y;
-            float go[CS];
-#pragma unroll
-            for (int k = 0; k < CS; ++k) go[k] = gop[k * (kTW * kTH) + r * kTW];
-            const int o = y0 * W + x0;                      // north-west tap; the others are o + 1, o + W, o + W + 1
-            const int o_left = __shfl_up_sync(0xffffffffu, o, 1);
-            // lane l hands its east taps to lane l + 1 when that lane's north-west tap is this lane's north-east one
-            // (x0 <= W - 2 in an interior tile: "offset + 1" never wraps into the next row)
-            const bool take = lane > 0 && o_left + 1 == o;
-            const bool given = ((__ballot_sync(0xffffffffu, take) >> 1) >> lane) & 1u;
-            const bool chain = co == o;                               // the parked south-west sum lands on this row's north-west tap
-            const bool vdup = kVdup && co == o + W;                   // ... on its south-west tap: same source row again
-            const bool broke = co >= 0 && !chain && !vdup;
-            const bool e_chain = kEcarry && eo == o + 1, e_vdup = kEcarry && kVdup && eo == o + W + 1;
-            const bool e_broke = kEcarry && eo >= 0 && !e_chain && !e_vdup;
-            // (scalar: pairs would need as many register moves here as they save multiplies)
-            const float nw = fmul(dw, dn), ne = fmul(de, dn), sw = fmul(dw, ds), se = fmul(de, ds);
-            float et[CS], eb[CS], old_c[CS], old_e[CS];
-#pragma unroll
-            for (int k = 0; k < CS; ++k) {
-                float top = fmul(nw, go[k]), bot = fmul(sw, go[k]);   // west column
-                et[k] = fmul(ne, go[k]); eb[k] = fmul(se, go[k]);     // east column
-                old_e[k] = ev[k];
-                if (e_chain) et[k] += ev[k];                // parked south-east sum: this row's north-east tap
-                if (e_vdup) eb[k] += ev[k];
-                const float pt = __shfl_up_sync(0xffffffffu, et[k], 1), pb = __shfl_up_sync(0xffffffffu, eb[k], 1);
-                if (take) { top += pt; bot += pb; }
-                old_c[k] = cv[k];
-                if (chain) top += cv[k];
-                if (vdup) bot += cv[k];
-                PWS_RED(at(gp[k], o), top);
-                cv[k] = bot;
-                ev[k] = eb[k];
-            }
-            // stragglers -> queue: the east taps nobody took, parked sums whose chain broke
-            if (kEcarry) queue_push<CS>(q, !given, o + 1, et, lt, gp, lane);
-            else queue_push2<CS>(q, !given, o + 1, et, o + W + 1, eb, lt, gp, lane);
-            queue_push<CS>(q, broke, co, old_c, lt, gp, lane);
-            if (kEcarry) queue_push<CS>(q, e_broke, eo, old_e, lt, gp, lane);
-            co = o + W;
-            eo = (kEcarry && !given) ? o + W + 1 : -1;
-        }
-#pragma unroll
-        for (int k = 0; k < CS; ++k) PWS_RED(at(gp[k], co), cv[k]);   // every lane parked a south-west sum in the last row
-        if (kEcarry) queue_push<CS>(q, eo >= 0, eo, ev, lt, gp, lane);
-    }
-}
-
-// The same strip with grad_grid and the scatter of a row fused in one body (one pass over the map and grad_output in shared
-// memory; fewer instructions than the two-phase form, longer dependent chains).  The product form.
-template <typename T, int CS, bool kAlign, bool kInter, bool kGin, bool kGgrid, int SHAPE>
-__device__ __forceinline__ void interior_strip_fused(
-    const int lane, const float *__restrict__ mq /* this lane's map element(s) in the strip's first row */,
-    const T *__restrict__ gop, const T *__restrict__ bp, const int pitch_rt, const int plane_rt,
-    const float2 size2 /* (W, H) as floats; (W-1, H-1) when kAlign */, const int W, const float2 gmul2 /* (gym, gxm) */,
-    float *const (&gp)[CS], float *__restrict__ ggq, const int gg_s1, const int gg_s3, Queue<CS> &q, const uint64_t pol_first)
-{
-    // SHAPE >= 0: the box's row pitch and plane size are compile-time (one copy of the body per shape); SHAPE < 0: run-time
-    const int kPitch = SHAPE >= 0 ? box_w(SHAPE < 0 ? 0 : SHAPE) : pitch_rt, kPlane = SHAPE >= 0 ? box_w(SHAPE < 0 ? 0 : SHAPE) * box_h(SHAPE < 0 ? 0 : SHAPE) : plane_rt;
     // the two grad_grid stores of a pixel: running byte pointers, one 64-bit add each per row
     char *gq_x = reinterpret_cast<char *>(ggq), *gq_y = reinterpret_cast<char *>(ggq + gg_s3);
     const int64_t gq_step = (int64_t)gg_s1 * 4;
-    // The two scatter refinements trade ~16 issue slots per row for a quarter fewer queue entries: 0.383 -> 0.367 ms / 16
-    // 1080p frames in the grad_input-only kernel, 0.426 -> 0.409 in the kernel that also computes grad_grid.  (While a single
-    // zero-fill warp still paced that kernel the same switch measured as a loss, 0.469 -> 0.474.)
-    constexpr bool kEcarry = PWS_BWD_ECARRY, kVdup = PWS_BWD_VDUP;
     const unsigned lt = (1u << lane) - 1u;
     int co = -1, eo = -1;        // linear offsets of the parked south-west / south-east sums' targets; -1: nothing parked
     float cv[CS], ev[CS];
@@ -571,18 +381,13 @@ __device__ __forceinline__ void interior_strip_fused(
         const float de = es.x, ds = es.y, dw = wn.x, dn = wn.y;
 
         if (kGgrid) {
-            const T *__restrict__ p0 = bp + (y0 * kPitch + x0);
-#if PWS_BWD_GGRID_EXACT
+            const T *__restrict__ p0 = bp + (y0 * pitch + x0);
             // per tap the weights of (giy, gix) with ATen's signs: nw (-dw, -dn), ne (-de, +dn), sw (+dw, -ds), se (+de, +ds)
             const float2 c_nw = make_float2(-dw, -dn), c_ne = make_float2(-de, dn), c_sw = make_float2(dw, -ds), c_se = es;
             float2 acc = make_float2(0.f, 0.f);
 #pragma unroll
             for (int k = 0; k < CS; ++k) {
-#if PWS_KO & 16
-                const float v0 = go[k], v1 = go[k] + 1.f, v2 = go[k] + 2.f, v3 = go[k] + 3.f; (void)p0;
-#else
-                const float v0 = to_acc(p0[k * kPlane]), v1 = to_acc(p0[k * kPlane + 1]), v2 = to_acc(p0[k * kPlane + kPitch]), v3 = to_acc(p0[k * kPlane + kPitch + 1]);
-#endif
+                const float v0 = to_acc(p0[k * plane]), v1 = to_acc(p0[k * plane + 1]), v2 = to_acc(p0[k * plane + pitch]), v3 = to_acc(p0[k * plane + pitch + 1]);
                 const float2 g2 = x2::bc(go[k]);
                 acc = x2::fma(x2::mul(x2::bc(v0), c_nw), g2, acc);
                 acc = x2::fma(x2::mul(x2::bc(v1), c_ne), g2, acc);
@@ -590,29 +395,7 @@ __device__ __forceinline__ void interior_strip_fused(
                 acc = x2::fma(x2::mul(x2::bc(v3), c_se), g2, acc);
             }
             acc = x2::mul(gmul2, acc);
-#else
-            // grad_grid through the channel sums of the four taps: S_t = sum_k go_k * v_t,k (12 multiply-adds), then
-            //   giy = gym * (dw * (S_sw - S_nw) + de * (S_se - S_ne)),  gix = gxm * (dn * (S_ne - S_nw) + ds * (S_se - S_sw))
-            // -- 22 scalar operations per pixel where ATen's statement order (the EXACT build) takes 48 (25 packed pairs, which
-            // issue at half rate).  Same real-number value; the rounding differs in the last bits (measured 2.4e-7 of the
-            // largest |grad_grid| at 1080p, the size of ATen's own rounding noise: both sum signed terms of the taps' magnitude).
-            float s_nw, s_ne, s_sw, s_se;
-#pragma unroll
-            for (int k = 0; k < CS; ++k) {
-#if PWS_KO & 16
-                const float v0 = go[k], v1 = go[k] + 1.f, v2 = go[k] + 2.f, v3 = go[k] + 3.f; (void)p0;
-#else
-                const float v0 = to_acc(p0[k * kPlane]), v1 = to_acc(p0[k * kPlane + 1]), v2 = to_acc(p0[k * kPlane + kPitch]), v3 = to_acc(p0[k * kPlane + kPitch + 1]);
-#endif
-                if (k == 0) { s_nw = fmul(go[0], v0); s_ne = fmul(go[0], v1); s_sw = fmul(go[0], v2); s_se = fmul(go[0], v3); }
-                else { s_nw = fmaf(go[k], v0, s_nw); s_ne = fmaf(go[k], v1, s_ne); s_sw = fmaf(go[k], v2, s_sw); s_se = fmaf(go[k], v3, s_se); }
-            }
-            float2 acc;
-            acc.x = fmaf(de, s_se - s_ne, fmul(dw, s_sw - s_nw));
-            acc.y = fmaf(ds, s_se - s_sw, fmul(dn, s_ne - s_nw));
-            acc.x = fmul(gmul2.x, acc.x); acc.y = fmul(gmul2.y, acc.y);
-#endif
-            if (!(PWS_KO & 4) || __float_as_int(acc.x) == 0x7fc12345) { tma::st_f32_hint(reinterpret_cast<float *>(gq_x), acc.y, pol_first); tma::st_f32_hint(reinterpret_cast<float *>(gq_y), acc.x, pol_first); }
+            tma::st_f32_hint(reinterpret_cast<float *>(gq_x), acc.y, pol_first); tma::st_f32_hint(reinterpret_cast<float *>(gq_y), acc.x, pol_first);
             // (volatile: the unrolled rows otherwise recompute base + r * step with twice the 64-bit adds)
             asm volatile("add.s64 %0, %0, %1;" : "+l"(gq_x) : "l"(gq_step));
             asm volatile("add.s64 %0, %0, %1;" : "+l"(gq_y) : "l"(gq_step));
@@ -620,32 +403,17 @@ __device__ __forceinline__ void interior_strip_fused(
 
         if (kGin) {
             const int o = y0 * W + x0;                      // north-west tap; the others are o + 1, o + W, o + W + 1
-            const int o_left = (PWS_KO & 32) ? o - 1 : __shfl_up_sync(0xffffffffu, o, 1);
+            const int o_left = __shfl_up_sync(0xffffffffu, o, 1);
             // lane l hands its east taps to lane l + 1 when that lane's north-west tap is this lane's north-east one
             // (x0 <= W - 2 in an interior tile: "offset + 1" never wraps into the next row)
             const bool take = lane > 0 && o_left + 1 == o;
             const bool given = ((__ballot_sync(0xffffffffu, take) >> 1) >> lane) & 1u;
             // (r > 0: nothing is parked in the strip's first row; the loop is unrolled, the test is free)
-            const bool chain = r > 0 && co == o;                           // the parked south-west sum lands on this row's north-west tap
-            const bool vdup = r > 0 && kVdup && co == o + W;        // ... on its south-west tap: same source row again
-            bool broke = r > 0 && !chain && !vdup;
-            const bool e_chain = r > 0 && kEcarry && eo == o + 1, e_vdup = r > 0 && kEcarry && kVdup && eo == o + W + 1;
-#if PWS_BWD_SIDEWAYS
-            // Sideways homes for parked sums whose vertical chain broke (the map slants: a lane's column moved by one).
-            // (a) the parked south-east sum lands on this lane's OWN north-west tap: add it to the row's top, no entry;
-            // (b) the RIGHT neighbour's broken south-west sum lands on this lane's north-east or north-west tap: take it
-            //     (one shuffle of the target, one per channel) -- on the bench map 1.7 of a row's 8.8 queue entries
-            //     (tools/sim/straggler_homes.py).
-            const bool e_self = r > 0 && kEcarry && eo == o;
-            const int rco = __shfl_down_sync(0xffffffffu, broke ? co : -1, 1);
-            const bool r_ne = r > 0 && lane < 31 && rco == o + 1, r_nw = r > 0 && lane < 31 && rco == o;
-            // (the vote stands alone: behind `broke &&` only the lanes with a broken chain would execute it)
-            const unsigned taken = __ballot_sync(0xffffffffu, r_ne || r_nw) << 1;   // bit l: lane l's sum went to lane l - 1
-            if ((taken >> lane) & 1u) broke = false;
-            const bool e_broke = r > 0 && kEcarry && eo >= 0 && !e_chain && !e_vdup && !e_self;
-#else
-            const bool e_broke = r > 0 && kEcarry && eo >= 0 && !e_chain && !e_vdup;
-#endif
+            const bool chain = r > 0 && co == o;                    // the parked south-west sum lands on this row's north-west tap
+            const bool vdup = r > 0 && co == o + W;                 // ... on its south-west tap: same source row again
+            const bool broke = r > 0 && !chain && !vdup;
+            const bool e_chain = r > 0 && eo == o + 1, e_vdup = r > 0 && eo == o + W + 1;
+            const bool e_broke = r > 0 && eo >= 0 && !e_chain && !e_vdup;
             // (scalar: pairs would need as many register moves here as they save multiplies)
             const float nw = fmul(dw, dn), ne = fmul(de, dn), sw = fmul(dw, ds), se = fmul(de, ds);
             float et[CS], eb[CS], old_c[CS], old_e[CS];
@@ -656,40 +424,27 @@ __device__ __forceinline__ void interior_strip_fused(
                 old_e[k] = ev[k];
                 if (e_chain) et[k] += ev[k];                // parked south-east sum: this row's north-east tap
                 if (e_vdup) eb[k] += ev[k];
-#if PWS_BWD_SIDEWAYS
-                if (r > 0) {
-                    const float rv = __shfl_down_sync(0xffffffffu, cv[k], 1);   // the right neighbour's parked south-west sum
-                    if (r_ne) et[k] += rv;
-                    if (r_nw) top += rv;
-                    if (e_self) top += ev[k];
-                }
-#endif
-                const float pt = (PWS_KO & 32) ? et[k] : __shfl_up_sync(0xffffffffu, et[k], 1), pb = (PWS_KO & 32) ? eb[k] : __shfl_up_sync(0xffffffffu, eb[k], 1);
+                const float pt = __shfl_up_sync(0xffffffffu, et[k], 1), pb = __shfl_up_sync(0xffffffffu, eb[k], 1);
                 if (take) { top += pt; bot += pb; }
                 old_c[k] = cv[k];
                 if (chain) top += cv[k];
                 if (vdup) bot += cv[k];
-                PWS_RED(at(gp[k], o), top);
+                tma::red_add_f32(at(gp[k], o), top);
                 cv[k] = bot;
                 ev[k] = eb[k];
             }
             // stragglers -> queue: the north-east tap nobody took, parked sums whose chain broke
-#if !(PWS_KO & 128)
-            if (kEcarry) queue_push<CS>(q, !given, o + 1, et, lt, gp, lane);
-            else queue_push2<CS>(q, !given, o + 1, et, o + W + 1, eb, lt, gp, lane);
+            queue_push<CS>(q, !given, o + 1, et, lt, gp, lane);
             queue_push<CS>(q, broke, co, old_c, lt, gp, lane);
-            if (kEcarry) queue_push<CS>(q, e_broke, eo, old_e, lt, gp, lane);
-#else
-            if (__float_as_int(old_c[0] + old_e[0] + et[0]) == 0x7fc12345 && (broke || e_broke || !given)) queue_push<CS>(q, true, co, old_c, lt, gp, lane);
-#endif
+            queue_push<CS>(q, e_broke, eo, old_e, lt, gp, lane);
             co = o + W;
-            eo = (kEcarry && !given) ? o + W + 1 : -1;
+            eo = !given ? o + W + 1 : -1;
         }
     }
     if (kGin) {
 #pragma unroll
-        for (int k = 0; k < CS; ++k) PWS_RED(at(gp[k], co), cv[k]);   // every lane parked a south-west sum in the last row
-        if (kEcarry) queue_push<CS>(q, eo >= 0, eo, ev, lt, gp, lane);
+        for (int k = 0; k < CS; ++k) tma::red_add_f32(at(gp[k], co), cv[k]);   // every lane parked a south-west sum in the last row
+        queue_push<CS>(q, eo >= 0, eo, ev, lt, gp, lane);
     }
 }
 
@@ -710,10 +465,9 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
     uint64_t *const empty = full + kStages;
     uint64_t *const map_full = empty + kStages;
     uint64_t *const map_empty = map_full + kMapStages;
-    // [0], [1] per scout: how far it has dispatched, in bands; [2]: the last band (8 * frame + band) known
-    // to be zero-filled by every CTA, published by the zero-fill warp.  Written by the scouts and polled by the zero-fill
-    // warp (volatile; compute-sanitizer's racecheck flags exactly this pair and nothing else -- build with
-    // -DPWS_BWD_ATOMIC_PROGRESS to run it clean)
+    // [0], [1]: how far scout 0 / 1 has dispatched, in bands (kBands * frame + band).  Written by the scouts and polled by
+    // the zero-fill warps (volatile; compute-sanitizer's racecheck flags exactly this pair and nothing else -- build with
+    // -DPWS_BWD_ATOMIC_PROGRESS to run it clean).  The other two words of the 16 bytes are unused.
     int *const s_progress = reinterpret_cast<int *>(smem + S::kProgressOff);
 
     // Roles are numbered from the TOP warp of the CTA down (the scheduler favours the higher warp ids when several
@@ -777,11 +531,7 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
                 break;
             }
             int t2 = 0;
-#if PWS_BWD_STATIC_TILES   // experiment: static round-robin instead of the launch's counter
-            t2 = t1 + stride;
-#else
             if (lane == 0) t2 = (int)atomicAdd(&g_tile_next[slot], 1u) + 2 * stride;  // the tile after the next
-#endif
             const TileCoord tc1 = tile_coord(min(t1, total_tiles - 1), tiles_x, tiles_xy);
             // next tile's map: its slot was last used kMapStages iterations ago and is normally free by now
             bool next_loaded = t1 >= total_tiles;
@@ -795,21 +545,10 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
             float xlo, xhi, ylo, yhi;
             map_tile_range<kInter>(s_map + ms * kMapTileFloats, rows, cols, lane, xlo, xhi, ylo, yhi);
             int4 info = box_of_range<kBorder, kAlign, false, 16 / (int)sizeof(T)>(xlo, xhi, ylo, yhi, g.W, g.H, cols == kTW && rows == kTH);
-            if (kGgrid && kSlotShape < kNumShapes - 1 && !(info.z & (kInfoFallback | kInfoEmpty)) && (info.z & 0xff) > kSlotShape)
-                info = make_int4(0, 0, kInfoFallback, 0);
             info.w = tc.n;
             const int progress = kBands * tc.n + (kBands * (t - tc.n * tiles_xy)) / tiles_xy;  // in bands
             const bool want_box = kGgrid && !(info.z & (kInfoFallback | kInfoEmpty));
             const int shape = info.z & 0xff;
-#if PWS_BWD_L2PF
-            // The tile's operands are known now, its ring stage usually is not free yet: pull grad_output and the frame box
-            // into L2 while the scout waits, so that the real loads below -- issued the moment the stage frees up, one tile
-            // time before the consumers need them -- find them there instead of paying a DRAM round trip under load.
-            if (lane == 0 && !tma::mbar_test(empty + st, ph ^ 1)) {
-                tma::prefetch_l2_4d(&tp.gout, tc.w0, tc.h0, 0, n_begin + tc.n);
-                if (want_box) tma::prefetch_l2_4d(&tp.box[shape], info.x, info.y, 0, n_begin + tc.n);
-            }
-#endif
             tma::mbar_wait_relaxed(empty + st, ph ^ 1);
             if (lane == 0) {
                 s_info[3 * st] = info;
@@ -834,7 +573,7 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
                     progress_store(&s_progress[warp], max(progress, need));
                     // (the zero-fill warps of a CTA take the bands round-robin: completion is not in order, check every band)
                     for (int b = zero_seen + 1; b <= need; ++b)
-                        while (!(PWS_KO & 8) && ld_acquire(&g_zero_done[slot][b]) < gridDim.x) __nanosleep(64);
+                        while (ld_acquire(&g_zero_done[slot][b]) < gridDim.x) __nanosleep(64);
                     zero_seen = max(zero_seen, need);
                 } else if (kGin) {
                     progress_store(&s_progress[warp], progress);
@@ -857,7 +596,7 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
             const int last = n_frames * kBands - 1;
             for (int idx = warp - kZeroWarp; idx <= last; idx += kZeroWarps) {
                 const int f = idx / kBands, b = idx % kBands;
-                while (max(progress_load(&s_progress[0]), progress_load(&s_progress[1])) + kZeroAhead < idx) __nanosleep(PWS_BWD_ZERO_POLL_NS);
+                while (max(progress_load(&s_progress[0]), progress_load(&s_progress[1])) + kZeroAhead < idx) __nanosleep(kZeroPollNs);
                 const int r0 = (b * g.H + kBands - 1) / kBands, r1 = ((b + 1) * g.H + kBands - 1) / kBands;
                 const int band_vec = (r1 - r0) * (g.W / 4);  // float4 per channel plane
                 const int share = (band_vec + gridDim.x - 1) / gridDim.x;
@@ -865,18 +604,11 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
                 float *const fp = (float *)gin.p + (int64_t)(n_begin + f) * gin.sN + (int64_t)r0 * g.W;
                 for (int c = 0; c < CS; ++c) {
                     float4 *__restrict__ dst = reinterpret_cast<float4 *>(fp + c * plane);
-                    for (int v = v0 + lane; v < v1; v += 32) if (!(PWS_KO & 1) || v < 0) tma::st_zero_v4_hint(dst + v, pol_zero);
+                    for (int v = v0 + lane; v < v1; v += 32) tma::st_zero_v4_hint(dst + v, pol_zero);
                 }
-#ifdef PWS_BWD_RELEASE_RED
-                // the warp's stores are ordered before lane 0's release by the warp barrier; the release makes them visible
-                // at gpu scope together with the count
-                __syncwarp();
-                if (lane == 0) asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(&g_zero_done[slot][idx]) : "memory");
-#else
                 __threadfence();
                 __syncwarp();
                 if (lane == 0) atomicAdd(&g_zero_done[slot][idx], 1u);
-#endif
             }
         }
     } else {
@@ -914,24 +646,11 @@ bwd_tma_kernel(const __grid_constant__ TmaParams tp, const View in, const View g
             for (int k = 1; k < CS; ++k) gp[k] = gp[k - 1] + plane_elems;
             float *__restrict__ ggq = kGgrid ? reinterpret_cast<float *>(base.y) + gg_lane : nullptr;
 
-            if ((PWS_KO & 64) && (info.z & kInfoInterior)) {
-            } else if (info.z & kInfoInterior) {
+            if (info.z & kInfoInterior) {
                 // the box address of source pixel (x, y) is bp + y * pitch + x: fold the box origin into the base
                 const int pitch = box_w(shape), plane = box_w(shape) * box_h(shape);
-#if PWS_BWD_STRIP == 0
-                static_assert(sizeof(T) == 4, "the two-phase strip is fp32-only");
-                interior_strip<CS, kAlign, kInter, kGin, kGgrid>(lane, mp + map_lane, gop, box0 - (info.y * pitch + info.x), pitch, plane,
-                                                                 size2, g.W, gmul2, gp, ggq, ggrid.s1, ggrid.s3, q, pol_gg);
-#elif PWS_BWD_STRIP == 1
-                interior_strip_fused<T, CS, kAlign, kInter, kGin, kGgrid, -1>(lane, mp + map_lane, gop, box0 - (info.y * pitch + info.x), pitch, plane,
-                                                                           size2, g.W, gmul2, gp, ggq, ggrid.s1, ggrid.s3, q, pol_gg);
-#else
-                switch (shape) {
-                case 0: interior_strip_fused<T, CS, kAlign, kInter, kGin, kGgrid, 0>(lane, mp + map_lane, gop, box0 - (info.y * pitch + info.x), pitch, plane, size2, g.W, gmul2, gp, ggq, ggrid.s1, ggrid.s3, q, pol_gg); break;
-                case 1: interior_strip_fused<T, CS, kAlign, kInter, kGin, kGgrid, 1>(lane, mp + map_lane, gop, box0 - (info.y * pitch + info.x), pitch, plane, size2, g.W, gmul2, gp, ggq, ggrid.s1, ggrid.s3, q, pol_gg); break;
-                default: interior_strip_fused<T, CS, kAlign, kInter, kGin, kGgrid, 2>(lane, mp + map_lane, gop, box0 - (info.y * pitch + info.x), pitch, plane, size2, g.W, gmul2, gp, ggq, ggrid.s1, ggrid.s3, q, pol_gg); break;
-                }
-#endif
+                interior_strip<T, CS, kAlign, kInter, kGin, kGgrid>(lane, mp + map_lane, gop, box0 - (info.y * pitch + info.x), pitch, plane,
+                                                                    size2, g.W, gmul2, gp, ggq, ggrid.s1, ggrid.s3, q, pol_gg);
             } else {
                 const int pitch = box_w(shape), plane = box_w(shape) * box_h(shape);
                 const T *__restrict__ ip = (const T *)in.p + (int64_t)n * in.sN;
@@ -970,10 +689,7 @@ bool launch_k(const TmaParams &tp, const Problem &pb, int tiles_x, int tiles_y, 
     if (!lease.ok()) return false;  // stream capture: the caller takes the memset + non-persistent kernel path
     int slot = lease.slot();
     const int64_t frame_bytes = (int64_t)CS * pb.g.H * pb.g.W * 4;
-#ifndef PWS_BWD_BAND_MB
-#define PWS_BWD_BAND_MB 4
-#endif
-    int bands = (int)((frame_bytes + ((int64_t)PWS_BWD_BAND_MB << 20) - 1) / ((int64_t)PWS_BWD_BAND_MB << 20));
+    int bands = (int)((frame_bytes + kBandBytes - 1) / kBandBytes);
     bands = bands < 1 ? 1 : bands > kMaxBands ? kMaxBands : bands;
     // The scouts wait for EVERY CTA of the launch to have zero-filled a band of grad_input: all CTAs must be resident at
     // the same time.  A cooperative launch makes the driver guarantee that (or refuse the launch: SM-limited contexts
