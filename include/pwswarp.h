@@ -81,7 +81,8 @@ const char *pws_last_error(void);
 uint64_t pws_launch_count(void);
 
 /* Debug / tests: name of the kernel family the last forward / backward call on THIS thread launched
- * ("fwd_tma", "fwd_lean", "fwd_direct", "bwd_tma", "bwd_lean", "bwd_march", "fused", ...; "" before any call). */
+ * ("fwd_tma", "fwd_lean", "fwd_direct", "bwd_tma", "bwd_lean", "bwd_march", "bwd_lean_16", "bwd_march_16", "fused",
+ * ...; "" before any call). */
 const char *pws_last_kernel(void);
 
 /* Tuning knob (process-wide, like a library's "benchmark" switch; results do not depend on it): calls whose output has at
@@ -104,7 +105,17 @@ int pws_warp2d_forward(const pws_tensor *in, const pws_tensor *grid, pws_tensor 
  * (== output_mask[0] / [1] false).  gin must be a dense (N,C,H,W)-contiguous
  * buffer; it does NOT need to arrive zeroed: the library zero-fills it itself,
  * frame by frame, just ahead of the scatter so the lines are still in L2 when
- * the atomics land (DESIGN.md "backward").  ggrid is fully overwritten. */
+ * the atomics land (DESIGN.md "backward").  ggrid is fully overwritten.
+ * Accepts every (frame, map) dtype pair pws_warp2d_forward accepts, any strides and C:
+ *     frame / gout   map / ggrid     gin
+ *     f32            f32             f32
+ *     f64            f64             f64
+ *     f16 | bf16     f32             f32
+ *     f16 | bf16     the frame's     f32
+ * For 16-bit frames the arithmetic is fp32: ggrid is the fp32 result rounded once to
+ * the map's dtype, and gin is an fp32 ACCUMULATION buffer holding the exact fp32
+ * sums, which the caller rounds to the frame dtype once (16-bit atomics would round
+ * after every add). */
 int pws_warp2d_backward(const pws_tensor *gout, const pws_tensor *in, const pws_tensor *grid,
                         pws_tensor *gin, pws_tensor *ggrid,
                         int interp, int padding, int align_corners, void *stream);

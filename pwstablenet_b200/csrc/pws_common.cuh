@@ -44,6 +44,14 @@ template <> __device__ __forceinline__ __nv_bfloat16 from_acc<__nv_bfloat16, flo
 
 template <typename T> __device__ __forceinline__ T ldg(const T *p) { return __ldg(p); }
 
+// one map pixel's (x, y) as a single vector access: 8 bytes for fp32 maps, 4 for 16-bit maps
+__device__ __forceinline__ float2 ldg_pair(const float *p) { return __ldg(reinterpret_cast<const float2 *>(p)); }
+__device__ __forceinline__ float2 ldg_pair(const __half *p) { return __half22float2(__ldg(reinterpret_cast<const __half2 *>(p))); }
+__device__ __forceinline__ float2 ldg_pair(const __nv_bfloat16 *p) { return __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162 *>(p))); }
+__device__ __forceinline__ void st_pair(float *p, float x, float y) { *reinterpret_cast<float2 *>(p) = make_float2(x, y); }
+__device__ __forceinline__ void st_pair(__half *p, float x, float y) { *reinterpret_cast<__half2 *>(p) = __floats2half2_rn(x, y); }
+__device__ __forceinline__ void st_pair(__nv_bfloat16 *p, float x, float y) { *reinterpret_cast<__nv_bfloat162 *>(p) = __floats2bfloat162_rn(x, y); }
+
 // ---- fp32 coordinate math, explicit rounding ----------------------------------------
 __device__ __forceinline__ float unnormalize(float coord, int size, bool align)
 {
@@ -126,6 +134,14 @@ __device__ __forceinline__ void make_taps(A ix, A iy, int H, int W, Taps<A> &t)
     bool xw = (unsigned)x0 < (unsigned)W, xe = (unsigned)(x0 + 1) < (unsigned)W;
     bool yn = (unsigned)y0 < (unsigned)H, ys = (unsigned)(y0 + 1) < (unsigned)H;
     t.mask = ((xw && yn) ? 1u : 0u) | ((xe && yn) ? 2u : 0u) | ((xw && ys) ? 4u : 0u) | ((xe && ys) ? 8u : 0u);
+}
+
+// The lean kernels access an interleaved map (s3 == 1) one (x, y) pair per pixel (ldg_pair / st_pair), which needs every
+// pixel's pair aligned to its size; planar maps take scalar accesses and always qualify.
+inline bool map_pairs_ok(const View &v, int elem_bytes)
+{
+    return v.s3 != 1 || (!(reinterpret_cast<uintptr_t>(v.p) & (uintptr_t)(2 * elem_bytes - 1)) && !(v.sN & 1) && !(v.s1 & 1) &&
+                         !(v.s2 & 1));
 }
 
 // ---- error plumbing (host) -----------------------------------------------------------

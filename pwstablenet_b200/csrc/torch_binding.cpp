@@ -71,7 +71,8 @@ at::Tensor like_layout(const at::Tensor &t)
 std::tuple<at::Tensor, at::Tensor> warp2d_backward(const at::Tensor &grad_output, const at::Tensor &input, const at::Tensor &grid,
                                                    int64_t padding, bool align_corners, bool need_input, bool need_grid)
 {
-    const bool half_frames = grid.scalar_type() != input.scalar_type();   // 16-bit frames with an fp32 map (BASELINE config 5)
+    // 16-bit frames, with an fp32 map or one of the frame's type
+    const bool half_frames = input.scalar_type() == at::kHalf || input.scalar_type() == at::kBFloat16;
     at::Tensor gin, ggrid;
     // with 16-bit frames the contributions are summed in fp32 and rounded to the frame type once
     if (need_input) gin = at::empty(input.sizes(), half_frames ? input.options().dtype(at::kFloat) : input.options());

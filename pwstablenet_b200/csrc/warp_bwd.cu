@@ -39,12 +39,47 @@ constexpr int kTileW = 32 * kWarpsX, kTileH = kRows * kWarpsY;
 
 template <typename T> __device__ __forceinline__ void red_add(T *p, T v) { atomicAdd(p, v); }
 
-template <typename T, int CS, bool kGin, bool kGgrid>
+// grad_grid of one pixel over all C channels in one pass, for maps too narrow to park partial sums between channel chunks:
+// the fma chain of bwd_march_kernel, channel after channel, rounded to G once
+template <typename T, typename G, typename A>
+__device__ __forceinline__ void ggrid_all_channels(const T *__restrict__ gop, const T *__restrict__ ip, G *__restrict__ ggp,
+                                                   const View &gout, const View &in, const View &ggrid, const Geometry &g,
+                                                   const Taps<A> &t, const A gxm, const A gym, const int h, const int w)
+{
+    const A x0f = (A)t.x0, y0f = (A)t.y0, x1f = (A)(t.x0 + 1), y1f = (A)(t.y0 + 1);
+    const A dn = fsub(y1f, t.iy), ds = fsub(t.iy, y0f), dw = fsub(x1f, t.ix), de = fsub(t.ix, x0f);
+    const int o_nw = t.y0 * in.s2 + t.x0 * in.s3;
+    const T *__restrict__ goc = gop + h * gout.s2 + w * gout.s3;
+    A gix = (A)0, giy = (A)0;
+    for (int c = 0; c < g.C; ++c) {
+        const A go = to_acc(ldg(goc + c * gout.s1));
+        const T *__restrict__ pc = ip + c * in.s1;
+        A v0 = (A)0, v1 = (A)0, v2 = (A)0, v3 = (A)0;
+        if (t.mask & 1u) v0 = to_acc(ldg(pc + o_nw));
+        if (t.mask & 2u) v1 = to_acc(ldg(pc + o_nw + in.s3));
+        if (t.mask & 4u) v2 = to_acc(ldg(pc + o_nw + in.s2));
+        if (t.mask & 8u) v3 = to_acc(ldg(pc + o_nw + in.s2 + in.s3));
+        if (t.mask & 1u) { gix = ffma(-fmul(v0, dn), go, gix); giy = ffma(-fmul(v0, dw), go, giy); }
+        if (t.mask & 2u) { gix = ffma(fmul(v1, dn), go, gix);  giy = ffma(-fmul(v1, de), go, giy); }
+        if (t.mask & 4u) { gix = ffma(-fmul(v2, ds), go, gix); giy = ffma(fmul(v2, dw), go, giy); }
+        if (t.mask & 8u) { gix = ffma(fmul(v3, ds), go, gix);  giy = ffma(fmul(v3, de), go, giy); }
+    }
+    const int off = h * ggrid.s1 + w * ggrid.s2;
+    ggp[off] = from_acc<G, A>(fmul(gxm, gix));
+    ggp[off + ggrid.s3] = from_acc<G, A>(fmul(gym, giy));
+}
+
+// T: element type of the frame and of grad_output; G: of the map and of grad_grid (T, or float for 16-bit frames).
+// grad_input is written in the accumulation type (fp32 for 16-bit frames: the caller rounds the sums once).
+template <typename T, typename G, int CS, bool kGin, bool kGgrid>
 __global__ void __launch_bounds__(kThreads)
 bwd_march_kernel(const View gout, const View in, const View grid, const View gin, const View ggrid,
                  const Geometry g, const int tiles_x, const int tiles_y, const int n_begin)
 {
     using A = typename Acc<T>::type;
+    // grad_grid can hold the raw partial sums between channel chunks only when it is at least as wide as the accumulator;
+    // a 16-bit grad_grid would round them, so those maps sum every channel in registers during the first chunk instead
+    constexpr bool kPark = sizeof(G) >= sizeof(A);
     const int tile = blockIdx.x;
     const int tx = tile % tiles_x;
     const int rest = tile / tiles_x;
@@ -59,9 +94,9 @@ bwd_march_kernel(const View gout, const View in, const View grid, const View gin
 
     const T *__restrict__ gop = (const T *)gout.p + (int64_t)n * gout.sN;
     const T *__restrict__ ip = (const T *)in.p + (int64_t)n * in.sN;
-    const T *__restrict__ gp = (const T *)grid.p + (int64_t)n * grid.sN;
-    T *__restrict__ gip = kGin ? (T *)gin.p + (int64_t)n * gin.sN : nullptr;
-    T *__restrict__ ggp = kGgrid ? (T *)ggrid.p + (int64_t)n * ggrid.sN : nullptr;
+    const G *__restrict__ gp = (const G *)grid.p + (int64_t)n * grid.sN;
+    A *__restrict__ gip = kGin ? (A *)gin.p + (int64_t)n * gin.sN : nullptr;
+    G *__restrict__ ggp = kGgrid ? (G *)ggrid.p + (int64_t)n * ggrid.sN : nullptr;
 
     const int rows = min(kRows, g.Ho - h0);
 
@@ -109,7 +144,7 @@ bwd_march_kernel(const View gout, const View in, const View grid, const View gin
             }
             if (!col_ok) t.mask = 0u;
 
-            if (kGgrid && col_ok) {
+            if (kPark && kGgrid && col_ok) {
                 const A x0f = (A)t.x0, y0f = (A)t.y0, x1f = (A)(t.x0 + 1), y1f = (A)(t.y0 + 1);
                 const A dn = fsub(y1f, t.iy), ds = fsub(t.iy, y0f), dw = fsub(x1f, t.ix), de = fsub(t.ix, x0f);
                 const int o_nw = t.y0 * in.s2 + t.x0 * in.s3;
@@ -133,8 +168,11 @@ bwd_march_kernel(const View gout, const View in, const View grid, const View gin
                     if (t.mask & 8u) { gix = ffma(fmul(v3, ds), go[k], gix);  giy = ffma(fmul(v3, de), go[k], giy); }
                 }
                 if (c0 + CS >= g.C) { gix = fmul(gxm, gix); giy = fmul(gym, giy); }
-                ggp[off] = from_acc<T, A>(gix);
-                ggp[off + ggrid.s3] = from_acc<T, A>(giy);
+                ggp[off] = from_acc<G, A>(gix);
+                ggp[off + ggrid.s3] = from_acc<G, A>(giy);
+            }
+            if constexpr (!kPark) {
+                if (kGgrid && col_ok && c0 == 0) ggrid_all_channels<T, G>(gop, ip, ggp, gout, in, ggrid, g, t, gxm, gym, h, w);
             }
 
             if (kGin) {
@@ -149,18 +187,18 @@ bwd_march_kernel(const View gout, const View in, const View grid, const View gin
                 const int o_carry = carry_y * gin.s2 + carry_x * gin.s3;
 #pragma unroll
                 for (int k = 0; k < CS; ++k) {
-                    T *__restrict__ pc = gip + (c0 + k) * gin.s1;
+                    A *__restrict__ pc = gip + (c0 + k) * gin.s1;
                     A top = fmul(t.nw, go[k]), bot = fmul(t.sw, go[k]);
                     const A etop = fmul(t.ne, go[k]), ebot = fmul(t.se, go[k]);
                     const A ptop = __shfl_up_sync(0xffffffffu, etop, 1), pbot = __shfl_up_sync(0xffffffffu, ebot, 1);
                     if (take) { top += ptop; bot += pbot; }
                     if (!given) {
-                        if (t.mask & 2u) red_add(pc + o_nw + gin.s3, from_acc<T, A>(etop));
-                        if (t.mask & 8u) red_add(pc + o_nw + gin.s2 + gin.s3, from_acc<T, A>(ebot));
+                        if (t.mask & 2u) red_add(pc + o_nw + gin.s3, etop);
+                        if (t.mask & 8u) red_add(pc + o_nw + gin.s2 + gin.s3, ebot);
                     }
                     if (chain) top += carry_v[k];
-                    else if (carry_live) red_add(pc + o_carry, from_acc<T, A>(carry_v[k]));
-                    if (t.mask & 1u) red_add(pc + o_nw, from_acc<T, A>(top));
+                    else if (carry_live) red_add(pc + o_carry, carry_v[k]);
+                    if (t.mask & 1u) red_add(pc + o_nw, top);
                     carry_v[k] = bot;
                 }
                 carry_x = t.x0; carry_y = t.y0 + 1;
@@ -170,20 +208,20 @@ bwd_march_kernel(const View gout, const View in, const View grid, const View gin
         if (kGin && carry_live) {
             const int o_carry = carry_y * gin.s2 + carry_x * gin.s3;
 #pragma unroll
-            for (int k = 0; k < CS; ++k) red_add(gip + (c0 + k) * gin.s1 + o_carry, from_acc<T, A>(carry_v[k]));
+            for (int k = 0; k < CS; ++k) red_add(gip + (c0 + k) * gin.s1 + o_carry, carry_v[k]);
         }
     }
 }
 
-template <typename T, int CS>
+template <typename T, typename G, int CS>
 void launch_cs(const Problem &pb, unsigned blocks, int tiles_x, int tiles_y, int n_begin, cudaStream_t st)
 {
     if (pb.want_gin && pb.want_ggrid)
-        { bwd_march_kernel<T, CS, true, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, tiles_x, tiles_y, n_begin); note_launch(); }
+        { bwd_march_kernel<T, G, CS, true, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, tiles_x, tiles_y, n_begin); note_launch(); }
     else if (pb.want_gin)
-        { bwd_march_kernel<T, CS, true, false><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, tiles_x, tiles_y, n_begin); note_launch(); }
+        { bwd_march_kernel<T, G, CS, true, false><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, tiles_x, tiles_y, n_begin); note_launch(); }
     else
-        { bwd_march_kernel<T, CS, false, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, tiles_x, tiles_y, n_begin); note_launch(); }
+        { bwd_march_kernel<T, G, CS, false, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, tiles_x, tiles_y, n_begin); note_launch(); }
 }
 
 }  // namespace
@@ -228,12 +266,15 @@ bool backward_tma(const Problem &pb, cudaStream_t st)
     return ok;
 }
 
-template <typename T>
+// f32 / f64 problems (TMA, lean or march kernel), and the march kernel for 16-bit frames (T 16-bit; grad_input is then the
+// fp32 accumulation buffer, so the zero-fill is sized by the accumulator type, not by T)
+template <typename T, typename G>
 int launch_typed(const Problem &pb, cudaStream_t st)
 {
     const Geometry &g = pb.g;
     const int tiles_x = (g.Wo + kTileW - 1) / kTileW, tiles_y = (g.Ho + kTileH - 1) / kTileH;
-    const int64_t frame_bytes = (int64_t)g.C * g.H * g.W * (int64_t)sizeof(T);
+    const int64_t gin_elem = (int64_t)sizeof(typename Acc<T>::type);
+    const int64_t frame_bytes = (int64_t)g.C * g.H * g.W * gin_elem;
     int per_chunk = g.N;
     if (pb.want_gin) {
         per_chunk = (int)(chunk_bytes() / (frame_bytes > 0 ? frame_bytes : 1));
@@ -242,39 +283,44 @@ int launch_typed(const Problem &pb, cudaStream_t st)
     }
     const bool lean = sizeof(T) == 4 && !force_generic() && backward_lean_eligible(pb);
     if (sizeof(T) == 4 && !force_generic() && !(lean && small_problem(pb)) && backward_tma(pb, st)) return PWS_OK;
-    const int cs = (g.C == 3) ? 3 : (g.C % 4 == 0) ? 4 : (g.C % 2 == 0) ? 2 : 1;
+    // 16-bit frames chunk at most 2 channels: their CS = 4 instantiation spills (128 registers)
+    constexpr int kCs4 = sizeof(T) == 2 ? 2 : 4;
+    const int cs = (g.C == 3) ? 3 : (g.C % kCs4 == 0) ? kCs4 : (g.C % 2 == 0) ? 2 : 1;
     for (int n0 = 0; n0 < g.N; n0 += per_chunk) {
         const int nn = (g.N - n0 < per_chunk) ? g.N - n0 : per_chunk;
         if (pb.want_gin) {
-            cudaError_t e = cudaMemsetAsync((char *)pb.gin.p + (int64_t)n0 * pb.gin.sN * (int64_t)sizeof(T), 0,
+            cudaError_t e = cudaMemsetAsync((char *)pb.gin.p + (int64_t)n0 * pb.gin.sN * gin_elem, 0,
                                             (size_t)(frame_bytes * nn), st);
             if (e != cudaSuccess) { set_error("backward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return PWS_ECUDA; }
         }
-        note_kernel(lean ? "bwd_lean" : "bwd_march");
+        note_kernel(lean ? "bwd_lean" : sizeof(T) == 2 ? "bwd_march_16" : "bwd_march");
         if (lean) { launch_backward_lean(pb, n0, nn, st); continue; }
         const int64_t tiles = (int64_t)tiles_x * tiles_y * nn;
         if (tiles == 0) continue;
         if (tiles > INT_MAX) { set_error("backward: too many tiles"); return PWS_EUNSUPPORTED; }
         switch (cs) {
-            case 3: launch_cs<T, 3>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
-            case 4: launch_cs<T, 4>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
-            case 2: launch_cs<T, 2>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
-            default: launch_cs<T, 1>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
+            case 3: launch_cs<T, G, 3>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
+            case 4: launch_cs<T, G, kCs4>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
+            case 2: launch_cs<T, G, 2>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
+            default: launch_cs<T, G, 1>(pb, (unsigned)tiles, tiles_x, tiles_y, n0, st); break;
         }
     }
     return PWS_OK;
 }
 
-// 16-bit frames and grad_output with an fp32 map (BASELINE config 5): fp32 arithmetic, fp32 grad_grid and an fp32
-// grad_input ACCUMULATION buffer (capi.cu requires it), which the caller rounds to the frame type once -- summing a
-// pixel's contributions in bf16 would round after every atomic.
+// 16-bit frames and grad_output with an fp32 map (BASELINE config 5) or a map of the frame's type: fp32 arithmetic, grad_grid
+// rounded to the map's type once, and an fp32 grad_input ACCUMULATION buffer (capi.cu requires it), which the caller rounds
+// to the frame type once -- summing a pixel's contributions in bf16 would round after every atomic.
 int launch_16bit(const Problem &pb, cudaStream_t st)
 {
-    // above the small-problem threshold: the persistent TMA kernel with 16-bit grad_output tiles and frame boxes (RGB only)
+    // above the small-problem threshold: the persistent TMA kernel with 16-bit grad_output tiles and frame boxes (RGB, fp32
+    // maps only)
     if (!force_generic() && !small_problem(pb) && backward_tma(pb, st)) return PWS_OK;
     if (!backward_lean_eligible(pb)) {
-        set_error("backward: 16-bit frames need W-contiguous frames / grad_output, C in {1,3} and an fp32 map");
-        return PWS_EUNSUPPORTED;
+        // any C, strides, channels-last or cropped frames: the marching kernel
+        const bool map32 = pb.grid_dtype == PWS_F32;
+        if (pb.in_dtype == PWS_F16) return map32 ? launch_typed<__half, float>(pb, st) : launch_typed<__half, __half>(pb, st);
+        return map32 ? launch_typed<__nv_bfloat16, float>(pb, st) : launch_typed<__nv_bfloat16, __nv_bfloat16>(pb, st);
     }
     const Geometry &g = pb.g;
     if (pb.want_gin) {
@@ -291,14 +337,14 @@ int launch_16bit(const Problem &pb, cudaStream_t st)
 int launch_backward(const Problem &pb, cudaStream_t st)
 {
     if (!pb.want_gin && !pb.want_ggrid) return PWS_OK;
-    if ((pb.in_dtype == PWS_F16 || pb.in_dtype == PWS_BF16) && pb.grid_dtype == PWS_F32) return launch_16bit(pb, st);
-    if (pb.in_dtype != pb.grid_dtype) {
+    if (pb.in_dtype != pb.grid_dtype && !(pb.grid_dtype == PWS_F32 && (pb.in_dtype == PWS_F16 || pb.in_dtype == PWS_BF16))) {
         set_error("backward: frame and map dtypes must match, or 16-bit frames with an fp32 map (got %d, %d)", pb.in_dtype, pb.grid_dtype);
         return PWS_EUNSUPPORTED;
     }
-    if (pb.in_dtype == PWS_F32) return launch_typed<float>(pb, st);
-    if (pb.in_dtype == PWS_F64) return launch_typed<double>(pb, st);
-    set_error("backward: unsupported dtype %d (f32 and f64 only)", pb.in_dtype);
+    if (pb.in_dtype == PWS_F16 || pb.in_dtype == PWS_BF16) return launch_16bit(pb, st);
+    if (pb.in_dtype == PWS_F32) return launch_typed<float, float>(pb, st);
+    if (pb.in_dtype == PWS_F64) return launch_typed<double, double>(pb, st);
+    set_error("backward: unsupported dtype %d", pb.in_dtype);
     return PWS_EUNSUPPORTED;
 }
 

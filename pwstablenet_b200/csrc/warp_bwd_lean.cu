@@ -1,5 +1,5 @@
 // warp_bwd_lean.cu -- backward warp specialised for the reference's hot layouts
-// (NCHW fp32 frames / grad_output W-contiguous, fp32 map planar or interleaved, C in {1,3}).
+// (NCHW frames / grad_output W-contiguous, map planar or interleaved, C in {1,3}).
 //
 // Same algorithm as the generic marching kernel in warp_bwd.cu (horizontal take-over of the
 // east taps by shuffle, vertical carry of the south taps in registers, one RED per source
@@ -25,13 +25,13 @@ struct Carry {
 };
 
 // One output row of a warp.  kMasked=false: every lane is a real pixel with 4 valid taps.
-template <typename T, int CS, bool kGin, bool kGgrid, bool kMasked>
+template <typename T, typename G, int CS, bool kGin, bool kGgrid, bool kMasked>
 __device__ __forceinline__ void row_body(
     const int lane, const bool px_ok, const unsigned live,
     const float ix, const float iy, const float gxm, const float gym, const float (&go)[CS],
     const T *__restrict__ ip, const int sH, const int i_ch, const int H, const int W,
     float *__restrict__ gip, const int gi_ch,
-    float *__restrict__ ggq, const int gg_s3, Carry<CS> &cy, int2 *__restrict__ queue)
+    G *__restrict__ ggq, const int gg_s3, Carry<CS> &cy, int2 *__restrict__ queue)
 {
     const float x0f = floorf(ix), y0f = floorf(iy);
     const int x0 = (int)x0f, y0 = (int)y0f;
@@ -62,8 +62,8 @@ __device__ __forceinline__ void row_body(
             if (!kMasked || (mask & 8u)) { gix = ffma(fmul(v3, ds), go[k], gix);  giy = ffma(fmul(v3, de), go[k], giy); }
         }
         gix = fmul(gxm, gix); giy = fmul(gym, giy);
-        if (gg_s3 == 1) *reinterpret_cast<float2 *>(ggq) = make_float2(gix, giy);
-        else { ggq[0] = gix; ggq[gg_s3] = giy; }
+        if (gg_s3 == 1) st_pair(ggq, gix, giy);
+        else { ggq[0] = from_acc<G, float>(gix); ggq[gg_s3] = from_acc<G, float>(giy); }
     }
 
     if (kGin) {
@@ -116,9 +116,10 @@ __device__ __forceinline__ void row_body(
     }
 }
 
-// T: element type of the frame and of grad_output (float, or __half / __nv_bfloat16 with fp32 maps -- BASELINE config 5);
-// the arithmetic, grad_grid and the grad_input accumulation buffer are fp32 whatever T is.
-template <typename T, int CS, bool kBorder, bool kAlign, bool kGin, bool kGgrid>
+// T: element type of the frame and of grad_output (float, __half or __nv_bfloat16).  G: element type of the map and of
+// grad_grid (float, or T for 16-bit frames).  The arithmetic and the grad_input accumulation buffer are fp32 whatever T and
+// G are; grad_grid is rounded to G once, at its store.
+template <typename T, typename G, int CS, bool kBorder, bool kAlign, bool kGin, bool kGgrid>
 #ifndef PWS_BWD_MINB
 #define PWS_BWD_MINB 4   // 64 registers, 32 warps/SM: measured 5-9 % faster than 3 CTAs at 80 registers
 #endif
@@ -144,9 +145,9 @@ bwd_lean_kernel(const View gout, const View in, const View grid, const View gin,
     const int i_ch = in.s1, gi_ch = kGin ? gin.s1 : 0, go_ch = gout.s1;  // 32-bit in-frame offsets (validated on the host)
 
     const bool inter = grid.s3 == 1;
-    const float *__restrict__ gq = (const float *)grid.p + (int64_t)n * grid.sN + (int64_t)h0 * grid.s1 + (int64_t)w * grid.s2;
+    const G *__restrict__ gq = (const G *)grid.p + (int64_t)n * grid.sN + (int64_t)h0 * grid.s1 + (int64_t)w * grid.s2;
     const T *__restrict__ goq = (const T *)gout.p + (int64_t)n * gout.sN + (int64_t)h0 * gout.s2 + w;
-    float *__restrict__ ggq = kGgrid ? (float *)ggrid.p + (int64_t)n * ggrid.sN + (int64_t)h0 * ggrid.s1 + (int64_t)w * ggrid.s2 : nullptr;
+    G *__restrict__ ggq = kGgrid ? (G *)ggrid.p + (int64_t)n * ggrid.sN + (int64_t)h0 * ggrid.s1 + (int64_t)w * ggrid.s2 : nullptr;
 
     Carry<CS> cy;
     cy.x = 0; cy.y = 0; cy.live = false;
@@ -158,8 +159,8 @@ bwd_lean_kernel(const View gout, const View in, const View grid, const View gin,
 #pragma unroll
     for (int k = 0; k < CS; ++k) go_n[k] = 0.f;
     if (col_ok) {
-        if (inter) { const float2 v = __ldg(reinterpret_cast<const float2 *>(gq)); gx_n = v.x; gy_n = v.y; }
-        else { gx_n = __ldg(gq); gy_n = __ldg(gq + grid.s3); }
+        if (inter) { const float2 v = ldg_pair(gq); gx_n = v.x; gy_n = v.y; }
+        else { gx_n = to_acc(ldg(gq)); gy_n = to_acc(ldg(gq + grid.s3)); }
 #pragma unroll
         for (int k = 0; k < CS; ++k) go_n[k] = to_acc(ldg(goq + k * go_ch));
     }
@@ -171,8 +172,8 @@ bwd_lean_kernel(const View gout, const View in, const View grid, const View gin,
         for (int k = 0; k < CS; ++k) go[k] = go_n[k];
         gq += grid.s1; goq += gout.s2;
         if (col_ok && r + 1 < rows) {
-            if (inter) { const float2 v = __ldg(reinterpret_cast<const float2 *>(gq)); gx_n = v.x; gy_n = v.y; }
-            else { gx_n = __ldg(gq); gy_n = __ldg(gq + grid.s3); }
+            if (inter) { const float2 v = ldg_pair(gq); gx_n = v.x; gy_n = v.y; }
+            else { gx_n = to_acc(ldg(gq)); gy_n = to_acc(ldg(gq + grid.s3)); }
 #pragma unroll
             for (int k = 0; k < CS; ++k) go_n[k] = to_acc(ldg(goq + k * go_ch));
         }
@@ -181,9 +182,9 @@ bwd_lean_kernel(const View gout, const View in, const View grid, const View gin,
         const float iy = src_index_grad<kBorder, kAlign>(gy, Hf, Hm1, &gym);
         const bool inside = col_ok && ix >= 0.0f && ix < Wm1 && iy >= 0.0f && iy < Hm1;  // floor in [0, size-2]
         if (__all_sync(0xffffffffu, inside))
-            row_body<T, CS, kGin, kGgrid, false>(lane, true, live, ix, iy, gxm, gym, go, ip, sH, i_ch, g.H, g.W, gip, gi_ch, ggq, ggrid.s3, cy, queue);
+            row_body<T, G, CS, kGin, kGgrid, false>(lane, true, live, ix, iy, gxm, gym, go, ip, sH, i_ch, g.H, g.W, gip, gi_ch, ggq, ggrid.s3, cy, queue);
         else
-            row_body<T, CS, kGin, kGgrid, true>(lane, col_ok, live, ix, iy, gxm, gym, go, ip, sH, i_ch, g.H, g.W, gip, gi_ch, ggq, ggrid.s3, cy, queue);
+            row_body<T, G, CS, kGin, kGgrid, true>(lane, col_ok, live, ix, iy, gxm, gym, go, ip, sH, i_ch, g.H, g.W, gip, gi_ch, ggq, ggrid.s3, cy, queue);
         if (kGgrid) ggq += ggrid.s1;
     }
     if (kGin && cy.live) {
@@ -193,25 +194,32 @@ bwd_lean_kernel(const View gout, const View in, const View grid, const View gin,
     }
 }
 
-template <typename T, int CS, bool kBorder, bool kAlign>
+template <typename T, typename G, int CS, bool kBorder, bool kAlign>
 void launch_ba(const Problem &pb, dim3 blocks, int n0, cudaStream_t st)
 {
     if (pb.want_gin && pb.want_ggrid)
-        { bwd_lean_kernel<T, CS, kBorder, kAlign, true, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, n0); note_launch(); }
+        { bwd_lean_kernel<T, G, CS, kBorder, kAlign, true, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, n0); note_launch(); }
     else if (pb.want_gin)
-        { bwd_lean_kernel<T, CS, kBorder, kAlign, true, false><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, n0); note_launch(); }
+        { bwd_lean_kernel<T, G, CS, kBorder, kAlign, true, false><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, n0); note_launch(); }
     else
-        { bwd_lean_kernel<T, CS, kBorder, kAlign, false, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, n0); note_launch(); }
+        { bwd_lean_kernel<T, G, CS, kBorder, kAlign, false, true><<<blocks, kThreads, 0, st>>>(pb.gout, pb.in, pb.grid, pb.gin, pb.ggrid, pb.g, n0); note_launch(); }
 }
 
-template <typename T, int CS>
+template <typename T, typename G, int CS>
 void launch_cs(const Problem &pb, dim3 blocks, int n0, cudaStream_t st)
 {
     const bool border = pb.g.padding == PWS_PAD_BORDER, align = pb.g.align != 0;
-    if (border && align) launch_ba<T, CS, true, true>(pb, blocks, n0, st);
-    else if (border) launch_ba<T, CS, true, false>(pb, blocks, n0, st);
-    else if (align) launch_ba<T, CS, false, true>(pb, blocks, n0, st);
-    else launch_ba<T, CS, false, false>(pb, blocks, n0, st);
+    if (border && align) launch_ba<T, G, CS, true, true>(pb, blocks, n0, st);
+    else if (border) launch_ba<T, G, CS, true, false>(pb, blocks, n0, st);
+    else if (align) launch_ba<T, G, CS, false, true>(pb, blocks, n0, st);
+    else launch_ba<T, G, CS, false, false>(pb, blocks, n0, st);
+}
+
+template <typename T, typename G>
+void launch_c(const Problem &pb, dim3 blocks, int n0, cudaStream_t st)
+{
+    if (pb.g.C == 3) launch_cs<T, G, 3>(pb, blocks, n0, st);
+    else launch_cs<T, G, 1>(pb, blocks, n0, st);
 }
 
 }  // namespace
@@ -219,17 +227,15 @@ void launch_cs(const Problem &pb, dim3 blocks, int n0, cudaStream_t st)
 bool backward_lean_eligible(const Problem &pb)
 {
     const Geometry &g = pb.g;
-    if (pb.grid_dtype != PWS_F32) return false;
     if (pb.in_dtype != PWS_F32 && pb.in_dtype != PWS_F16 && pb.in_dtype != PWS_BF16) return false;
+    const bool map32 = pb.grid_dtype == PWS_F32;
+    if (!map32 && pb.grid_dtype != pb.in_dtype) return false;
     if (g.C != 1 && g.C != 3) return false;
     if (pb.in.s3 != 1 || pb.gout.s3 != 1) return false;
     // the scatter reuses the frame's in-plane offset for grad_input: same pitch required
     if (pb.want_gin && !(pb.gin.s3 == 1 && pb.gin.s2 == pb.in.s2)) return false;
-    if (pb.grid.s3 == 1 && ((reinterpret_cast<uintptr_t>(pb.grid.p) & 7) || (pb.grid.sN & 1) || (pb.grid.s1 & 1) || (pb.grid.s2 & 1)))
-        return false;
-    if (pb.want_ggrid && pb.ggrid.s3 == 1 &&
-        ((reinterpret_cast<uintptr_t>(pb.ggrid.p) & 7) || (pb.ggrid.sN & 1) || (pb.ggrid.s1 & 1) || (pb.ggrid.s2 & 1)))
-        return false;
+    if (!map_pairs_ok(pb.grid, map32 ? 4 : 2)) return false;
+    if (pb.want_ggrid && !map_pairs_ok(pb.ggrid, map32 ? 4 : 2)) return false;
     if ((g.Ho + kTH - 1) / kTH > 65535) return false;
     return true;
 }
@@ -241,9 +247,10 @@ void launch_backward_lean(const Problem &pb, int n0, int nn, cudaStream_t st)
     for (int z0 = 0; z0 < nn; z0 += 65535) {
         const int nz = nn - z0 < 65535 ? nn - z0 : 65535;
         dim3 blocks((g.Wo + kTW - 1) / kTW, (g.Ho + kTH - 1) / kTH, nz);
-        if (pb.in_dtype == PWS_F32) { if (g.C == 3) launch_cs<float, 3>(pb, blocks, n0 + z0, st); else launch_cs<float, 1>(pb, blocks, n0 + z0, st); }
-        else if (pb.in_dtype == PWS_F16) { if (g.C == 3) launch_cs<__half, 3>(pb, blocks, n0 + z0, st); else launch_cs<__half, 1>(pb, blocks, n0 + z0, st); }
-        else { if (g.C == 3) launch_cs<__nv_bfloat16, 3>(pb, blocks, n0 + z0, st); else launch_cs<__nv_bfloat16, 1>(pb, blocks, n0 + z0, st); }
+        const bool map32 = pb.grid_dtype == PWS_F32;
+        if (pb.in_dtype == PWS_F32) launch_c<float, float>(pb, blocks, n0 + z0, st);
+        else if (pb.in_dtype == PWS_F16) { if (map32) launch_c<__half, float>(pb, blocks, n0 + z0, st); else launch_c<__half, __half>(pb, blocks, n0 + z0, st); }
+        else { if (map32) launch_c<__nv_bfloat16, float>(pb, blocks, n0 + z0, st); else launch_c<__nv_bfloat16, __nv_bfloat16>(pb, blocks, n0 + z0, st); }
     }
 }
 

@@ -3,7 +3,7 @@
 // Call sites: R/main_new.py:106,116 (NCHW frames, planar-stored maps), :197 (NCHW
 // frames, interleaved affine_grid maps), :716 (same at native video resolution).
 // Host-checked requirements: frame and output W-contiguous and 16-byte row aligned,
-// fp32 map, C in {1,3}, f32 / f16 / bf16 frames.  Everything else takes the direct
+// C in {1,3}, f32 / f16 / bf16 frames, an fp32 map or one of the frame's 16-bit type.  Everything else takes the direct
 // kernel (warp_fwd.cu).
 #include "pws_tile.cuh"
 
@@ -17,7 +17,8 @@ constexpr int kTW = 64, kTH = 32, kBW = 80, kBH = 40, kThreads = 256, kWarps = 8
 constexpr int kPX = kTW / 32, kPY = kTH / kWarps;
 
 // Layout-specialised direct gather: taps through L1 (no staging, no barrier).  4 pixels per thread, 64x16 tile.
-template <typename T, int CS, bool kBorder, bool kAlign>
+// G: map element type (float, or T for 16-bit frames); map coordinates are upcast to fp32 on load.
+template <typename T, typename G, int CS, bool kBorder, bool kAlign>
 #ifndef PWS_FWD_MINB
 #define PWS_FWD_MINB 5   // 48 registers, 40 warps/SM: measured ~7 % faster than 4 CTAs at 56 registers
 #endif
@@ -28,7 +29,7 @@ fwd_lean_kernel(const View in, const View grid, const View out, const Geometry g
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
     const int n = blockIdx.z;
     const int w_base = blockIdx.x * kTW + lane, h_base = blockIdx.y * (kWarps * PY) + wrp;
-    const float *__restrict__ gp = (const float *)grid.p + (int64_t)n * grid.sN;
+    const G *__restrict__ gp = (const G *)grid.p + (int64_t)n * grid.sN;
     const T *__restrict__ ip = (const T *)in.p + (int64_t)n * in.sN;
     T *__restrict__ op = (T *)out.p + (int64_t)n * out.sN;
     const float Wf = (float)g.W, Hf = (float)g.H, Wm1 = (float)(g.W - 1), Hm1 = (float)(g.H - 1);
@@ -37,7 +38,7 @@ fwd_lean_kernel(const View in, const View grid, const View out, const Geometry g
     float sx[PY][kPX], sy[PY][kPX];
     {
         const bool inter = grid.s3 == 1;
-        const float *__restrict__ q = gp + (int64_t)h_base * grid.s1 + (int64_t)w_base * grid.s2;
+        const G *__restrict__ q = gp + (int64_t)h_base * grid.s1 + (int64_t)w_base * grid.s2;
         const int64_t row = (int64_t)kWarps * grid.s1;
         const int col = 32 * grid.s2;
 #pragma unroll
@@ -46,13 +47,13 @@ fwd_lean_kernel(const View in, const View grid, const View out, const Geometry g
             for (int i = 0; i < kPX; ++i) {
                 sx[j][i] = -4.0f; sy[j][i] = -4.0f;
                 if (full || (w_base + 32 * i < g.Wo && h_base + kWarps * j < g.Ho)) {
-                    const float *__restrict__ a = q + j * row + i * col;
+                    const G *__restrict__ a = q + j * row + i * col;
                     if (inter) {
-                        const float2 v = __ldg(reinterpret_cast<const float2 *>(a));
+                        const float2 v = ldg_pair(a);
                         sx[j][i] = v.x; sy[j][i] = v.y;
                     } else {
-                        sx[j][i] = __ldg(a);
-                        sy[j][i] = __ldg(a + grid.s3);
+                        sx[j][i] = to_acc(ldg(a));
+                        sy[j][i] = to_acc(ldg(a + grid.s3));
                     }
                 }
             }
@@ -104,26 +105,26 @@ fwd_lean_kernel(const View in, const View grid, const View out, const Geometry g
         }
 }
 
-template <typename T, int CS>
+template <typename T, typename G, int CS>
 void launch_cs(const Problem &pb, cudaStream_t st)
 {
     const Geometry &g = pb.g;
     const bool border = g.padding == PWS_PAD_BORDER, align = g.align != 0;
     {
         dim3 lb((g.Wo + kTW - 1) / kTW, (g.Ho + 15) / 16, g.N);
-        if (border && align) { fwd_lean_kernel<T, CS, true, true><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
-        else if (border) { fwd_lean_kernel<T, CS, true, false><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
-        else if (align) { fwd_lean_kernel<T, CS, false, true><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
-        else { fwd_lean_kernel<T, CS, false, false><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
+        if (border && align) { fwd_lean_kernel<T, G, CS, true, true><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
+        else if (border) { fwd_lean_kernel<T, G, CS, true, false><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
+        else if (align) { fwd_lean_kernel<T, G, CS, false, true><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
+        else { fwd_lean_kernel<T, G, CS, false, false><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
     }
 }
 
-template <typename T>
+template <typename T, typename G>
 bool launch_t(const Problem &pb, cudaStream_t st)
 {
     if (!rows_vectorizable(pb.in, 16 / (int)sizeof(T), pb.g.W)) return false;
-    if (pb.g.C == 3) { launch_cs<T, 3>(pb, st); return true; }
-    if (pb.g.C == 1) { launch_cs<T, 1>(pb, st); return true; }
+    if (pb.g.C == 3) { launch_cs<T, G, 3>(pb, st); return true; }
+    if (pb.g.C == 1) { launch_cs<T, G, 1>(pb, st); return true; }
     return false;
 }
 
@@ -133,14 +134,14 @@ bool launch_t(const Problem &pb, cudaStream_t st)
 bool launch_forward_tile(const Problem &pb, cudaStream_t st)
 {
     const Geometry &g = pb.g;
-    if (pb.in.s3 != 1 || pb.out.s3 != 1 || pb.grid_dtype != PWS_F32) return false;
+    if (pb.in.s3 != 1 || pb.out.s3 != 1) return false;
     if (g.N > 65535 || (g.Ho + kTH - 1) / kTH > 65535) return false;
-    // interleaved maps are read as float2: needs 8-byte alignment of every pixel's pair
-    if (pb.grid.s3 == 1 && ((reinterpret_cast<uintptr_t>(pb.grid.p) & 7) || (pb.grid.sN & 1) || (pb.grid.s1 & 1) || (pb.grid.s2 & 1)))
-        return false;
-    if (pb.in_dtype == PWS_F32) return launch_t<float>(pb, st);
-    if (pb.in_dtype == PWS_F16) return launch_t<__half>(pb, st);
-    if (pb.in_dtype == PWS_BF16) return launch_t<__nv_bfloat16>(pb, st);
+    const bool map32 = pb.grid_dtype == PWS_F32;
+    if (!map32 && pb.grid_dtype != pb.in_dtype) return false;
+    if (!map_pairs_ok(pb.grid, map32 ? 4 : 2)) return false;
+    if (pb.in_dtype == PWS_F32) return map32 && launch_t<float, float>(pb, st);
+    if (pb.in_dtype == PWS_F16) return map32 ? launch_t<__half, float>(pb, st) : launch_t<__half, __half>(pb, st);
+    if (pb.in_dtype == PWS_BF16) return map32 ? launch_t<__nv_bfloat16, float>(pb, st) : launch_t<__nv_bfloat16, __nv_bfloat16>(pb, st);
     return false;
 }
 

@@ -116,7 +116,7 @@ def warp2d_backward(grad_output: torch.Tensor, input: torch.Tensor, grid: torch.
     """aten::grid_sampler_2d_backward replacement. Returns (grad_input | None, grad_grid | None);
     caller-provided buffers are filled when given (grad_input need not be zeroed)."""
     lib = _lib.load()
-    half_frames = grid.dtype != input.dtype      # 16-bit frames with an fp32 map (BASELINE config 5)
+    half_frames = input.dtype in (torch.float16, torch.bfloat16)     # with an fp32 map or one of the frame's type
     gin = ggrid = None
     if output_mask[0]:
         if half_frames:
