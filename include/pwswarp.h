@@ -81,8 +81,8 @@ const char *pws_last_error(void);
 uint64_t pws_launch_count(void);
 
 /* Debug / tests: name of the kernel family the last forward / backward call on THIS thread launched
- * ("fwd_tma", "fwd_lean", "fwd_direct", "bwd_tma", "bwd_lean", "bwd_march", "bwd_lean_16", "bwd_march_16", "fused",
- * ...; "" before any call). */
+ * ("fwd_tma", "fwd_lean", "fwd_direct", "bwd_tma", "bwd_lean", "bwd_march", "bwd_lean_16", "bwd_march_16", "fwd_fused",
+ * "stages_fwd", "stages_fwd_16", ...; "" before any call). */
 const char *pws_last_kernel(void);
 
 /* Tuning knob (process-wide, like a library's "benchmark" switch; results do not depend on it): calls whose output has at
@@ -148,7 +148,8 @@ enum { PWS_BASE_NONE = 0, PWS_BASE_IDENTITY = 1, PWS_BASE_AFFINE = 2 };
 enum { PWS_UP_NONE = 0, PWS_UP_ALIGNED = 1, PWS_UP_HALF_PIXEL = 2 };
 
 typedef struct pws_map_spec {
-    const pws_tensor *drift; /* (N, map_h, map_w, 2) f32 view, any strides; NULL = zero drift */
+    const pws_tensor *drift; /* (N, map_h, map_w, 2) f32, f16 or bf16 view, any strides; NULL = zero drift.  A 16-bit
+                                drift is upcast exactly: results equal those of the same call with its f32 copy */
     const float *theta;      /* (N,2,3) f32 contiguous device memory; PWS_BASE_AFFINE only */
     int32_t base;
     int32_t base_align_corners;
@@ -162,7 +163,7 @@ typedef struct pws_map_spec {
 int pws_warp2d_forward_fused(const pws_tensor *in, const pws_map_spec *spec, pws_tensor *out,
                              int padding, int align_corners, void *stream);
 
-/* Debug / parity: writes the map the fused kernel uses into map_out (N,Ho,Wo,2) f32. */
+/* Debug / parity: writes the map the fused kernel uses into map_out (N,Ho,Wo,2) f32 (also for a 16-bit drift). */
 int pws_compose_map(const pws_map_spec *spec, int64_t n, pws_tensor *map_out, void *stream);
 
 /* ---- K maps, one frame, one launch (SURVEY.md 8(a) rows a8, a11; north_star "map composition across cascade
@@ -174,9 +175,21 @@ int pws_compose_map(const pws_map_spec *spec, int64_t n, pws_tensor *map_out, vo
  *     outs[k]   = sample((in + pre_add) * pre_mul, grids[k]) * (1 / post_div) + post_add        k < n_stages <= 4
  *     ggrids[k] = d outs[k] / d grids[k] applied to gouts[k]      (entries may be NULL)
  *     gin       = sum_k d outs[k] / d in applied to gouts[k]      (may be NULL; dense NCHW, zero-filled by the library)
- * f32 frames and maps, C in {1, 3}, any strides.  `1 / post_div` is the rounded fp32 reciprocal torch's
- * `tensor / scalar` multiplies by, so the results equal the reference's sequence of torch calls bit for bit.
- * (0, 1, 1, 0) switches the scales off. */
+ * C in {1, 3}, any strides.  `1 / post_div` is the rounded fp32 reciprocal torch's `tensor / scalar` multiplies by, so
+ * the results equal the reference's sequence of torch calls bit for bit.  (0, 1, 1, 0) switches the scales off.
+ * dtypes (all grids share one dtype; anything else is PWS_EINVAL):
+ *     in / outs / gouts   grids / ggrids     gin
+ *     f32                 f32                f32
+ *     f16 | bf16          f32                f32 accumulation buffer
+ *     f16 | bf16          the frame's        f32 accumulation buffer
+ * For 16-bit frames the results equal that sequence evaluated by torch on tensors of the frame's type, where every
+ * elementwise op computes in fp32 and rounds to the type (round_T):
+ *     tap  = round_T(round_T(x + pre_add) * pre_mul)                 (pre scale on)
+ *     s    = round_T(fp32 bilinear sample of the taps, ATen's order)
+ *     out  = round_T(round_T(s * (1 / post_div)) + post_add)          (post scale on)
+ * The backward is that sequence's autograd through pws_warp2d_backward: go = round_T(gout * (1 / post_div)), fp32
+ * arithmetic on the rounded taps, ggrid rounded once to the map's type; gin holds the exact fp32 sums (times pre_mul,
+ * over all stages), which the caller rounds to the frame type once. */
 int pws_warp2d_stages_forward(const pws_tensor *in, const pws_tensor *const *grids, pws_tensor *const *outs, int n_stages,
                               float pre_add, float pre_mul, float post_div, float post_add,
                               int padding, int align_corners, void *stream);

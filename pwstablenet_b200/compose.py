@@ -23,6 +23,7 @@ from .functional import _PADDING, _stream
 _BASE = {"none": _lib.PWS_BASE_NONE, "identity": _lib.PWS_BASE_IDENTITY, "affine": _lib.PWS_BASE_AFFINE}
 _UP = {None: _lib.PWS_UP_NONE, "none": _lib.PWS_UP_NONE, "aligned": _lib.PWS_UP_ALIGNED, "half_pixel": _lib.PWS_UP_HALF_PIXEL}
 _DT = {torch.float32: _lib.PWS_F32, torch.float16: _lib.PWS_F16, torch.bfloat16: _lib.PWS_BF16, torch.uint8: _lib.PWS_U8}
+_LATTICE_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
 
 
 def _desc(t: torch.Tensor) -> _lib.PwsTensor:
@@ -39,8 +40,8 @@ def _desc(t: torch.Tensor) -> _lib.PwsTensor:
 def _spec(n, drift, base, theta, base_align_corners, upsample, map_size, pre, post, keep):
     s = _lib.PwsMapSpec()
     if drift is not None:
-        if not (drift.is_cuda and drift.dtype == torch.float32 and drift.dim() == 4 and drift.size(3) == 2 and drift.size(0) == n):
-            raise RuntimeError("warp_fused: drift must be a float32 CUDA tensor of sizes (N, h, w, 2) "
+        if not (drift.is_cuda and drift.dtype in _LATTICE_DTYPES and drift.dim() == 4 and drift.size(3) == 2 and drift.size(0) == n):
+            raise RuntimeError("warp_fused: drift must be a float32, float16 or bfloat16 CUDA tensor of sizes (N, h, w, 2) "
                                "(pass netG's planar (N,2,h,w) output as drift.permute(0,2,3,1))")
         d = _desc(drift)
         keep.append(d)
@@ -66,7 +67,8 @@ def _spec(n, drift, base, theta, base_align_corners, upsample, map_size, pre, po
 def compose_map(n: int, out_size: Tuple[int, int], drift: Optional[torch.Tensor] = None, base: str = "none",
                 theta: Optional[torch.Tensor] = None, base_align_corners: bool = False, upsample: Optional[str] = None,
                 map_size: Optional[Tuple[int, int]] = None, device=None) -> torch.Tensor:
-    """The (N, Ho, Wo, 2) float32 map the fused kernel samples with (debug / parity)."""
+    """The (N, Ho, Wo, 2) float32 map the fused kernel samples with (debug / parity).  A 16-bit drift is upcast exactly, so
+    the map equals the one composed from drift.float()."""
     lib = _lib.load()
     keep = []
     spec = _spec(n, drift, base, theta, base_align_corners, upsample, map_size, (0.0, 1.0), (1.0, 0.0), keep)
@@ -89,7 +91,13 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
 
     frame:  (N,C,H,W) view, float32/16-bit float or uint8, any strides (a cv2 HWC buffer is
             `buf.permute(0,3,1,2)`).
-    drift:  (N,h,w,2) float32 view (netG's planar output permuted), or None.
+    drift:  (N,h,w,2) view (netG's planar output permuted), or None.  float32, or the float16 / bfloat16 lattice of a
+            half-precision netG: it is upcast exactly and everything after that is fp32, so the result equals the same
+            call with drift.float() bit for bit.  A 16-bit lattice is coarse at 1080p: for |x| in [0.5, 1) an f16
+            coordinate steps by 2**-11 (about 0.5 px at a width of 1920), a bf16 one by 2**-8 (about 3.75 px), and the
+            upsample interpolates between those values (DESIGN.md section 3.8).  That coarseness is in netG's output,
+            not in this call.
+    theta:  (N,2,3) float32.
     base:   'none' | 'identity' (generate_maps) | 'affine' (affine_grid(theta, base_align_corners)).
     upsample: None | 'aligned' (UpsamplingBilinear2d) | 'half_pixel' (nn.Upsample bilinear); needs out_size.
     pre=(a,b): frame' = (frame+a)*b.   post=(d,e): out = acc/d + e.
@@ -115,8 +123,9 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
         base, theta = "none", None
     if upsample is not None and drift is not None and base == "none" and not drift.is_contiguous():
         # netG hands its map over as a permuted view of planar storage (R/lib/networks_cascading.py:235-237); the
-        # specialised inference kernel reads an interleaved lattice with 8-byte loads.  Repacking 0.5 MB per frame is
-        # nothing next to the frame; the values, hence the result, are the same.
+        # specialised inference kernel reads an interleaved lattice with one load per node (8 bytes, 4 for a 16-bit
+        # lattice, whose dtype the repack keeps).  Repacking 0.5 MB per frame is nothing next to the frame; the values,
+        # hence the result, are the same.
         drift = drift.contiguous()
     spec = _spec(n, drift, base, theta, base_align_corners, upsample, map_size, pre, post, keep)
     if out_size is None:
@@ -134,6 +143,9 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
 
 
 # ---- K maps, one frame, one launch: forward + backward (include/pwswarp.h, csrc/warp_stages.cu) ---------------------
+_STAGE_FRAMES = (torch.float32, torch.float16, torch.bfloat16)
+
+
 def _desc_ptrs(tensors, keep):
     arr = (ctypes.POINTER(_lib.PwsTensor) * len(tensors))()
     for i, t in enumerate(tensors):
@@ -172,7 +184,9 @@ class _WarpStages(torch.autograd.Function):
         gouts = [g if g is not None else torch.zeros((frame.size(0), frame.size(1), grids[i].size(1), grids[i].size(2)),
                                                      dtype=frame.dtype, device=frame.device) for i, g in enumerate(gouts)]
         from .functional import _like_layout
-        gin = torch.empty(frame.size(), dtype=frame.dtype, device=frame.device) if ctx.needs_input_grad[0] else None
+        # grad_input is an fp32 buffer for every frame type: 16-bit frames sum their contributions in fp32 and are rounded
+        # to the frame type once, below (as functional.warp2d_backward does)
+        gin = torch.empty(frame.size(), dtype=torch.float32, device=frame.device) if ctx.needs_input_grad[0] else None
         ggrids = [_like_layout(grids[i]) if ctx.needs_input_grad[7 + i] else None for i in range(k)]
         keep = []
         with torch.cuda.device_of(frame):
@@ -180,6 +194,8 @@ class _WarpStages(torch.autograd.Function):
                                                 ctypes.byref(_desc(gin)) if gin is not None else None, _desc_ptrs(ggrids, keep), k,
                                                 pre_add, pre_mul, post_div, post_add, padding, int(align_corners), _stream(frame))
         _lib.check(rc)
+        if gin is not None and gin.dtype != frame.dtype:
+            gin = gin.to(frame.dtype)
         return (gin, None, None, None, None, None, None, *ggrids)
 
 
@@ -189,16 +205,29 @@ def warp_stages(frame: torch.Tensor, grids, padding_mode: str = "zeros", align_c
     in ONE kernel launch that reads the frame once, with autograd to every map (and to the frame when it asks for it).
 
     The reference's per-stage loop R/main_new.py:103-110: `warp_stages(rgb, grid1, pre=(1, 127.5), post=(127.5, -1))`.
-    Up to 4 maps; f32, C in {1, 3}.  Values and gradients are bit-identical to the sequence of torch calls it replaces."""
+    Up to 4 maps, C in {1, 3}, any strides.  Values and map gradients are bit-identical to the sequence of torch calls it
+    replaces, with pw.grid_sample as the sampler.
+
+    dtypes (what a half-precision netG hands over):
+        frame            maps (all one dtype)      outputs, grad_grids
+        float32          float32                   float32
+        float16/bfloat16 float32 or the frame's    the frame's dtype; each grad_grid in its map's dtype and layout
+    With a 16-bit frame every elementwise op of that sequence rounds to the frame type, as torch does on a half-precision
+    tensor (fp32 arithmetic, one rounding per op), and the kernel reproduces each rounding: the pre-scaled taps, the
+    sample, `/ post[0]` and `+ post[1]`.  grad_input is summed in fp32 and rounded to the frame type once."""
     grids = list(grids)
     if not 1 <= len(grids) <= 4:
         raise ValueError("warp_stages: 1 to 4 maps")
     if padding_mode not in ("zeros", "border"):
         raise NotImplementedError("warp_stages: padding_mode must be 'zeros' or 'border'")
-    if not frame.is_cuda or frame.dtype != torch.float32 or frame.dim() != 4:
-        raise RuntimeError("warp_stages: frame must be a 4-D float32 CUDA tensor (no CPU fallback)")
+    if not frame.is_cuda or frame.dtype not in _STAGE_FRAMES or frame.dim() != 4:
+        raise RuntimeError("warp_stages: frame must be a 4-D float32, float16 or bfloat16 CUDA tensor (no CPU fallback)")
+    map_dtypes = (torch.float32,) if frame.dtype == torch.float32 else (torch.float32, frame.dtype)
     for g in grids:
-        if not g.is_cuda or g.dtype != torch.float32 or g.dim() != 4 or g.size(3) != 2 or g.size(0) != frame.size(0):
-            raise RuntimeError("warp_stages: every map must be a float32 CUDA tensor of sizes (N, Ho, Wo, 2)")
+        if not g.is_cuda or g.dtype not in map_dtypes or g.dim() != 4 or g.size(3) != 2 or g.size(0) != frame.size(0):
+            raise RuntimeError(f"warp_stages: every map must be a CUDA tensor of sizes (N, Ho, Wo, 2) and dtype "
+                               f"{' or '.join(str(d) for d in map_dtypes)} for a {frame.dtype} frame")
+    if any(g.dtype != grids[0].dtype for g in grids):
+        raise RuntimeError("warp_stages: all maps must have one dtype, got " + ", ".join(str(g.dtype) for g in grids))
     return _WarpStages.apply(frame, _PADDING[padding_mode], bool(align_corners), float(pre[0]), float(pre[1]),
                              float(post[0]), float(post[1]), *grids)

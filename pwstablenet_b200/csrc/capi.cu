@@ -172,6 +172,23 @@ static int make_scale(float pre_add, float pre_mul, float post_div, float post_a
     return PWS_OK;
 }
 
+// warp_stages dtype matrix: f32 frames with f32 maps; f16 / bf16 frames with f32 maps or maps of the frame's type; one map
+// dtype for all stages.  Outputs and grad_outputs have the frame's dtype, grad_grids the maps'.
+static int check_stage_dtypes(const pws_tensor *in, const pws_tensor *const *grids, int n_stages, const char *what)
+{
+    const bool half_in = in->dtype == PWS_F16 || in->dtype == PWS_BF16;
+    if (in->dtype != PWS_F32 && !half_in) { set_error("%s: frames must be f32, f16 or bf16", what); return PWS_EUNSUPPORTED; }
+    for (int k = 0; k < n_stages; ++k) {
+        if (!grids[k]) { set_error("grid_sampler(): expected input and grid to not be undefined"); return PWS_EINVAL; }
+        if (grids[k]->dtype != grids[0]->dtype) { set_error("%s: all maps must have one dtype (map 0: %d, map %d: %d)", what, grids[0]->dtype, k, grids[k]->dtype); return PWS_EINVAL; }
+    }
+    if (grids[0]->dtype != in->dtype && !(half_in && grids[0]->dtype == PWS_F32)) {
+        set_error("%s: maps must be f32 or the frame's dtype (frame %d, maps %d)", what, in->dtype, grids[0]->dtype);
+        return PWS_EINVAL;
+    }
+    return PWS_OK;
+}
+
 int launch_forward_fused(const View &in, int in_dtype, const MapSpec &m, const View &out, int out_dtype,
                          const Geometry &g, cudaStream_t st);
 int launch_compose_map(const MapSpec &m, const View &out, int N, int Ho, int Wo, cudaStream_t st);
@@ -182,8 +199,11 @@ static int make_spec(const pws_map_spec *spec, int64_t N, int64_t Ho, int64_t Wo
     if (spec->base < 0 || spec->base > 2 || spec->upsample < 0 || spec->upsample > 2) { set_error("map spec: bad base/upsample enum"); return PWS_EINVAL; }
     if (spec->map_h <= 0 || spec->map_w <= 0 || spec->map_h > INT_MAX || spec->map_w > INT_MAX) { set_error("map spec: bad lattice size"); return PWS_EINVAL; }
     m->drift.p = nullptr; m->drift.sN = 0; m->drift.s1 = m->drift.s2 = m->drift.s3 = 0;
+    m->drift_dtype = PWS_F32;
     if (spec->drift) {
-        if (spec->drift->dtype != PWS_F32) { set_error("map spec: drift must be f32"); return PWS_EUNSUPPORTED; }
+        const int dt = spec->drift->dtype;
+        if (dt != PWS_F32 && dt != PWS_F16 && dt != PWS_BF16) { set_error("map spec: drift must be f32, f16 or bf16"); return PWS_EUNSUPPORTED; }
+        m->drift_dtype = dt;
         if (spec->drift->size[0] != N || spec->drift->size[1] != spec->map_h || spec->drift->size[2] != spec->map_w || spec->drift->size[3] != 2) {
             set_error("map spec: drift must have sizes [N, map_h, map_w, 2]"); return PWS_EINVAL;
         }
@@ -374,7 +394,7 @@ int pws_warp2d_stages_forward(const pws_tensor *in, const pws_tensor *const *gri
     PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
     if (!in || !grids || !outs) { set_error("stages forward: null argument"); return PWS_EINVAL; }
     if (n_stages < 1 || n_stages > kMaxStages) { set_error("stages forward: n_stages must be 1..%d", kMaxStages); return PWS_EINVAL; }
-    if (in->dtype != PWS_F32) { set_error("stages forward: f32 frames only"); return PWS_EUNSUPPORTED; }
+    PWS_TRY(check_stage_dtypes(in, grids, n_stages, "stages forward"));
     View vin;
     PWS_TRY(make_view(in, "input", &vin));
     StageViews sv{};
@@ -382,7 +402,7 @@ int pws_warp2d_stages_forward(const pws_tensor *in, const pws_tensor *const *gri
     for (int k = 0; k < n_stages; ++k) {
         PWS_TRY(check_pair(in, grids[k]));
         if (!outs[k]) { set_error("stages forward: null output %d", k); return PWS_EINVAL; }
-        if (grids[k]->dtype != PWS_F32 || outs[k]->dtype != PWS_F32) { set_error("stages forward: f32 maps and outputs only"); return PWS_EUNSUPPORTED; }
+        if (outs[k]->dtype != in->dtype) { set_error("stages forward: output %d: dtype must equal the input's", k); return PWS_EINVAL; }
         if (k && (grids[k]->size[1] != grids[0]->size[1] || grids[k]->size[2] != grids[0]->size[2])) { set_error("stages forward: all maps must have the same size"); return PWS_EINVAL; }
         PWS_TRY(make_view(grids[k], "grid", &sv.map[k]));
         PWS_TRY(make_view(outs[k], "output", &sv.io[k]));
@@ -395,7 +415,7 @@ int pws_warp2d_stages_forward(const pws_tensor *in, const pws_tensor *const *gri
     if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0) return PWS_OK;
     DeviceGuard dg(in->device);
     if (!dg.ok) { set_error("stages forward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    PWS_TRY(launch_stages_forward(vin, sv, n_stages, g, sc, (cudaStream_t)stream));
+    PWS_TRY(launch_stages_forward(vin, in->dtype, sv, grids[0]->dtype, n_stages, g, sc, (cudaStream_t)stream));
     return finish("stages forward");
 }
 
@@ -408,7 +428,7 @@ int pws_warp2d_stages_backward(const pws_tensor *const *gouts, const pws_tensor 
     PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
     if (!in || !grids || !gouts || !ggrids) { set_error("stages backward: null argument"); return PWS_EINVAL; }
     if (n_stages < 1 || n_stages > kMaxStages) { set_error("stages backward: n_stages must be 1..%d", kMaxStages); return PWS_EINVAL; }
-    if (in->dtype != PWS_F32) { set_error("stages backward: f32 frames only"); return PWS_EUNSUPPORTED; }
+    PWS_TRY(check_stage_dtypes(in, grids, n_stages, "stages backward"));
     View vin, vgin{};
     PWS_TRY(make_view(in, "input", &vin));
     StageViews sv{};
@@ -416,13 +436,15 @@ int pws_warp2d_stages_backward(const pws_tensor *const *gouts, const pws_tensor 
     for (int k = 0; k < n_stages; ++k) {
         PWS_TRY(check_pair(in, grids[k]));
         if (!gouts[k]) { set_error("stages backward: null grad_output %d", k); return PWS_EINVAL; }
-        if (grids[k]->dtype != PWS_F32 || gouts[k]->dtype != PWS_F32) { set_error("stages backward: f32 only"); return PWS_EUNSUPPORTED; }
+        if (gouts[k]->dtype != in->dtype) { set_error("stages backward: grad_output %d: dtype must equal the input's", k); return PWS_EINVAL; }
+        if (gouts[k]->device != in->device) { set_error("stages backward: grad_output %d: must be on the input's device", k); return PWS_EINVAL; }
         if (k && (grids[k]->size[1] != grids[0]->size[1] || grids[k]->size[2] != grids[0]->size[2])) { set_error("stages backward: all maps must have the same size"); return PWS_EINVAL; }
         PWS_TRY(make_view(grids[k], "grid", &sv.map[k]));
         PWS_TRY(make_view(gouts[k], "grad_output", &sv.io[k]));
         PWS_TRY(same_shape(gouts[k], in->size[0], in->size[1], grids[k]->size[1], grids[k]->size[2], "grad_output"));
         if (ggrids[k]) {
-            if (ggrids[k]->dtype != PWS_F32) { set_error("stages backward: f32 grad_grid only"); return PWS_EUNSUPPORTED; }
+            if (ggrids[k]->dtype != grids[k]->dtype) { set_error("stages backward: grad_grid %d: dtype must equal the map's", k); return PWS_EINVAL; }
+            if (ggrids[k]->device != in->device) { set_error("stages backward: grad_grid %d: must be on the input's device", k); return PWS_EINVAL; }
             PWS_TRY(make_view(ggrids[k], "grad_grid", &sv.gg[k]));
             PWS_TRY(same_shape(ggrids[k], grids[k]->size[0], grids[k]->size[1], grids[k]->size[2], 2, "grad_grid"));
         }
@@ -433,7 +455,11 @@ int pws_warp2d_stages_backward(const pws_tensor *const *gouts, const pws_tensor 
         const int64_t C = in->size[1], H = in->size[2], W = in->size[3];
         const bool dense = gin->dtype == PWS_F32 && gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
                            (gin->stride[0] == C * H * W || in->size[0] <= 1);
-        if (!dense) { set_error("grad_input: must be f32 (N,C,H,W)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
+        if (!dense) {
+            set_error("grad_input: must be f32 (N,C,H,W)-contiguous (the library zero-fills it; 16-bit frames accumulate in fp32)");
+            return PWS_EINVAL;
+        }
+        if (gin->device != in->device) { set_error("stages backward: grad_input must be on the input's device"); return PWS_EINVAL; }
         vgin.sN = C * H * W;
     }
     fill_geometry(in, grids[0], padding, align_corners, &g);
@@ -443,10 +469,13 @@ int pws_warp2d_stages_backward(const pws_tensor *const *gouts, const pws_tensor 
     if (!dg.ok) { set_error("stages backward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
     if (g.N == 0) return PWS_OK;
     if ((int64_t)g.C * g.Ho * g.Wo == 0) {
-        if (gin && (int64_t)g.C * g.H * g.W > 0) cudaMemsetAsync(gin->data, 0, (size_t)(in->size[0] * vgin.sN * 4), (cudaStream_t)stream);
+        if (gin && (int64_t)g.C * g.H * g.W > 0) {
+            cudaError_t e = cudaMemsetAsync(gin->data, 0, (size_t)(in->size[0] * vgin.sN * 4), (cudaStream_t)stream);
+            if (e != cudaSuccess) { set_error("stages backward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return PWS_ECUDA; }
+        }
         return PWS_OK;
     }
-    PWS_TRY(launch_stages_backward(vin, sv, n_stages, vgin, gin != nullptr, g, sc, (cudaStream_t)stream));
+    PWS_TRY(launch_stages_backward(vin, in->dtype, sv, grids[0]->dtype, n_stages, vgin, gin != nullptr, g, sc, (cudaStream_t)stream));
     return finish("stages backward");
 }
 

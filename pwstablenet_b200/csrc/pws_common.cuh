@@ -158,7 +158,7 @@ struct Problem {  // validated, kernel-ready description of one call
 };
 
 struct MapSpec {  // kernel-side form of pws_map_spec (warp_fused.cu)
-    View drift;          // (N, mh, mw, 2) fp32; p == nullptr: zero drift
+    View drift;          // (N, mh, mw, 2) of drift_dtype; p == nullptr: zero drift
     const float *theta;  // (N,2,3) for the affine base
     int base;            // PWS_BASE_*
     int base_align;      // align_corners of affine_grid
@@ -166,6 +166,7 @@ struct MapSpec {  // kernel-side form of pws_map_spec (warp_fused.cu)
     int mh, mw;          // map lattice size
     float pre_add, pre_mul, post_div, post_add;
     int has_pre, has_post;
+    int drift_dtype;     // PWS_F32 / PWS_F16 / PWS_BF16 (host dispatch only)
 };
 
 // K maps applied to one frame (warp_stages.cu)
@@ -179,9 +180,11 @@ struct StageScale {
     float pre_add, pre_mul, post_mul, post_add;
     int has_pre, has_post;
 };
-int launch_stages_forward(const View &in, const StageViews &sv, int K, const Geometry &g, const StageScale &sc, cudaStream_t st);
-int launch_stages_backward(const View &in, const StageViews &sv, int K, const View &gin, bool want_gin, const Geometry &g,
-                           const StageScale &sc, cudaStream_t st);
+// in_dtype: f32 / f16 / bf16; map_dtype: f32 or in_dtype (one dtype for all K maps); gin is f32 for every frame type
+int launch_stages_forward(const View &in, int in_dtype, const StageViews &sv, int map_dtype, int K, const Geometry &g,
+                          const StageScale &sc, cudaStream_t st);
+int launch_stages_backward(const View &in, int in_dtype, const StageViews &sv, int map_dtype, int K, const View &gin, bool want_gin,
+                           const Geometry &g, const StageScale &sc, cudaStream_t st);
 
 // Calls whose whole working set sits in L2 (the reference's training shapes: 16 x 3 x 256 x 256 = 12.6 MB) are bound by the
 // launch, not by HBM: they take the plain one-wave kernels (no tensor maps to encode, no counter slot to lease, no

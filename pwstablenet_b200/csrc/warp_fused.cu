@@ -33,18 +33,20 @@ __device__ __forceinline__ float lattice_base(int i, int S, int base, int align)
     return v;
 }
 
-// map value at lattice point (i, j) of item n:  drift + base
+// map value at lattice point (i, j) of item n:  drift + base.  L: the drift's element type (float, or the __half /
+// __nv_bfloat16 lattice of a half-precision netG); the upcast is exact and everything after it is fp32.
+template <typename L>
 __device__ __forceinline__ void lattice_map(const MapSpec &m, int n, int i, int j, float &mx, float &my)
 {
     float dx = 0.f, dy = 0.f;
     if (m.drift.p) {
-        const float *d = (const float *)m.drift.p + (int64_t)n * m.drift.sN + i * m.drift.s1 + j * m.drift.s2;
-        // interleaved (x,y) pairs -- the lattice the host side composes -- come as one 8-byte load
-        if (m.drift.s3 == 1 && !((reinterpret_cast<uintptr_t>(m.drift.p) & 7) | ((m.drift.sN | m.drift.s1 | m.drift.s2) & 1))) {
-            const float2 v = __ldg(reinterpret_cast<const float2 *>(d));
+        const L *d = (const L *)m.drift.p + (int64_t)n * m.drift.sN + i * m.drift.s1 + j * m.drift.s2;
+        // interleaved (x,y) pairs -- the lattice the host side composes -- come as one 8-byte (fp32) or 4-byte (16-bit) load
+        if (m.drift.s3 == 1 && !((reinterpret_cast<uintptr_t>(m.drift.p) & (2 * sizeof(L) - 1)) | ((m.drift.sN | m.drift.s1 | m.drift.s2) & 1))) {
+            const float2 v = ldg_pair(d);
             dx = v.x; dy = v.y;
         } else {
-            dx = __ldg(d); dy = __ldg(d + m.drift.s3);
+            dx = to_acc(ldg(d)); dy = to_acc(ldg(d + m.drift.s3));
         }
     }
     if (m.base == PWS_BASE_NONE) { mx = dx; my = dy; return; }
@@ -72,24 +74,26 @@ __device__ __forceinline__ UpCoef up_coef(int dst, int src_size, float scale, bo
 }
 
 // the upsampled map from the row / column coefficients of an output pixel
+template <typename L>
 __device__ __forceinline__ void map_up(const MapSpec &m, int n, const UpCoef &cy, const UpCoef &cx, float &gx, float &gy)
 {
     float x00, y00, x01, y01, x10, y10, x11, y11;
-    lattice_map(m, n, cy.i0, cx.i0, x00, y00);
-    lattice_map(m, n, cy.i0, cx.i0 + cx.ip, x01, y01);
-    lattice_map(m, n, cy.i0 + cy.ip, cx.i0, x10, y10);
-    lattice_map(m, n, cy.i0 + cy.ip, cx.i0 + cx.ip, x11, y11);
+    lattice_map<L>(m, n, cy.i0, cx.i0, x00, y00);
+    lattice_map<L>(m, n, cy.i0, cx.i0 + cx.ip, x01, y01);
+    lattice_map<L>(m, n, cy.i0 + cy.ip, cx.i0, x10, y10);
+    lattice_map<L>(m, n, cy.i0 + cy.ip, cx.i0 + cx.ip, x11, y11);
     // h0*(w0*v00 + w1*v01) + h1*(w0*v10 + w1*v11), contracted as nvcc contracts ATen's expression
     gx = __fmaf_rn(cy.l0, __fmaf_rn(cx.l0, x00, __fmul_rn(cx.l1, x01)), __fmul_rn(cy.l1, __fmaf_rn(cx.l0, x10, __fmul_rn(cx.l1, x11))));
     gy = __fmaf_rn(cy.l0, __fmaf_rn(cx.l0, y00, __fmul_rn(cx.l1, y01)), __fmul_rn(cy.l1, __fmaf_rn(cx.l0, y10, __fmul_rn(cx.l1, y11))));
 }
 
 // the map the sampler sees at output pixel (h, w)
+template <typename L>
 __device__ __forceinline__ void map_at(const MapSpec &m, int n, int h, int w, float rh, float rw, float &gx, float &gy)
 {
-    if (m.upsample == PWS_UP_NONE) { lattice_map(m, n, h, w, gx, gy); return; }
+    if (m.upsample == PWS_UP_NONE) { lattice_map<L>(m, n, h, w, gx, gy); return; }
     const bool al = m.upsample == PWS_UP_ALIGNED;
-    map_up(m, n, up_coef(h, m.mh, rh, al), up_coef(w, m.mw, rw, al), gx, gy);
+    map_up<L>(m, n, up_coef(h, m.mh, rh, al), up_coef(w, m.mw, rw, al), gx, gy);
 }
 
 __device__ __forceinline__ void up_scales(const MapSpec &m, int Ho, int Wo, float &rh, float &rw)
@@ -125,7 +129,12 @@ template <> __device__ __forceinline__ void store_px<uint8_t>(uint8_t *p, float 
 
 constexpr int kTileW = 64, kTileH = 16, kThreads = 256;
 
-template <typename TI, typename TO, int CS>
+// a lattice node read as one vector, upcast (exact)
+__device__ __forceinline__ float2 node_f2(float2 v) { return v; }
+__device__ __forceinline__ float2 node_f2(__half2 v) { return __half22float2(v); }
+__device__ __forceinline__ float2 node_f2(__nv_bfloat162 v) { return __bfloat1622float2(v); }
+
+template <typename TI, typename TO, typename L, int CS>
 __global__ void __launch_bounds__(kThreads)
 fwd_fused_kernel(const View in, const MapSpec m, const View out, const Geometry g)
 {
@@ -146,7 +155,7 @@ fwd_fused_kernel(const View in, const MapSpec m, const View out, const Geometry 
             for (int i = 0; i < 2; ++i) {
                 const int w = blockIdx.x * kTileW + lane + 32 * i, h = blockIdx.y * kTileH + wrp + 8 * j;
                 gx[j][i] = 0.f; gy[j][i] = 0.f;
-                if (w < g.Wo && h < g.Ho) lattice_map(m, n, h, w, gx[j][i], gy[j][i]);
+                if (w < g.Wo && h < g.Ho) lattice_map<L>(m, n, h, w, gx[j][i], gy[j][i]);
             }
     } else {
         // a thread's four pixels share two rows and two columns: two row and two column coefficient sets
@@ -159,7 +168,7 @@ fwd_fused_kernel(const View in, const MapSpec m, const View out, const Geometry 
 #pragma unroll
         for (int j = 0; j < 2; ++j)
 #pragma unroll
-            for (int i = 0; i < 2; ++i) map_up(m, n, cy[j], cx[i], gx[j][i], gy[j][i]);
+            for (int i = 0; i < 2; ++i) map_up<L>(m, n, cy[j], cx[i], gx[j][i], gy[j][i]);
     }
 #pragma unroll
     for (int j = 0; j < 2; ++j)
@@ -198,17 +207,20 @@ fwd_fused_kernel(const View in, const MapSpec m, const View out, const Geometry 
 // is the bilinear upsample of a dense interleaved low-resolution lattice (what the host side composes once per call).
 // Same arithmetic as the generic kernel above, statement for statement -- only the addressing is compile-time: the
 // generic kernel spends 390 instructions per pixel, most of them on run-time strides and layout checks, and is
-// issue-bound (79 % of the issue slots).
-template <bool kBorder, bool kAlignCorners, bool kUpAligned>
-__global__ void __launch_bounds__(kThreads)
-fwd_fused_u8_kernel(const uint8_t *__restrict__ in, const float2 *__restrict__ lattice, uint8_t *__restrict__ out,
+// issue-bound (79 % of the issue slots).  LP: one lattice node, float2 or the __half2 / __nv_bfloat162 of a 16-bit lattice.
+// Without a minimum-blocks hint ptxas caps the kUpAligned instantiations at 32 registers and spills 8 bytes; the 16-bit
+// ones ask for one block per SM and get 66-72 registers, no spill (the fp32 ones keep the code they have always had).
+template <typename LP> constexpr int kU8MinBlocks = sizeof(LP) == 8 ? 0 : 1;
+template <typename LP, bool kBorder, bool kAlignCorners, bool kUpAligned>
+__global__ void __launch_bounds__(kThreads, kU8MinBlocks<LP>)
+fwd_fused_u8_kernel(const uint8_t *__restrict__ in, const LP *__restrict__ lattice, uint8_t *__restrict__ out,
                     const int H, const int W, const int Ho, const int Wo, const int mh, const int mw, const float rh, const float rw)
 {
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
     const int n = blockIdx.z;
     const uint8_t *__restrict__ ip = in + (int64_t)n * H * W * 3;
     uint8_t *__restrict__ op = out + (int64_t)n * Ho * Wo * 3;
-    const float2 *__restrict__ L = lattice + (int64_t)n * mh * mw;
+    const LP *__restrict__ L = lattice + (int64_t)n * mh * mw;
     const int padding = kBorder ? PWS_PAD_BORDER : PWS_PAD_ZEROS;
 
     UpCoef cy[2], cx[2];
@@ -222,8 +234,8 @@ fwd_fused_u8_kernel(const uint8_t *__restrict__ in, const float2 *__restrict__ l
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             if (!(ww[i] < Wo && hh[j] < Ho)) continue;
-            const float2 *r0 = L + cy[j].i0 * mw + cx[i].i0, *r1 = r0 + cy[j].ip * mw;
-            const float2 v00 = __ldg(r0), v01 = __ldg(r0 + cx[i].ip), v10 = __ldg(r1), v11 = __ldg(r1 + cx[i].ip);
+            const LP *r0 = L + cy[j].i0 * mw + cx[i].i0, *r1 = r0 + cy[j].ip * mw;
+            const float2 v00 = node_f2(__ldg(r0)), v01 = node_f2(__ldg(r0 + cx[i].ip)), v10 = node_f2(__ldg(r1)), v11 = node_f2(__ldg(r1 + cx[i].ip));
             // h0*(w0*v00 + w1*v01) + h1*(w0*v10 + w1*v11), contracted as in map_up()
             const float gx = __fmaf_rn(cy[j].l0, __fmaf_rn(cx[i].l0, v00.x, __fmul_rn(cx[i].l1, v01.x)), __fmul_rn(cy[j].l1, __fmaf_rn(cx[i].l0, v10.x, __fmul_rn(cx[i].l1, v11.x))));
             const float gy = __fmaf_rn(cy[j].l0, __fmaf_rn(cx[i].l0, v00.y, __fmul_rn(cx[i].l1, v01.y)), __fmul_rn(cy[j].l1, __fmaf_rn(cx[i].l0, v10.y, __fmul_rn(cx[i].l1, v11.y))));
@@ -255,6 +267,7 @@ fwd_fused_u8_kernel(const uint8_t *__restrict__ in, const float2 *__restrict__ l
         }
 }
 
+template <typename L>
 __global__ void __launch_bounds__(256)
 compose_map_kernel(const MapSpec m, const View out, const int N, const int Ho, const int Wo)
 {
@@ -265,19 +278,43 @@ compose_map_kernel(const MapSpec m, const View out, const int N, const int Ho, c
     const int h = (int)(r % Ho), n = (int)(r / Ho);
     float rh, rw, gx, gy;
     up_scales(m, Ho, Wo, rh, rw);
-    map_at(m, n, h, w, rh, rw, gx, gy);
+    map_at<L>(m, n, h, w, rh, rw, gx, gy);
     float *o = (float *)out.p + (int64_t)n * out.sN + h * out.s1 + w * out.s2;
     o[0] = gx; o[out.s3] = gy;
+}
+
+template <typename TI, typename TO, typename L>
+void launch_io_l(const View &in, const MapSpec &m, const View &out, const Geometry &g, cudaStream_t st)
+{
+    dim3 blocks((g.Wo + kTileW - 1) / kTileW, (g.Ho + kTileH - 1) / kTileH, g.N);
+    if (g.C == 3) { fwd_fused_kernel<TI, TO, L, 3><<<blocks, kThreads, 0, st>>>(in, m, out, g); note_launch(); }
+    else if (g.C == 1) { fwd_fused_kernel<TI, TO, L, 1><<<blocks, kThreads, 0, st>>>(in, m, out, g); note_launch(); }
+    else { fwd_fused_kernel<TI, TO, L, 0><<<blocks, kThreads, 0, st>>>(in, m, out, g); note_launch(); }
+    note_kernel("fwd_fused");
 }
 
 template <typename TI, typename TO>
 void launch_io(const View &in, const MapSpec &m, const View &out, const Geometry &g, cudaStream_t st)
 {
+    if (m.drift_dtype == PWS_F16) launch_io_l<TI, TO, __half>(in, m, out, g, st);
+    else if (m.drift_dtype == PWS_BF16) launch_io_l<TI, TO, __nv_bfloat16>(in, m, out, g, st);
+    else launch_io_l<TI, TO, float>(in, m, out, g, st);
+}
+
+template <typename LP>
+void launch_u8(const View &in, const MapSpec &m, const View &out, const Geometry &g, cudaStream_t st)
+{
     dim3 blocks((g.Wo + kTileW - 1) / kTileW, (g.Ho + kTileH - 1) / kTileH, g.N);
-    if (g.C == 3) { fwd_fused_kernel<TI, TO, 3><<<blocks, kThreads, 0, st>>>(in, m, out, g); note_launch(); }
-    else if (g.C == 1) { fwd_fused_kernel<TI, TO, 1><<<blocks, kThreads, 0, st>>>(in, m, out, g); note_launch(); }
-    else { fwd_fused_kernel<TI, TO, 0><<<blocks, kThreads, 0, st>>>(in, m, out, g); note_launch(); }
-    note_kernel("fwd_fused");
+    float rh, rw;
+    up_scales_host(m, g.Ho, g.Wo, rh, rw);
+    const uint8_t *ip = (const uint8_t *)in.p;
+    const LP *lp = (const LP *)m.drift.p;
+    uint8_t *op = (uint8_t *)out.p;
+    const bool border = g.padding == PWS_PAD_BORDER, al = g.align != 0, upa = m.upsample == PWS_UP_ALIGNED;
+#define PWS_U8(B, A, U) fwd_fused_u8_kernel<LP, B, A, U><<<blocks, kThreads, 0, st>>>(ip, lp, op, g.H, g.W, g.Ho, g.Wo, m.mh, m.mw, rh, rw)
+    if (border) { if (al) { if (upa) PWS_U8(true, true, true); else PWS_U8(true, true, false); } else { if (upa) PWS_U8(true, false, true); else PWS_U8(true, false, false); } }
+    else        { if (al) { if (upa) PWS_U8(false, true, true); else PWS_U8(false, true, false); } else { if (upa) PWS_U8(false, false, true); else PWS_U8(false, false, false); } }
+#undef PWS_U8
 }
 
 }  // namespace
@@ -286,25 +323,18 @@ int launch_forward_fused(const View &in, int in_dtype, const MapSpec &m, const V
                          const Geometry &g, cudaStream_t st)
 {
     if (g.N > 65535 || (g.Ho + kTileH - 1) / kTileH > 65535) { set_error("fused forward: batch or height too large"); return PWS_EUNSUPPORTED; }
-    // the inference site: dense uint8 HWC in and out, dense interleaved lattice, upsampling, nothing else
+    // the inference site: dense uint8 HWC in and out, dense interleaved lattice (fp32 or 16-bit), upsampling, nothing else
+    const int lat_bytes = m.drift_dtype == PWS_F32 ? 4 : 2;
     const bool u8_fast = in_dtype == PWS_U8 && out_dtype == PWS_U8 && g.C == 3 && m.base == PWS_BASE_NONE && m.drift.p &&
         m.upsample != PWS_UP_NONE && !m.has_pre && !m.has_post &&
         in.s1 == 1 && in.s3 == 3 && in.s2 == 3 * g.W && (g.N == 1 || in.sN == (int64_t)3 * g.W * g.H) &&
         out.s1 == 1 && out.s3 == 3 && out.s2 == 3 * g.Wo && (g.N == 1 || out.sN == (int64_t)3 * g.Wo * g.Ho) &&
         m.drift.s3 == 1 && m.drift.s2 == 2 && m.drift.s1 == 2 * m.mw && (g.N == 1 || m.drift.sN == (int64_t)2 * m.mw * m.mh) &&
-        !(reinterpret_cast<uintptr_t>(m.drift.p) & 7);
+        !(reinterpret_cast<uintptr_t>(m.drift.p) & (2 * lat_bytes - 1));
     if (u8_fast) {
-        dim3 blocks((g.Wo + kTileW - 1) / kTileW, (g.Ho + kTileH - 1) / kTileH, g.N);
-        float rh, rw;
-        up_scales_host(m, g.Ho, g.Wo, rh, rw);
-        const uint8_t *ip = (const uint8_t *)in.p;
-        const float2 *lp = (const float2 *)m.drift.p;
-        uint8_t *op = (uint8_t *)out.p;
-        const bool border = g.padding == PWS_PAD_BORDER, al = g.align != 0, upa = m.upsample == PWS_UP_ALIGNED;
-#define PWS_U8(B, A, U) fwd_fused_u8_kernel<B, A, U><<<blocks, kThreads, 0, st>>>(ip, lp, op, g.H, g.W, g.Ho, g.Wo, m.mh, m.mw, rh, rw)
-        if (border) { if (al) { if (upa) PWS_U8(true, true, true); else PWS_U8(true, true, false); } else { if (upa) PWS_U8(true, false, true); else PWS_U8(true, false, false); } }
-        else        { if (al) { if (upa) PWS_U8(false, true, true); else PWS_U8(false, true, false); } else { if (upa) PWS_U8(false, false, true); else PWS_U8(false, false, false); } }
-#undef PWS_U8
+        if (m.drift_dtype == PWS_F16) launch_u8<__half2>(in, m, out, g, st);
+        else if (m.drift_dtype == PWS_BF16) launch_u8<__nv_bfloat162>(in, m, out, g, st);
+        else launch_u8<float2>(in, m, out, g, st);
         note_launch();
         note_kernel("fwd_fused_u8");
         return PWS_OK;
@@ -325,7 +355,9 @@ int launch_compose_map(const MapSpec &m, const View &out, int N, int Ho, int Wo,
     if (total == 0) return PWS_OK;
     const int64_t blocks = (total + 255) / 256;
     if (blocks > INT_MAX) { set_error("compose_map: too many pixels"); return PWS_EUNSUPPORTED; }
-    compose_map_kernel<<<(unsigned)blocks, 256, 0, st>>>(m, out, N, Ho, Wo);
+    if (m.drift_dtype == PWS_F16) compose_map_kernel<__half><<<(unsigned)blocks, 256, 0, st>>>(m, out, N, Ho, Wo);
+    else if (m.drift_dtype == PWS_BF16) compose_map_kernel<__nv_bfloat16><<<(unsigned)blocks, 256, 0, st>>>(m, out, N, Ho, Wo);
+    else compose_map_kernel<float><<<(unsigned)blocks, 256, 0, st>>>(m, out, N, Ho, Wo);
     note_launch();
     note_kernel("compose_map");
     return PWS_OK;
