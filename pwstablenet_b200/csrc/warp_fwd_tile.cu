@@ -13,8 +13,9 @@ namespace pws {
 
 namespace {
 
-constexpr int kTW = 64, kTH = 32, kBW = 80, kBH = 40, kThreads = 256, kWarps = 8;
-constexpr int kPX = kTW / 32, kPY = kTH / kWarps;
+// a block covers kTW x kTH output pixels: 8 warps of kPY rows, a lane owns kPX columns of each
+constexpr int kTW = 64, kThreads = 256, kWarps = 8;
+constexpr int kPX = kTW / 32, kPY = 2, kTH = kWarps * kPY;
 
 // Layout-specialised direct gather: taps through L1 (no staging, no barrier).  4 pixels per thread, 64x16 tile.
 // G: map element type (float, or T for 16-bit frames); map coordinates are upcast to fp32 on load.
@@ -25,24 +26,23 @@ template <typename T, typename G, int CS, bool kBorder, bool kAlign>
 __global__ void __launch_bounds__(kThreads, PWS_FWD_MINB)
 fwd_lean_kernel(const View in, const View grid, const View out, const Geometry g)
 {
-    constexpr int PY = 2;
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
     const int n = blockIdx.z;
-    const int w_base = blockIdx.x * kTW + lane, h_base = blockIdx.y * (kWarps * PY) + wrp;
+    const int w_base = blockIdx.x * kTW + lane, h_base = blockIdx.y * kTH + wrp;
     const G *__restrict__ gp = (const G *)grid.p + (int64_t)n * grid.sN;
     const T *__restrict__ ip = (const T *)in.p + (int64_t)n * in.sN;
     T *__restrict__ op = (T *)out.p + (int64_t)n * out.sN;
     const float Wf = (float)g.W, Hf = (float)g.H, Wm1 = (float)(g.W - 1), Hm1 = (float)(g.H - 1);
-    const bool full = (blockIdx.x + 1) * kTW <= g.Wo && (blockIdx.y + 1) * (kWarps * PY) <= g.Ho;
+    const bool full = (blockIdx.x + 1) * kTW <= g.Wo && (blockIdx.y + 1) * kTH <= g.Ho;
 
-    float sx[PY][kPX], sy[PY][kPX];
+    float sx[kPY][kPX], sy[kPY][kPX];
     {
         const bool inter = grid.s3 == 1;
         const G *__restrict__ q = gp + (int64_t)h_base * grid.s1 + (int64_t)w_base * grid.s2;
         const int64_t row = (int64_t)kWarps * grid.s1;
         const int col = 32 * grid.s2;
 #pragma unroll
-        for (int j = 0; j < PY; ++j)
+        for (int j = 0; j < kPY; ++j)
 #pragma unroll
             for (int i = 0; i < kPX; ++i) {
                 sx[j][i] = -4.0f; sy[j][i] = -4.0f;
@@ -62,7 +62,7 @@ fwd_lean_kernel(const View in, const View grid, const View out, const Geometry g
     const int sH = in.s2;
     T *__restrict__ o0 = op + (int64_t)h_base * out.s2 + w_base;
 #pragma unroll
-    for (int j = 0; j < PY; ++j)
+    for (int j = 0; j < kPY; ++j)
 #pragma unroll
         for (int i = 0; i < kPX; ++i) {
             const bool ok = full || (w_base + 32 * i < g.Wo && h_base + kWarps * j < g.Ho);
@@ -111,7 +111,7 @@ void launch_cs(const Problem &pb, cudaStream_t st)
     const Geometry &g = pb.g;
     const bool border = g.padding == PWS_PAD_BORDER, align = g.align != 0;
     {
-        dim3 lb((g.Wo + kTW - 1) / kTW, (g.Ho + 15) / 16, g.N);
+        dim3 lb((g.Wo + kTW - 1) / kTW, (g.Ho + kTH - 1) / kTH, g.N);
         if (border && align) { fwd_lean_kernel<T, G, CS, true, true><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
         else if (border) { fwd_lean_kernel<T, G, CS, true, false><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
         else if (align) { fwd_lean_kernel<T, G, CS, false, true><<<lb, kThreads, 0, st>>>(pb.in, pb.grid, pb.out, g); note_launch(); }
