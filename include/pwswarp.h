@@ -159,7 +159,13 @@ typedef struct pws_map_spec {
     float pre_add, pre_mul, post_div, post_add;
 } pws_map_spec;
 
-/* Forward warp with the composed map; `out` (N,C,Ho,Wo) fixes the output size. */
+/* Forward warp with the composed map; `out` (N,C,Ho,Wo) fixes the output size.
+ * Arithmetic is fp32 for every frame type (uint8 and 16-bit frames are upcast exactly): (x + pre_add) * pre_mul per tap,
+ * the bilinear sample in ATen's order, acc / post_div (a true division) + post_add, each op rounded in fp32.  The result
+ * is rounded ONCE, at the store: to the output's 16-bit type (round to nearest even), or for a PWS_U8 output clamped to
+ * [0, 255] and truncated (NaN -> 0).  This differs on purpose from pws_warp2d_stages_forward, which reproduces torch's
+ * rounding to the frame type after every elementwise op: warp_fused replaces an inference pipeline whose intermediates
+ * were fp32, and one rounding is the closer result. */
 int pws_warp2d_forward_fused(const pws_tensor *in, const pws_map_spec *spec, pws_tensor *out,
                              int padding, int align_corners, void *stream);
 

@@ -102,6 +102,11 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
     upsample: None | 'aligned' (UpsamplingBilinear2d) | 'half_pixel' (nn.Upsample bilinear); needs out_size.
     pre=(a,b): frame' = (frame+a)*b.   post=(d,e): out = acc/d + e.
     out_dtype: frame dtype by default; torch.float32 or torch.uint8 (truncating) are also offered.
+
+    Arithmetic is fp32 for every frame dtype (uint8 and 16-bit frames are upcast exactly): (x + a) * b, the sample,
+    acc / d (a true division) + e, and the result is rounded once, at the store: to a float16 / bfloat16 output by round
+    to nearest, to a uint8 one by clamping to [0, 255] and truncating (NaN -> 0).  warp_stages instead rounds after every
+    op on a 16-bit frame, as torch does on half-precision tensors.
     """
     lib = _lib.load()
     if not frame.is_cuda or frame.dim() != 4 or frame.dtype not in _DT:
