@@ -169,6 +169,24 @@ typedef struct pws_map_spec {
 int pws_warp2d_forward_fused(const pws_tensor *in, const pws_map_spec *spec, pws_tensor *out,
                              int padding, int align_corners, void *stream);
 
+/* Autograd of pws_warp2d_forward_fused.  spec, padding and align_corners are what the forward was given; gout has the
+ * forward output's sizes (any strides) and dtype, which must be a float one: f32 for f32 and uint8 frames, the frame's
+ * type for f16 / bf16 frames (a uint8 output is not differentiable: PWS_EINVAL).  Every output is optional (NULL):
+ *     gin       (N,C,H,W) dense f32 accumulation buffer, zero-filled by the library; the caller rounds it to the frame
+ *               dtype once.  Not for uint8 frames.
+ *     glattice  (N,map_h,map_w,2) dense f32, 8-byte aligned (each node's pair is one 8-byte access), zero-filled by
+ *               the library: d loss / d lattice, which is d loss / d drift (the drift enters additively); also allowed
+ *               without a drift.
+ *     gtheta    (N,2,3) f32 contiguous device memory, PWS_BASE_AFFINE only, needs glattice:
+ *               gtheta[n,c,:] = sum_ij glattice[n,i,j,c] * (bx_j, by_i, 1), with the base coordinates the forward uses.
+ * The map is recomputed with the forward's statements (same taps); go = gout / post_div (a true division, as the forward
+ * divides); grad_grid follows ATen's statement order on the pre-scaled taps; fp32 throughout.  Without upsample glattice
+ * equals pws_warp2d_backward's grad_grid of the composed map bit for bit; with upsample it is that grad_grid pushed
+ * through the upsample's adjoint, summed with atomics (order-dependent in the last bits). */
+int pws_warp2d_backward_fused(const pws_tensor *gout, const pws_tensor *in, const pws_map_spec *spec,
+                              pws_tensor *gin, pws_tensor *glattice, float *gtheta,
+                              int padding, int align_corners, void *stream);
+
 /* Debug / parity: writes the map the fused kernel uses into map_out (N,Ho,Wo,2) f32 (also for a 16-bit drift). */
 int pws_compose_map(const pws_map_spec *spec, int64_t n, pws_tensor *map_out, void *stream);
 

@@ -22,6 +22,7 @@ EXPORTS = (
     "pws_warp2d_backward",
     "pws_warp2d_taps",
     "pws_warp2d_forward_fused",
+    "pws_warp2d_backward_fused",
     "pws_compose_map",
     "pws_warp2d_stages_forward",
     "pws_warp2d_stages_backward",
@@ -91,6 +92,8 @@ def load() -> ctypes.CDLL:
     S = ctypes.POINTER(PwsMapSpec)
     lib.pws_warp2d_forward_fused.restype = ctypes.c_int
     lib.pws_warp2d_forward_fused.argtypes = [P, S, P, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
+    lib.pws_warp2d_backward_fused.restype = ctypes.c_int
+    lib.pws_warp2d_backward_fused.argtypes = [P, P, S, P, P, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
     lib.pws_compose_map.restype = ctypes.c_int
     lib.pws_compose_map.argtypes = [S, ctypes.c_int64, P, ctypes.c_void_p]
     PP = ctypes.c_void_p

@@ -87,7 +87,7 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
                map_size: Optional[Tuple[int, int]] = None, padding_mode: str = "zeros", align_corners: bool = False,
                pre: Tuple[float, float] = (0.0, 1.0), post: Tuple[float, float] = (1.0, 0.0),
                out_dtype: Optional[torch.dtype] = None, out_channels_last: bool = False) -> torch.Tensor:
-    """grid_sample(pre(frame), upsample(drift + base)) -> post, in one kernel (forward only).
+    """grid_sample(pre(frame), upsample(drift + base)) -> post, in one kernel, with autograd to frame, drift and theta.
 
     frame:  (N,C,H,W) view, float32/16-bit float or uint8, any strides (a cv2 HWC buffer is
             `buf.permute(0,3,1,2)`).
@@ -107,12 +107,32 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
     acc / d (a true division) + e, and the result is rounded once, at the store: to a float16 / bfloat16 output by round
     to nearest, to a uint8 one by clamping to [0, 255] and truncating (NaN -> 0).  warp_stages instead rounds after every
     op on a 16-bit frame, as torch does on half-precision tensors.
+
+    Backward: when grad mode is on, the output is float and the frame (float), drift or theta requires grad, the call
+    records one autograd node whose backward is one kernel (pws_warp2d_backward_fused): the map is recomputed with the
+    forward's statements and the gradient reaches the lattice through the upsample's adjoint, so neither the
+    full-resolution map nor its gradient is ever written.  It is the gradient of the forward's own fp32 arithmetic:
+    frame gradient summed in fp32 and rounded once to the frame dtype, drift gradient rounded once to drift's dtype,
+    theta gradient in float32.  Every other call (a uint8 output in particular) takes the forward kernel alone and its
+    output has no grad_fn.
     """
-    lib = _lib.load()
     if not frame.is_cuda or frame.dim() != 4 or frame.dtype not in _DT:
         raise RuntimeError("warp_fused: frame must be a 4-D CUDA tensor of dtype float32/float16/bfloat16/uint8")
     if padding_mode not in ("zeros", "border"):
         raise NotImplementedError("warp_fused: padding_mode must be 'zeros' or 'border'")
+    opts = (base, base_align_corners, upsample, out_size, map_size, padding_mode, align_corners, tuple(pre), tuple(post),
+            out_dtype, out_channels_last)
+    final_dtype = out_dtype or (torch.float32 if frame.dtype == torch.uint8 else frame.dtype)
+    wants_grad = (frame.dtype != torch.uint8 and frame.requires_grad) or (drift is not None and drift.requires_grad) or \
+        (theta is not None and theta.requires_grad)
+    if torch.is_grad_enabled() and final_dtype.is_floating_point and wants_grad:
+        return _WarpFused.apply(frame, drift, theta, opts)
+    return _fused_forward(frame, drift, theta, *opts)
+
+
+def _fused_forward(frame, drift, theta, base, base_align_corners, upsample, out_size, map_size, padding_mode,
+                   align_corners, pre, post, out_dtype, out_channels_last):
+    lib = _lib.load()
     n, c = frame.size(0), frame.size(1)
     keep = []
     if upsample is not None and base != "none":
@@ -145,6 +165,46 @@ def warp_fused(frame: torch.Tensor, drift: Optional[torch.Tensor] = None, base: 
                                           _PADDING[padding_mode], int(bool(align_corners)), _stream(frame))
     _lib.check(rc)
     return out
+
+
+class _WarpFused(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, frame, drift, theta, opts):
+        out = _fused_forward(frame, drift, theta, *opts)
+        ctx.save_for_backward(frame, drift, theta)
+        ctx.opts = opts
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, gout):
+        lib = _lib.load()
+        frame, drift, theta = ctx.saved_tensors
+        base, base_align_corners, upsample, out_size, map_size, padding_mode, align_corners, pre, post, _, _ = ctx.opts
+        n = frame.size(0)
+        # the original spec (not the forward's pre-composed lattice): the kernel recomposes the map node for node, and
+        # theta's gradient needs the base
+        keep = []
+        spec = _spec(n, drift, base, theta, base_align_corners, upsample, map_size, pre, post, keep)
+        want_frame = ctx.needs_input_grad[0] and frame.dtype != torch.uint8
+        want_drift = ctx.needs_input_grad[1] and drift is not None
+        want_theta = ctx.needs_input_grad[2] and base == "affine"
+        # grad_input sums in fp32 for every frame type and is rounded to the frame dtype once, below
+        gin = torch.empty(frame.size(), dtype=torch.float32, device=frame.device) if want_frame else None
+        glat = torch.empty((n, spec.map_h, spec.map_w, 2), dtype=torch.float32, device=frame.device) \
+            if (want_drift or want_theta) else None
+        gtheta = torch.empty((n, 2, 3), dtype=torch.float32, device=frame.device) if want_theta else None
+        with torch.cuda.device_of(frame):
+            rc = lib.pws_warp2d_backward_fused(ctypes.byref(_desc(gout)), ctypes.byref(_desc(frame)), ctypes.byref(spec),
+                                               ctypes.byref(_desc(gin)) if gin is not None else None,
+                                               ctypes.byref(_desc(glat)) if glat is not None else None,
+                                               gtheta.data_ptr() if gtheta is not None else None,
+                                               _PADDING[padding_mode], int(bool(align_corners)), _stream(frame))
+        _lib.check(rc)
+        if gin is not None and gin.dtype != frame.dtype:
+            gin = gin.to(frame.dtype)
+        gdrift = glat.to(drift.dtype) if want_drift else None
+        return gin, gdrift, gtheta, None
 
 
 # ---- K maps, one frame, one launch: forward + backward (include/pwswarp.h, csrc/warp_stages.cu) ---------------------

@@ -192,6 +192,8 @@ static int check_stage_dtypes(const pws_tensor *in, const pws_tensor *const *gri
 int launch_forward_fused(const View &in, int in_dtype, const MapSpec &m, const View &out, int out_dtype,
                          const Geometry &g, cudaStream_t st);
 int launch_compose_map(const MapSpec &m, const View &out, int N, int Ho, int Wo, cudaStream_t st);
+int launch_backward_fused(const View &gout, const View &in, int in_dtype, const MapSpec &m, const View &gin, bool want_gin,
+                          float *glat, float *gtheta, const Geometry &g, cudaStream_t st);
 
 static int make_spec(const pws_map_spec *spec, int64_t N, int64_t Ho, int64_t Wo, MapSpec *m)
 {
@@ -369,6 +371,74 @@ int pws_warp2d_forward_fused(const pws_tensor *in, const pws_map_spec *spec, pws
     if (!dg.ok) { set_error("fused forward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
     PWS_TRY(launch_forward_fused(vin, in->dtype, m, vout, out->dtype, g, (cudaStream_t)stream));
     return finish("fused forward");
+}
+
+__attribute__((visibility("default")))
+int pws_warp2d_backward_fused(const pws_tensor *gout, const pws_tensor *in, const pws_map_spec *spec,
+                              pws_tensor *gin, pws_tensor *glattice, float *gtheta,
+                              int padding, int align_corners, void *stream)
+{
+    PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
+    if (!in || !gout) { set_error("fused backward: null tensor descriptor"); return PWS_EINVAL; }
+    for (int d = 2; d < 4; ++d)
+        if (in->size[d] <= 0) { set_error("grid_sampler(): expected input to have non-empty spatial dimensions"); return PWS_EINVAL; }
+    if (gout->size[0] != in->size[0] || gout->size[1] != in->size[1]) { set_error("fused backward: grad_output batch/channels must equal the input's"); return PWS_EINVAL; }
+    if (gout->device != in->device) { set_error("fused backward: grad_output must be on the input's device"); return PWS_EINVAL; }
+    const bool half_in = in->dtype == PWS_F16 || in->dtype == PWS_BF16;
+    if (in->dtype != PWS_F32 && in->dtype != PWS_U8 && !half_in) { set_error("fused backward: frames must be f32, f16, bf16 or uint8"); return PWS_EUNSUPPORTED; }
+    if (gout->dtype == PWS_U8) { set_error("fused backward: a uint8 output is not differentiable"); return PWS_EINVAL; }
+    if (gout->dtype != (half_in ? in->dtype : PWS_F32)) {
+        set_error("fused backward: grad_output must be f32 (f32 or uint8 frames) or the frame's 16-bit type (frame %d, grad_output %d)", in->dtype, gout->dtype);
+        return PWS_EINVAL;
+    }
+    if (gtheta && (!spec || spec->base != PWS_BASE_AFFINE)) { set_error("fused backward: gtheta needs the affine base"); return PWS_EINVAL; }
+    if (gtheta && !glattice) { set_error("fused backward: gtheta needs glattice (the library never allocates)"); return PWS_EINVAL; }
+    View vin, vgout, vgin{}, vglat{};
+    PWS_TRY(make_view(in, "input", &vin));
+    PWS_TRY(make_view(gout, "grad_output", &vgout));
+    MapSpec m;
+    PWS_TRY(make_spec(spec, in->size[0], gout->size[2], gout->size[3], &m));
+    if (gin) {
+        if (in->dtype == PWS_U8) { set_error("fused backward: a uint8 frame has no gradient (gin must be NULL)"); return PWS_EINVAL; }
+        PWS_TRY(make_view(gin, "grad_input", &vgin));
+        PWS_TRY(same_shape(gin, in->size[0], in->size[1], in->size[2], in->size[3], "grad_input"));
+        const int64_t C = in->size[1], H = in->size[2], W = in->size[3];
+        const bool dense = gin->dtype == PWS_F32 && gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
+                           (gin->stride[0] == C * H * W || in->size[0] <= 1);
+        if (!dense) { set_error("grad_input: must be f32 (N,C,H,W)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
+        if (gin->device != in->device) { set_error("fused backward: grad_input must be on the input's device"); return PWS_EINVAL; }
+        vgin.sN = C * H * W;
+    }
+    if (glattice) {
+        PWS_TRY(make_view(glattice, "glattice", &vglat));
+        PWS_TRY(same_shape(glattice, in->size[0], spec->map_h, spec->map_w, 2, "glattice"));
+        const int64_t h = spec->map_h, w = spec->map_w;
+        const bool dense = glattice->dtype == PWS_F32 && glattice->stride[3] == 1 && glattice->stride[2] == 2 &&
+                           glattice->stride[1] == 2 * w && (glattice->stride[0] == 2 * h * w || in->size[0] <= 1);
+        if (!dense) { set_error("glattice: must be f32 (N,map_h,map_w,2)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
+        // every node's (x, y) is stored, reduced into and read back as one 8-byte pair
+        if (reinterpret_cast<uintptr_t>(glattice->data) & 7) { set_error("glattice: must be 8-byte aligned (one float2 per node)"); return PWS_EINVAL; }
+        if (glattice->device != in->device) { set_error("fused backward: glattice must be on the input's device"); return PWS_EINVAL; }
+    }
+    Geometry g{};
+    g.N = (int32_t)in->size[0]; g.C = (int32_t)in->size[1]; g.H = (int32_t)in->size[2]; g.W = (int32_t)in->size[3];
+    g.Ho = (int32_t)gout->size[2]; g.Wo = (int32_t)gout->size[3]; g.padding = padding; g.align = align_corners ? 1 : 0;
+    DeviceGuard dg(in->device);
+    if (!dg.ok) { set_error("fused backward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
+    if (g.N == 0) return PWS_OK;
+    if ((int64_t)g.C * g.Ho * g.Wo == 0) {
+        // nothing flows back; the gradients are still defined (all zeros)
+        cudaStream_t st = (cudaStream_t)stream;
+        cudaError_t e = cudaSuccess;
+        if (gin && (int64_t)g.C * g.H * g.W > 0) e = cudaMemsetAsync(gin->data, 0, (size_t)(g.N * vgin.sN * 4), st);
+        if (e == cudaSuccess && glattice) e = cudaMemsetAsync(glattice->data, 0, (size_t)g.N * m.mh * m.mw * 2 * 4, st);
+        if (e == cudaSuccess && gtheta) e = cudaMemsetAsync(gtheta, 0, (size_t)g.N * 6 * 4, st);
+        if (e != cudaSuccess) { set_error("fused backward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return PWS_ECUDA; }
+        return PWS_OK;
+    }
+    PWS_TRY(launch_backward_fused(vgout, vin, in->dtype, m, vgin, gin != nullptr, glattice ? (float *)glattice->data : nullptr,
+                                  gtheta, g, (cudaStream_t)stream));
+    return finish("fused backward");
 }
 
 __attribute__((visibility("default")))
