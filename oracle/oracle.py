@@ -10,6 +10,7 @@ Reference call sites restated (R = /root/reference):
   generate_maps        R/lib/utils.py:386-403
   affine_map           R/lib/networks_cascading.py:164,235 (F.affine_grid + drift)
   upsample_map         R/main_new.py:706-710, R/main.py:639-641
+  upsample_map_backward, affine_theta_grad   their adjoints (warp_fused's backward, R/main_new.py:214)
 """
 from __future__ import annotations
 
@@ -39,7 +40,7 @@ def lib() -> ctypes.CDLL:
     if _lib is None:
         build()
         _lib = ctypes.CDLL(_LIB_PATH)
-        assert _lib.oracle_abi_version() == 1
+        assert _lib.oracle_abi_version() == 2
     return _lib
 
 
@@ -141,3 +142,35 @@ def upsample_map(src: np.ndarray, H: int, W: int, align_corners: bool = True):
     out = np.empty((N, 2, H, W), np.float32)
     lib().oracle_upsample_map_f32(_ptr(src), _ptr(out), N, h, w, H, W, int(bool(align_corners)))
     return out
+
+
+def upsample_coefs(src: int, dst: int, align_corners: bool = True):
+    """(i0, ip, l0, l1) of destination indices 0..dst-1 from a source of size src: upsample_map's coefficients."""
+    i0, ip = np.empty(dst, np.int32), np.empty(dst, np.int32)
+    l0, l1 = np.empty(dst, np.float32), np.empty(dst, np.float32)
+    lib().oracle_upsample_coefs_f32(src, dst, int(bool(align_corners)), _ptr(i0), _ptr(ip), _ptr(l0), _ptr(l1))
+    return i0, ip, l0, l1
+
+
+def upsample_map_backward(gmap: np.ndarray, h: int, w: int, align_corners: bool = True):
+    """Adjoint of upsample_map with its fp32 coefficients: gmap planar (N,2,H,W) -> (glat, gabs, nterms), each
+    (N,2,h,w): the fp64 sum of the terms h_l * w_l * g each node receives, the sum of their magnitudes, their count."""
+    gmap = np.ascontiguousarray(gmap, np.float64)
+    N, two, H, W = gmap.shape
+    assert two == 2
+    glat, gabs = np.zeros((N, 2, h, w)), np.zeros((N, 2, h, w))
+    nterms = np.zeros((N, 2, h, w), np.int64)
+    lib().oracle_upsample_map_backward_f64(_ptr(gmap), N, h, w, H, W, int(bool(align_corners)), _ptr(glat), _ptr(gabs),
+                                           _ptr(nterms))
+    return glat, gabs, nterms
+
+
+def affine_theta_grad(glat: np.ndarray, align_corners: bool = False):
+    """glat interleaved (N,h,w,2) -> (gtheta, gabs), each (N,2,3) fp64: sum_ij glat[n,i,j,c] * (bx_j, by_i, 1) with
+    affine_map's base coordinates, and the sums of the terms' magnitudes."""
+    glat = np.ascontiguousarray(glat, np.float64)
+    N, h, w, two = glat.shape
+    assert two == 2
+    gtheta, gabs = np.zeros((N, 2, 3)), np.zeros((N, 2, 3))
+    lib().oracle_affine_theta_grad_f64(_ptr(glat), N, h, w, int(bool(align_corners)), _ptr(gtheta), _ptr(gabs))
+    return gtheta, gabs

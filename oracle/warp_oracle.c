@@ -400,42 +400,114 @@ ORACLE_API void oracle_affine_map_f32(const float *theta, const float *drift, fl
     }
 }
 
+/* ---- the map upsample (UpSample.cuh:96-130) and its adjoint ------------------- */
+
+/* Source scale of upsample_bilinear2d: (src-1)/(dst-1) aligned (0 for a 1-pixel
+ * destination), src/dst otherwise; one IEEE division, as on the GPU. */
+static inline float up_scale_f32(int src, int dst, int align)
+{
+    if (align) return dst > 1 ? (float)(src - 1) / (float)(dst - 1) : 0.0f;
+    return (float)src / (float)dst;
+}
+
+typedef struct { int i0, ip; float l0, l1; } up_coef_t;
+
+/* Source index of destination index dst: one fp32 multiply aligned, one fma
+ * half_pixel (clamped at 0); lambdas l1 = s - i0, l0 = 1 - l1. */
+static inline up_coef_t up_coef_f32(int dst, int src, float scale, int align)
+{
+    float s = align ? scale * (float)dst : fmaf(scale, (float)dst + 0.5f, -0.5f);
+    if (!align && s < 0.0f) s = 0.0f;
+    up_coef_t c;
+    c.i0 = (int)s;
+    c.ip = (c.i0 < src - 1) ? 1 : 0;
+    c.l1 = s - (float)c.i0;
+    c.l0 = 1.0f - c.l1;
+    return c;
+}
+
+/* The coefficients of destination indices 0..dst-1 from a source of size src
+ * (what the backward's tile census restates). */
+ORACLE_API void oracle_upsample_coefs_f32(int src, int dst, int align, int32_t *i0, int32_t *ip,
+                                          float *l0, float *l1)
+{
+    const float r = up_scale_f32(src, dst, align);
+    for (int d = 0; d < dst; ++d) {
+        up_coef_t c = up_coef_f32(d, src, r, align);
+        i0[d] = c.i0; ip[d] = c.ip; l0[d] = c.l0; l1[d] = c.l1;
+    }
+}
+
 /* Bilinear resize of a planar map (N,2,h,w) -> (N,2,H,W), the map upsample of
  * R/main_new.py:706-710 (UpsamplingBilinear2d: align_corners=True) and
  * R/main.py:639-641 (nn.Upsample bilinear: align_corners=False).
- * Index math: UpSample.cuh:96-130; blend order as upsample_bilinear2d_out_frame:
+ * Blend order as upsample_bilinear2d_out_frame:
  *   h0lambda*(w0lambda*v00 + w1lambda*v01) + h1lambda*(w0lambda*v10 + w1lambda*v11)
  * with nvcc contraction: inner = fma(w0l, v00, w1l*v01), outer = fma(h0l, top, h1l*bot). */
 ORACLE_API void oracle_upsample_map_f32(const float *src, float *dst, int N, int h, int w,
                                         int H, int W, int align)
 {
-    float rh, rw;
-    if (align) {
-        rh = H > 1 ? (float)(h - 1) / (float)(H - 1) : 0.0f;
-        rw = W > 1 ? (float)(w - 1) / (float)(W - 1) : 0.0f;
-    } else {
-        rh = (float)h / (float)H;
-        rw = (float)w / (float)W;
-    }
+    const float rh = up_scale_f32(h, H, align), rw = up_scale_f32(w, W, align);
     for (int n = 0; n < N * 2; ++n)
         for (int y = 0; y < H; ++y) {
-            float sy = align ? rh * (float)y : fmaf(rh, (float)y + 0.5f, -0.5f);
-            if (!align && sy < 0.0f) sy = 0.0f;
-            int y0 = (int)sy; int yp = (y0 < h - 1) ? 1 : 0;
-            float h1l = sy - (float)y0, h0l = 1.0f - h1l;
+            const up_coef_t cy = up_coef_f32(y, h, rh, align);
             for (int x = 0; x < W; ++x) {
-                float sx = align ? rw * (float)x : fmaf(rw, (float)x + 0.5f, -0.5f);
-                if (!align && sx < 0.0f) sx = 0.0f;
-                int x0 = (int)sx; int xp = (x0 < w - 1) ? 1 : 0;
-                float w1l = sx - (float)x0, w0l = 1.0f - w1l;
+                const up_coef_t cx = up_coef_f32(x, w, rw, align);
                 const float *p = src + (int64_t)n * h * w;
-                float v00 = p[y0 * w + x0], v01 = p[y0 * w + x0 + xp];
-                float v10 = p[(y0 + yp) * w + x0], v11 = p[(y0 + yp) * w + x0 + xp];
-                float top = fmaf(w0l, v00, w1l * v01);
-                float bot = fmaf(w0l, v10, w1l * v11);
-                dst[((int64_t)n * H + y) * W + x] = fmaf(h0l, top, h1l * bot);
+                float v00 = p[cy.i0 * w + cx.i0], v01 = p[cy.i0 * w + cx.i0 + cx.ip];
+                float v10 = p[(cy.i0 + cy.ip) * w + cx.i0], v11 = p[(cy.i0 + cy.ip) * w + cx.i0 + cx.ip];
+                float top = fmaf(cx.l0, v00, cx.l1 * v01);
+                float bot = fmaf(cx.l0, v10, cx.l1 * v11);
+                dst[((int64_t)n * H + y) * W + x] = fmaf(cy.l0, top, cy.l1 * bot);
             }
         }
 }
 
-ORACLE_API int oracle_abi_version(void) { return 1; }
+/* Adjoint of oracle_upsample_map_f32 with its fp32 coefficients: the gradient gmap
+ * (planar (N,2,H,W), fp64) of the upsampled map pushed to the lattice (N,2,h,w).
+ * Every pixel hands each of the four nodes it blends the term t = h_l * w_l * g
+ * (a node read twice, ip == 0, takes two terms).  Per node, in fp64: glat = sum t,
+ * gabs = sum |t|, nterms = the number of terms.  All three must arrive zeroed. */
+ORACLE_API void oracle_upsample_map_backward_f64(const double *gmap, int N, int h, int w, int H, int W, int align,
+                                                 double *glat, double *gabs, int64_t *nterms)
+{
+    const float rh = up_scale_f32(h, H, align), rw = up_scale_f32(w, W, align);
+    for (int n = 0; n < N * 2; ++n)
+        for (int y = 0; y < H; ++y) {
+            const up_coef_t cy = up_coef_f32(y, h, rh, align);
+            for (int x = 0; x < W; ++x) {
+                const up_coef_t cx = up_coef_f32(x, w, rw, align);
+                const double g = gmap[((int64_t)n * H + y) * W + x];
+                const int rows[2] = { cy.i0, cy.i0 + cy.ip }, cols[2] = { cx.i0, cx.i0 + cx.ip };
+                const double hl[2] = { cy.l0, cy.l1 }, wl[2] = { cx.l0, cx.l1 };
+                for (int a = 0; a < 2; ++a)
+                    for (int b = 0; b < 2; ++b) {
+                        const int64_t o = ((int64_t)n * h + rows[a]) * w + cols[b];
+                        const double t = hl[a] * wl[b] * g;
+                        glat[o] += t; gabs[o] += fabs(t); nterms[o] += 1;
+                    }
+            }
+        }
+}
+
+/* d loss / d theta of the affine base: gtheta[n,c,:] = sum_ij glat[n,i,j,c] *
+ * (bx_j, by_i, 1) with affine_base_f32's coordinates, in fp64; gabs the sums of
+ * the terms' magnitudes.  glat interleaved (N,h,w,2); gtheta, gabs (N,2,3), zeroed. */
+ORACLE_API void oracle_affine_theta_grad_f64(const double *glat, int N, int h, int w, int align,
+                                             double *gtheta, double *gabs)
+{
+    for (int n = 0; n < N; ++n)
+        for (int i = 0; i < h; ++i)
+            for (int j = 0; j < w; ++j) {
+                const double b[3] = { affine_base_f32(j, w, align), affine_base_f32(i, h, align), 1.0 };
+                for (int c = 0; c < 2; ++c) {
+                    const double g = glat[(((int64_t)n * h + i) * w + j) * 2 + c];
+                    for (int k = 0; k < 3; ++k) {
+                        gtheta[(n * 2 + c) * 3 + k] += g * b[k];
+                        gabs[(n * 2 + c) * 3 + k] += fabs(g * b[k]);
+                    }
+                }
+            }
+}
+
+ORACLE_API int oracle_abi_version(void) { return 2; }

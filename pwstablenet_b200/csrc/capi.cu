@@ -403,8 +403,10 @@ int pws_warp2d_backward_fused(const pws_tensor *gout, const pws_tensor *in, cons
         PWS_TRY(make_view(gin, "grad_input", &vgin));
         PWS_TRY(same_shape(gin, in->size[0], in->size[1], in->size[2], in->size[3], "grad_input"));
         const int64_t C = in->size[1], H = in->size[2], W = in->size[3];
-        const bool dense = gin->dtype == PWS_F32 && gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
-                           (gin->stride[0] == C * H * W || in->size[0] <= 1);
+        // an empty buffer (N = 0 or C = 0) is dense whatever its strides: torch keeps (C*H*W, H*W, W, 1) for C = 0
+        const bool dense = gin->dtype == PWS_F32 && (in->size[0] * C == 0 ||
+                           (gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
+                            (gin->stride[0] == C * H * W || in->size[0] <= 1)));
         if (!dense) { set_error("grad_input: must be f32 (N,C,H,W)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
         if (gin->device != in->device) { set_error("fused backward: grad_input must be on the input's device"); return PWS_EINVAL; }
         vgin.sN = C * H * W;

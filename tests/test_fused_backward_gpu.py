@@ -293,21 +293,22 @@ def test_grad_call_forward_equals_the_no_grad_call(pw, case):
 
 # ---- 6. 1080p geometry ----------------------------------------------------------------------------------------------
 def test_1080p_sums(pw):
+    """1080p from a 256^2 lattice with the affine base (a window of ~66 nodes per tile, runs of ~7 lanes, 2 x 65536
+    nodes): every node within its own bound, theta per item and entry, grad_input to its maximum and its checksum
+    (test_fusion_edges_gpu.FusedBackwardRef states the bounds)."""
+    import numpy as np
+    from test_fusion_edges_gpu import FusedBackwardRef, check_gin, check_glattice, check_gtheta, host
     n, C, H, W, h, w = 2, 3, 1080, 1920, 256, 256
-    frame, drift, _ = make_inputs(n, C, H, W, h, w, "none", seed=9)
+    frame, drift, theta = make_inputs(n, C, H, W, h, w, "affine", seed=9)
     gout = torch.randn(n, C, H, W, device="cuda")
     pre, post = (1.0, 127.5), (127.5, -1.0)
-    _, gf, gd, _ = fused_grads(pw, frame, drift, None, gout, upsample="aligned", out_size=(H, W), pre=pre, post=post)
-    m = pw.compose_map(n, (H, W), drift=drift, upsample="aligned")
-    go = (gout / post[0]).contiguous()
-    _, ggrid = pw.warp2d_backward(go, (frame + pre[0]) * pre[1], m, 0, False, (False, True))
-    # the upsample weights of a pixel sum to 1: the adjoint preserves the total
-    s_ref = ggrid.double().sum((0, 1, 2))
-    assert float((gd.double().sum((0, 1, 2)) - s_ref).abs().max()) <= 1e-4 * float(ggrid.double().abs().sum())
-    # sum of grad_input: every output pixel hands go * pre_mul times its valid tap weights to the frame
-    valid = pw.grid_sample(torch.ones(n, 1, H, W, device="cuda"), m, "bilinear", "zeros", False)
-    s_gin = float((go.double().sum(1, keepdim=True) * valid.double()).sum() * pre[1])
-    assert abs(float(gf.double().sum()) - s_gin) <= 1e-4 * float((go.double().abs().sum(1, keepdim=True) * valid.double()).sum() * pre[1])
+    _, gf, gd, gt = fused_grads(pw, frame, drift, theta, gout, base="affine", upsample="aligned", out_size=(H, W),
+                                pre=pre, post=post)
+    ref = FusedBackwardRef(host(frame), np.ascontiguousarray(host(drift).transpose(0, 3, 1, 2)), "affine", host(theta),
+                           False, "aligned", host(gout), "zeros", False, pre, post)
+    check_glattice(host(gd), ref)
+    check_gtheta(host(gt), ref)
+    check_gin(gf, ref)
 
 
 # ---- 7. training steps ----------------------------------------------------------------------------------------------

@@ -20,6 +20,8 @@ guard probes, on which ATen's CUDA sampler has faulted, only ever meet this libr
     map = oracle upsample / affine / generate_maps composition                             bit for bit
     out = store(sample((x + a) * b, map) / d + e), all fp32, one rounding at the store     bit for bit
     store: the frame's 16-bit type (round to nearest), or uint8 (clamp to [0, 255], truncate, NaN -> 0)
+  warp_fused backward (pws_warp2d_backward_fused): FusedBackwardRef states the contract and its per-node bounds;
+    backward_census restates the kernel's tile window and column runs to pick the cases that reach their edges.
 
 `PYTHONPATH=.:tests python tests/test_fusion_edges_gpu.py` prints the coverage table (no GPU needed)."""
 import ctypes
@@ -40,6 +42,8 @@ DTYPES = {"f32": torch.float32, "f16": torch.float16, "bf16": torch.bfloat16, "u
 OFF_PRE, OFF_POST = (0.0, 1.0), (1.0, 0.0)
 PRE, POST = (1.0, 127.5), (127.5, -1.0)          # the reference's (x + 1) * 127.5 ... / 127.5 - 1
 PAD_ALIGN = [("zeros", False), ("border", True)]
+BASE_SIZES = [(1, 1), (1, 6), (6, 1), (2, 2), (2, 7), (16, 24), (37, 53)]   # 7, 16, 24, 37, 53: the two linspace halves
+                                                                            # round their middle node differently
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -159,6 +163,187 @@ def fused_sample_ref(x, grid, pad, align, pre, post, out_dtype):
     return store(s, out_dtype)
 
 
+U = 2.0 ** -24     # unit roundoff of fp32
+
+
+class FusedBackwardRef:
+    """The contract of pws_warp2d_backward_fused (include/pwswarp.h), restated on the CPU.  x: the frame as float32 (uint8
+    and 16-bit frames upcast exactly), drift: planar (N, 2, h, w) float32, gout: float32 (a 16-bit grad_output upcast and
+    not rounded back: the fused contract, not the stages one).
+        x' = f32((x + a) * b), go' = f32(gout / d) (a true division), map = fused_map_ref
+        gg, gin64 = oracle.backward(go', x', map)
+    Lattice gradient (interleaved (N, h, w, 2)):
+      - no upsample: glattice == gg bit for bit (tol 0), probe and NaN / inf lattices included;
+      - upsample: the fp64 adjoint of the upsample (oracle.upsample_map_backward, the forward's fp32 coefficients).  Per
+        node k with m_k terms t = h_l * w_l * gg: |got_k - ref_k| <= (m_k + 3) * u * sum|t|_k.  The kernel forms each
+        term with two fp32 products and sums the m_k terms in some order (a shuffle scan per run of lanes, then the
+        REDs); first-order fp32 summation error of m_k terms in any order is (m_k - 1) * u * sum|t|, plus one rounding
+        per product and one for the RED.  A node no pixel touches is exactly 0.  Unlike a max-norm this fails when a
+        run, a row of REDs or a tile's contribution goes missing from any node.
+    Theta gradient: oracle.affine_theta_grad of the fp64 lattice reference, per item and entry
+        |got - ref| <= sum_k |b_k| * tol_k + (ceil(nodes / 256) + 9) * u * sum_k |glat_k * b_k|
+      (the kernel's glattice differs from ref by at most tol_k per node; theta_grad_kernel sums ceil(nodes / 256) fmas
+      per thread, then a tree of 8 levels).
+    grad_input: b * gin64, held to 1e-4 of its maximum, and its sum to b * sum go' * (valid tap weights) within 1e-6
+      (check_gin); never element by element: the REDs make it order-dependent."""
+
+    def __init__(self, x, drift, base, theta, base_align, upsample, gout, pad, align, pre=OFF_PRE, post=OFF_POST):
+        has_pre, a, b, has_post, _, d, _ = scales(pre, post)
+        N, C, H, W = x.shape
+        Ho, Wo = gout.shape[2:]
+        h, w = drift.shape[2:]
+        self.upsample, self.base = upsample, base
+        grid = fused_map_ref(drift, base, theta, base_align, upsample, Ho, Wo)
+        with np.errstate(all="ignore"):
+            xs = (np.asarray(x, F32) + a) * b if has_pre else np.ascontiguousarray(x, F32)
+            go = np.asarray(gout, F32) / d if has_post else np.ascontiguousarray(gout, F32)
+        _, gg, gin64 = oracle.backward(np.ascontiguousarray(go), np.ascontiguousarray(xs), grid, pad, align,
+                                       want_f64_accum=True)
+        if upsample is None:
+            self.glat32 = gg
+            self.glat64, self.tol = gg.astype(np.float64), np.zeros(gg.shape)
+            self.nterms = np.ones(gg.shape, np.int64)
+        else:
+            g64, gabs, nterms = oracle.upsample_map_backward(gg.transpose(0, 3, 1, 2), h, w, upsample == "aligned")
+            il = lambda p: np.ascontiguousarray(p.transpose(0, 2, 3, 1))   # noqa: E731  planar -> interleaved
+            self.glat32 = None
+            self.glat64, self.nterms = il(g64), il(nterms)
+            self.tol = (self.nterms + 3) * U * il(gabs)
+        if base == "affine":
+            self.gtheta, gabs = oracle.affine_theta_grad(self.glat64, base_align)
+            _, tol_b = oracle.affine_theta_grad(self.tol, base_align)            # sum_k |b_k| * tol_k
+            self.theta_tol = tol_b + (-(-h * w // 256) + 9) * U * gabs
+        self.gin64 = gin64 * float(b) if has_pre else gin64
+        wsum = tap_weight_sums(grid, H, W, pad, align)
+        self.checksum = float((go.astype(np.float64) * wsum[:, None]).sum()) * float(b)
+        self.checksum_scale = float((np.abs(go.astype(np.float64)) * wsum[:, None]).sum()) * abs(float(b))
+
+
+def half_ulp_bound(ref, dtype):
+    """Half an ulp of `dtype` at |ref| (an upper bound), for a float32 result rounded once to a 16-bit type."""
+    if dtype in (None, torch.float32):
+        return np.zeros(np.shape(ref))
+    fi = torch.finfo(dtype)
+    return 0.5 * fi.eps * np.abs(ref) + float(fi.smallest_normal) * fi.eps
+
+
+def check_glattice(got, ref, dtype=None, what="glattice"):
+    """got: (N, h, w, 2) float32 holding the kernel's lattice gradient (rounded once to `dtype` when it is 16-bit)."""
+    got = np.asarray(got, np.float64)
+    if ref.upsample is None:
+        want = ref.glat32 if dtype in (None, torch.float32) else round_to(ref.glat32, dtype)
+        np.testing.assert_array_equal(got, want, err_msg=what)
+        return
+    fin = np.isfinite(ref.glat64)
+    np.testing.assert_array_equal(got[~fin], ref.glat64[~fin], err_msg=what + ": non-finite nodes")
+    untouched = ref.nterms == 0
+    assert (got[untouched] == 0).all(), what + ": a node no pixel touches is not 0"
+    tol = ref.tol + half_ulp_bound(ref.glat64, dtype)
+    with np.errstate(invalid="ignore"):
+        bad = fin & ~(np.abs(got - ref.glat64) <= tol)
+    if bad.any():
+        k = tuple(np.argwhere(bad)[0])
+        raise AssertionError(f"{what}: {int(bad.sum())} of {bad.size} nodes out of bound; first {k}: got {got[k]!r}, "
+                             f"ref {ref.glat64[k]!r}, bound {tol[k]!r}, terms {ref.nterms[k]}")
+
+
+def check_gtheta(got, ref, what="gtheta"):
+    err = np.abs(np.asarray(got, np.float64) - ref.gtheta)
+    bad = ~(err <= ref.theta_tol)
+    assert not bad.any(), f"{what}: entries {np.argwhere(bad).tolist()} out of bound: got {got}, ref {ref.gtheta}, " \
+                          f"bound {ref.theta_tol}"
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# census of the fused backward's tiles: shared-memory window or per-pixel maps, and the runs of its column scan
+# ---------------------------------------------------------------------------------------------------------------------
+KW_TILE, KH_TILE, WIN_NODES = 64, 16, 1280      # warp_fused.cu: kTileW, kTileH, kWinNodes
+
+
+def up_scale(src, dst, aligned):
+    """warp_fused.cu's up_scales: (src - 1) / (dst - 1) aligned (0 for dst = 1), src / dst half_pixel, fp32 division."""
+    if aligned:
+        return F32(src - 1) / F32(dst - 1) if dst > 1 else F32(0)
+    return F32(src) / F32(dst)
+
+
+def up_coef(dst, src, scale, aligned):
+    """warp_fused.cu's up_coef for an integer array dst: (i0, ip, l0, l1).  Aligned: one fp32 multiply.  half_pixel:
+    fmaf(scale, dst + 0.5, -0.5) clamped at 0; the product of two fp32 values is exact in fp64 and, for a result >= 0
+    (the only one the clamp keeps), so is the sum with -0.5: one rounding, as the fma."""
+    d = np.asarray(dst, np.int64).astype(F32)
+    if aligned:
+        s = (F32(scale) * d).astype(F32)
+    else:
+        s = (np.float64(scale) * (d + F32(0.5)).astype(np.float64) - 0.5).astype(F32)
+        s = np.where(s < 0, F32(0), s)
+    i0 = s.astype(np.int64)
+    ip = (i0 < src - 1).astype(np.int64)
+    l1 = (s - i0.astype(F32)).astype(F32)
+    return i0, ip, (F32(1) - l1).astype(F32), l1
+
+
+def backward_census(mh, mw, Ho, Wo, upsample):
+    """bwd_fused_kernel's structure for an upsample from an mh x mw lattice to Ho x Wo:
+      nodes[ty, tx]  nr * nc of the tile's window (first / last row and column, the last clamped to Ho-1 / Wo-1);
+                     <= WIN_NODES composes the window in shared memory, more evaluates the map per pixel
+      runs           lengths of the runs of equal cx.i0 over the 32 lanes of each half tile row (i = 0, 1)
+      split          runs that continue from lane 31 of the first half into lane 0 of the second
+      ip0_runs       runs whose column has ip == 0 (two REDs into one node)
+      edge_lanes     lanes past the right edge, per half (they carry zeros and join the last run)"""
+    al = upsample == "aligned"
+    rh, rw = up_scale(mh, Ho, al), up_scale(mw, Wo, al)
+    ty, tx = -(-Ho // KH_TILE), -(-Wo // KW_TILE)
+    r0 = up_coef(np.arange(ty) * KH_TILE, mh, rh, al)
+    r1 = up_coef(np.minimum(np.arange(ty) * KH_TILE + KH_TILE - 1, Ho - 1), mh, rh, al)
+    c0 = up_coef(np.arange(tx) * KW_TILE, mw, rw, al)
+    c1 = up_coef(np.minimum(np.arange(tx) * KW_TILE + KW_TILE - 1, Wo - 1), mw, rw, al)
+    nr, nc = r1[0] + r1[1] - r0[0] + 1, c1[0] + c1[1] - c0[0] + 1
+    nodes = nr[:, None] * nc[None, :]
+    runs, split, ip0_runs, edge = [], 0, 0, [0, 0]
+    for bx in range(tx):
+        w = bx * KW_TILE + np.arange(KW_TILE)
+        i0, ip, _, _ = up_coef(np.minimum(w, Wo - 1), mw, rw, al)
+        for half in (0, 1):
+            k, p = i0[32 * half:32 * half + 32], ip[32 * half:32 * half + 32]
+            starts = np.flatnonzero(np.r_[True, k[1:] != k[:-1]])
+            runs += np.diff(np.r_[starts, 32]).tolist()
+            ip0_runs += int((p[starts] == 0).sum())
+            edge[half] += int((w[32 * half:32 * half + 32] >= Wo).sum())
+        split += int(i0[31] == i0[32])
+    return dict(nodes=nodes, window=int((nodes <= WIN_NODES).sum()), per_pixel=int((nodes > WIN_NODES).sum()),
+                runs=np.array(runs), split=split, ip0_runs=ip0_runs, edge_lanes=tuple(edge))
+
+
+def census_row(c):
+    n, r = c["nodes"], c["runs"]
+    return (f"nodes {', '.join(str(v) for v in sorted(set(n.ravel().tolist())))}; window {c['window']} / per-pixel "
+            f"{c['per_pixel']} tiles; runs {r.min()}..{r.max()} lanes; split at 31/32: {c['split']}; ip == 0 runs: "
+            f"{c['ip0_runs']}; edge lanes (first / second half): {c['edge_lanes'][0]} / {c['edge_lanes'][1]}")
+
+
+# (mh, mw, Ho, Wo, upsample, what the case reaches)
+BWD_CASES = [
+    (8, 160, 16, 64, "aligned", "window exactly full (1280)"),
+    (8, 250, 16, 100, "aligned", "full window and a clamped right tile"),
+    (13, 183, 40, 64, "aligned", "window, per-pixel and window in one call (1281)"),
+    (8, 251, 16, 100, "aligned", "per-pixel (1288) next to a window"),
+    (20, 64, 16, 64, "half_pixel", "half_pixel window exactly full"),
+    (21, 64, 16, 64, "half_pixel", "half_pixel per-pixel"),
+    (4, 4, 1080, 1920, "aligned", "runs of 32 lanes, 1e5 terms per node"),
+    (9, 1, 37, 90, "half_pixel", "mw = 1: ip == 0 everywhere"),
+    (7, 11, 20, 65, "aligned", "Wo = 1 mod 64"),
+    (7, 11, 20, 95, "half_pixel", "Wo = 31 mod 64"),
+    (7, 11, 20, 97, "aligned", "Wo = 33 mod 64"),
+    (7, 11, 20, 127, "half_pixel", "Wo = 63 mod 64"),
+    (7, 11, 1, 70, "aligned", "Ho = 1"),
+    (7, 11, 30, 1, "half_pixel", "Wo = 1"),
+    (40, 9, 20, 70, "aligned", "downsample in y, upsample in x"),
+    (6, 150, 50, 70, "half_pixel", "upsample in y, downsample in x: runs of one lane"),
+]
+BWD_IDS = [f"{c[0]}x{c[1]}-{c[2]}x{c[3]}-{c[4]}" for c in BWD_CASES]
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # inputs
 # ---------------------------------------------------------------------------------------------------------------------
@@ -270,6 +455,113 @@ def test_fused_16bit_reference_rounds_once(dt):
 def test_offframe_maps_are_off_the_frame():
     g = make_map("offframe", 2, 30, 40, False, seed=7)
     assert (np.abs(g) > 1.2).all()
+
+
+ADJ_SIZES = [  # (h, w, Ho, Wo): upsample, same size, downsample, 1 x w, h x 1, 1 x 1 lattices, Ho = 1, Wo = 1
+    (9, 13, 37, 53), (12, 17, 12, 17), (41, 61, 23, 29), (1, 19, 30, 40), (13, 1, 30, 40), (1, 1, 5, 7),
+    (13, 19, 1, 37), (13, 19, 29, 1), (6, 150, 50, 70)]
+
+
+def upsample_f64(lat, Ho, Wo, aligned):
+    """fp64 bilinear resize of a planar (N, 2, h, w) array with upsample_map's fp32 coefficients: a gather, written apart
+    from the oracle's scatter."""
+    (yi, yp, yl0, yl1), (xi, xp, xl0, xl1) = (oracle.upsample_coefs(lat.shape[2], Ho, aligned),
+                                              oracle.upsample_coefs(lat.shape[3], Wo, aligned))
+    r0, r1, c0, c1 = yi, yi + yp, xi, xi + xp
+    top = xl0.astype(np.float64) * lat[:, :, r0][..., c0] + xl1.astype(np.float64) * lat[:, :, r0][..., c1]
+    bot = xl0.astype(np.float64) * lat[:, :, r1][..., c0] + xl1.astype(np.float64) * lat[:, :, r1][..., c1]
+    return yl0.astype(np.float64)[:, None] * top + yl1.astype(np.float64)[:, None] * bot
+
+
+@pytest.mark.parametrize("mode", ["aligned", "half_pixel"])
+@pytest.mark.parametrize("size", ADJ_SIZES, ids=[f"{a}x{b}-{c}x{d}" for a, b, c, d in ADJ_SIZES])
+def test_upsample_adjoint_identity(mode, size):
+    """<U x, y> == <x, U^T y> in fp64, U the upsample with the forward's fp32 coefficients; the gather U x is the oracle's
+    fp32 forward up to its own rounding.  Also the term counts: 4 per output pixel, spread over the nodes."""
+    h, w, Ho, Wo = size
+    al = mode == "aligned"
+    rng = np.random.default_rng(h * 1000 + w)
+    x = rng.standard_normal((2, 2, h, w)).astype(F32).astype(np.float64)
+    y = rng.standard_normal((2, 2, Ho, Wo))
+    ux = upsample_f64(x, Ho, Wo, al)
+    np.testing.assert_allclose(ux, oracle.upsample_map(x.astype(F32), Ho, Wo, al), rtol=0, atol=4e-7 * np.abs(x).max())
+    uty, gabs, nterms = oracle.upsample_map_backward(y, h, w, al)
+    lhs, rhs = float((ux * y).sum()), float((x * uty).sum())
+    assert abs(lhs - rhs) <= 1e-12 * float((np.abs(ux) * np.abs(y)).sum() + (np.abs(x) * gabs).sum())
+    assert (nterms.sum(axis=(2, 3)) == 4 * Ho * Wo).all()
+    assert (gabs >= np.abs(uty)).all()
+
+
+@pytest.mark.parametrize("mode", ["aligned", "half_pixel"])
+@pytest.mark.parametrize("size", ADJ_SIZES, ids=[f"{a}x{b}-{c}x{d}" for a, b, c, d in ADJ_SIZES])
+def test_upsample_adjoint_matches_torch_interpolate(mode, size):
+    """Against autograd of F.interpolate in fp64 on the CPU.  torch computes the coefficients in fp64 here, the oracle in
+    fp32: a source index s < max(h, w) is off by at most 2 ulp of fp32 (scale, then fma / multiply), which moves each of
+    a node's terms by at most that times |y|."""
+    h, w, Ho, Wo = size
+    rng = np.random.default_rng(h * 7 + w)
+    y = rng.standard_normal((2, 2, Ho, Wo))
+    lat = torch.zeros((2, 2, h, w), dtype=torch.float64, requires_grad=True)
+    F.interpolate(lat, size=(Ho, Wo), mode="bilinear", align_corners=mode == "aligned").backward(torch.from_numpy(y))
+    got, _, nterms = oracle.upsample_map_backward(y, h, w, mode == "aligned")
+    tol = 4 * max(h, w) * 2.0 ** -23 * nterms * float(np.abs(y).max())
+    assert (np.abs(got - lat.grad.numpy()) <= tol).all()
+
+
+@pytest.mark.parametrize("base_align", [False, True])
+@pytest.mark.parametrize("size", BASE_SIZES, ids=[f"{h}x{w}" for h, w in BASE_SIZES])
+def test_theta_grad_matches_affine_grid_autograd(base_align, size):
+    """oracle.affine_theta_grad against the fp64 CPU autograd of F.affine_grid (torch's linspace differs from the fp32
+    base by its rounding); one item per N with its own theta."""
+    h, w = size
+    rng = np.random.default_rng(h * 31 + w)
+    N = 3
+    glat = rng.standard_normal((N, h, w, 2))
+    theta = torch.from_numpy(rng.standard_normal((N, 2, 3))).requires_grad_(True)
+    F.affine_grid(theta, (N, 1, h, w), align_corners=base_align).backward(torch.from_numpy(glat))
+    got, gabs = oracle.affine_theta_grad(glat, base_align)
+    assert np.abs(got - theta.grad.numpy()).max() <= 1e-6 * max(float(gabs.max()), 1.0)
+    # the forward base the gradient uses is the one affine_map composes
+    unit = oracle.affine_map(np.tile(np.array([[1, 0, 0], [0, 1, 0]], F32), (N, 1, 1)), h, w, None, base_align)
+    ones = np.zeros((N, h, w, 2))
+    ones[..., 0] = 1
+    gx, _ = oracle.affine_theta_grad(ones, base_align)
+    np.testing.assert_allclose(gx[:, 0, 0], unit[..., 0].astype(np.float64).sum((1, 2)), rtol=1e-12, atol=1e-12)
+
+
+@pytest.mark.parametrize("mode", ["aligned", "half_pixel"])
+@pytest.mark.parametrize("src,dst", [(256, 1080), (256, 1920), (4, 1920), (7, 20), (20, 16), (21, 16), (183, 64),
+                                     (150, 70), (1, 30), (9, 1), (13, 1), (1000, 3)])
+def test_census_coefficients_are_the_oracles(mode, src, dst):
+    """The census restates up_coef; it must give the C oracle's coefficients exactly (aligned: one fp32 multiply,
+    half_pixel: one fma)."""
+    al = mode == "aligned"
+    want = oracle.upsample_coefs(src, dst, al)
+    got = up_coef(np.arange(dst), src, up_scale(src, dst, al), al)
+    for g, w_, name in zip(got, want, ("i0", "ip", "l0", "l1")):
+        np.testing.assert_array_equal(np.asarray(g, w_.dtype), w_, err_msg=name)
+
+
+def test_backward_census_cases_reach_what_they_claim():
+    c = {case[-1]: backward_census(*case[:5]) for case in BWD_CASES}
+    nodes = lambda what: set(c[what]["nodes"].ravel().tolist())   # noqa: E731
+    assert nodes("window exactly full (1280)") == {1280}
+    assert nodes("full window and a clamped right tile") == {1280, 720}
+    one_call = c["window, per-pixel and window in one call (1281)"]
+    assert nodes("window, per-pixel and window in one call (1281)") == {1098, 1281, 732}
+    assert one_call["window"] == 2 and one_call["per_pixel"] == 1
+    assert nodes("per-pixel (1288) next to a window") == {1288, 720}
+    assert nodes("half_pixel window exactly full") == {1280}
+    assert nodes("half_pixel per-pixel") == {1344}
+    assert c["runs of 32 lanes, 1e5 terms per node"]["runs"].max() == 32
+    assert c["mw = 1: ip == 0 everywhere"]["ip0_runs"] == len(c["mw = 1: ip == 0 everywhere"]["runs"])
+    for what, half in (("Wo = 1 mod 64", 0), ("Wo = 31 mod 64", 0), ("Wo = 33 mod 64", 1), ("Wo = 63 mod 64", 1)):
+        assert c[what]["edge_lanes"][half] > 0, what
+    assert c["upsample in y, downsample in x: runs of one lane"]["runs"].min() == 1
+    every = {k: sum(v[k] for v in c.values()) for k in ("split", "ip0_runs", "per_pixel")}
+    assert all(every.values()), every
+    lengths = set(np.concatenate([v["runs"] for v in c.values()]).tolist())
+    assert {1, 32} <= lengths
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -603,7 +895,58 @@ def run_fused(pw, frame, drift, out_size, base="none", theta=None, base_align=Fa
     want = fused_sample_ref(host(frame), want_map, pad, align, pre, post, out.dtype)
     got = out.cpu().numpy() if out.dtype == torch.uint8 else host(out)
     np.testing.assert_array_equal(got, want, err_msg="fused sample")
+    if out.dtype.is_floating_point:    # a differentiable call: its backward too
+        check_fused_backward(frame, drift, out_size, base, theta, base_align, upsample, pad, align, pre, post)
     return out, emitted
+
+
+def grad_out_dtype(frame):
+    return frame.dtype if frame.dtype in (torch.float16, torch.bfloat16) else torch.float32
+
+
+def fused_backward_raw(frame, drift, gout, base="none", theta=None, base_align=False, upsample=None, pad="zeros",
+                       align=False, pre=OFF_PRE, post=OFF_POST, want_gin=True, map_size=None):
+    """pws_warp2d_backward_fused with caller-made buffers, each NaN-filled first (the library zero-fills or stores every
+    element): (rc, gin, glattice, gtheta, kernel).  gtheta is asked for with the affine base."""
+    from pwstablenet_b200 import _lib, compose
+    lib = _lib.load()
+    N = frame.size(0)
+    keep = []
+    spec = compose._spec(N, drift, base, theta, base_align, upsample, map_size, pre, post, keep)
+    nan = float("nan")
+    gin = torch.full(frame.shape, nan, dtype=torch.float32, device="cuda") if want_gin else None
+    glat = torch.full((N, spec.map_h, spec.map_w, 2), nan, dtype=torch.float32, device="cuda")
+    gtheta = torch.full((N, 2, 3), nan, dtype=torch.float32, device="cuda") if base == "affine" else None
+    rc = lib.pws_warp2d_backward_fused(ctypes.byref(compose._desc(gout)), ctypes.byref(compose._desc(frame)),
+                                       ctypes.byref(spec), ctypes.byref(compose._desc(gin)) if gin is not None else None,
+                                       ctypes.byref(compose._desc(glat)),
+                                       gtheta.data_ptr() if gtheta is not None else None, PAD[pad], int(align),
+                                       compose._stream(frame))
+    kernel = last_kernel()
+    torch.cuda.synchronize()
+    return rc, gin, glat, gtheta, kernel
+
+
+def check_fused_backward(frame, drift, out_size, base="none", theta=None, base_align=False, upsample=None, pad="zeros",
+                         align=False, pre=OFF_PRE, post=OFF_POST, want_gin=True, seed=0):
+    """The backward of a warp_fused call through the C entry point (a [-1, 1] grad_output of the frame's gradient dtype)
+    against FusedBackwardRef; every buffer NaN-filled first.  Returns the reference."""
+    from pwstablenet_b200 import _lib
+    N, C = frame.shape[:2]
+    gout = dev(synth.make_gout(N, C, *out_size, seed=seed) * F32(2) - F32(1), grad_out_dtype(frame))
+    want_gin = want_gin and frame.dtype != torch.uint8
+    rc, gin, glat, gtheta, kernel = fused_backward_raw(frame, drift, gout, base, theta, base_align, upsample, pad, align,
+                                                       pre, post, want_gin)
+    _lib.check(rc)
+    assert kernel == "bwd_fused"
+    ref = FusedBackwardRef(host(frame), host(drift).transpose(0, 3, 1, 2), base, None if theta is None else host(theta),
+                           base_align, upsample, host(gout), pad, align, pre, post)
+    check_glattice(host(glat), ref)
+    if base == "affine":
+        check_gtheta(host(gtheta), ref)
+    if want_gin:
+        check_gin(gin, ref)
+    return ref
 
 
 UP_SIZES = [  # (h, w, Ho, Wo, what)
@@ -637,8 +980,6 @@ def test_fused_upsample(pw, mode, size):
     assert torch.equal(emitted.permute(0, 3, 1, 2), ref)
 
 
-BASE_SIZES = [(1, 1), (1, 6), (6, 1), (2, 2), (2, 7), (16, 24), (37, 53)]   # 7, 16, 24, 37, 53: the two linspace halves
-                                                                            # round their middle node differently
 
 
 @gpu
@@ -766,6 +1107,186 @@ def test_fused_u8_fast_path_predicate(pw, upsample):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+# warp_fused backward: window and scan boundaries, autograd layouts and routing, the C entry's edges
+# ---------------------------------------------------------------------------------------------------------------------
+def rough_lattice(N, h, w, seed):
+    """planar (N, 2, h, w) float32 in [-1.1, 1.1]"""
+    return (np.random.default_rng(seed).random((N, 2, h, w), dtype=F32) * F32(2.2) - F32(1.1)).astype(F32)
+
+
+def affine_thetas(N, seed):
+    """(N, 2, 3) float32, a distinct theta per item near the identity"""
+    rng = np.random.default_rng(seed)
+    return (np.array([[1, 0, 0], [0, 1, 0]], F32)[None] + rng.standard_normal((N, 2, 3)).astype(F32) * F32(0.08))
+
+
+LATTICE_LAYOUTS = {"interleaved": lambda t: t, "planar": planar, "offset_by_one": offset_by_one}
+
+
+@gpu
+@pytest.mark.parametrize("case", BWD_CASES, ids=BWD_IDS)
+def test_fused_backward_window_and_scan(pw, case):
+    """The census cases (backward_census): shared-memory windows exactly full and one node over, both kinds of tile in
+    one call, runs of 1 and 32 lanes, ip == 0 columns, lanes past the right edge in either half of a tile row.  fp32 and
+    bf16 lattices, interleaved, planar (with the affine base: the window composes drift + base per node) and one element
+    into its buffer (lattice_map's scalar loads); with and without a frame gradient."""
+    mh, mw, Ho, Wo, upsample, _ = case
+    N, C, H, W = 2, 3, 30, 44
+    frame = dev(frames_pm1(N, C, H, W, seed=131))
+    lat = rough_lattice(N, mh, mw, seed=132)
+    theta = dev(affine_thetas(N, seed=133))
+    for lt in ("f32", "bf16"):
+        for layout, make in LATTICE_LAYOUTS.items():
+            base = "affine" if layout == "planar" else "none"
+            drift = make(dev(lat if base == "none" else lat * F32(0.05), DTYPES[lt]).permute(0, 2, 3, 1).contiguous())
+            for pad, align in PAD_ALIGN:
+                check_fused_backward(frame, drift, (Ho, Wo), base, theta if base == "affine" else None, align, upsample,
+                                     pad, align, PRE, POST, want_gin=pad == "zeros", seed=134)
+
+
+def fused_autograd_run(pw, frame, drift, theta, want, loss, **kw):
+    """pw.warp_fused under autograd with requires_grad per `want` (frame, drift, theta).  Returns (grads, the grad_output
+    the output received, the kernels the backward ran, read on autograd's device thread)."""
+    leaves = [t.detach().requires_grad_(w and t.is_floating_point()) if t is not None else None
+              for t, w in zip((frame, drift, theta), want)]
+    f, d, t = leaves
+    out = pw.warp_fused(f, drift=d, theta=t, **kw)
+    seen, kernels = [], []
+    out.register_hook(seen.append)
+    for x in leaves:
+        if x is not None and x.requires_grad:
+            x.register_hook(lambda g: kernels.append(last_kernel()))
+    loss(out).backward()
+    return [x.grad if x is not None else None for x in leaves], seen[0], kernels
+
+
+def check_autograd_grads(grads, want, ref, frame, drift, what):
+    fg, dg, tg = grads
+    if want[0] and frame.dtype != torch.uint8:
+        assert fg.dtype == frame.dtype and fg.shape == frame.shape, what
+        check_gin(fg, ref, extra_tol=float(torch.finfo(frame.dtype).eps) if frame.dtype != torch.float32 else 0.0)
+    else:
+        assert fg is None, what
+    if want[1]:
+        assert dg.dtype == drift.dtype and dg.shape == drift.shape, what
+        check_glattice(host(dg), ref, drift.dtype, what + ": drift")
+    else:
+        assert dg is None, what
+    if want[2]:
+        check_gtheta(host(tg), ref, what + ": theta")
+    else:
+        assert tg is None, what
+
+
+@gpu
+@pytest.mark.parametrize("layout", ["channels_last", "channel_slice", "window", "out_channels_last"])
+@pytest.mark.parametrize("dt,lt", [("f32", "f32"), ("bf16", "bf16"), ("f16", "f32")])
+def test_fused_autograd_layouts(pw, layout, dt, lt):
+    """Frame layouts, a channels-last output, and losses whose grad_output has all strides 0 (out.sum()) or a C stride of
+    0, through pw.warp_fused(...).backward."""
+    N, C, H, W, h, w, Ho, Wo = 2, 3, 34, 58, 11, 17, 29, 67
+    T, L = DTYPES[dt], DTYPES[lt]
+    frame = frame_layout(frames_pm1(N, C, H, W, seed=141), "contiguous" if layout == "out_channels_last" else layout, T)
+    drift = dev(rough_lattice(N, h, w, seed=142) * F32(0.05), L).permute(0, 2, 3, 1)      # planar storage
+    theta = dev(affine_thetas(N, seed=143))
+    wt = dev(synth.make_gout(N, C, Ho, Wo, seed=144), T)
+    w1 = dev(synth.make_gout(N, 1, Ho, Wo, seed=145)[:, 0], T)
+    losses = {"(out * w).sum()": lambda o: (o * wt).sum(), "out.sum()": lambda o: o.sum(),
+              "(out.sum(1) * w).sum()": lambda o: (o.sum(1) * w1).sum()}
+    kw = dict(base="affine", base_align_corners=True, upsample="half_pixel", out_size=(Ho, Wo), padding_mode="border",
+              align_corners=False, pre=PRE, post=POST, out_channels_last=layout == "out_channels_last")
+    for name, loss in losses.items():
+        grads, seen, kernels = fused_autograd_run(pw, frame, drift, theta, (True, True, True), loss, **kw)
+        assert kernels and set(kernels) == {"bwd_fused"}, (name, kernels)
+        if name == "out.sum()":
+            assert seen.stride() == (0, 0, 0, 0)
+        if name == "(out.sum(1) * w).sum()":
+            assert seen.stride(1) == 0
+        ref = FusedBackwardRef(host(frame), host(drift).transpose(0, 3, 1, 2), "affine", host(theta), True, "half_pixel",
+                               host(seen), "border", False, PRE, POST)
+        check_autograd_grads(grads, (True, True, True), ref, frame, drift, f"{layout}, {name}")
+
+
+@gpu
+@pytest.mark.parametrize("case", ["f32_n3", "u8_pre", "broadcast_drift"])
+@pytest.mark.parametrize("upsample", [None, "aligned"])
+def test_fused_autograd_routing(pw, case, upsample):
+    """Each combination of frame, drift and theta requiring grad (theta alone: glattice is internal and drift.grad None),
+    N = 3 with a distinct theta per item, checked per item; a uint8 frame with a pre scale; an N-broadcast drift, whose
+    gradient autograd sums over the N items."""
+    N, C, H, W, h, w = 3, 3, 26, 40, 9, 14
+    Ho, Wo = (h, w) if upsample is None else (23, 37)
+    lat = dev(rough_lattice(N, h, w, seed=151) * F32(0.05)).permute(0, 2, 3, 1).contiguous()
+    theta = dev(affine_thetas(N, seed=152))
+    gout = dev(synth.make_gout(N, C, Ho, Wo, seed=153) * F32(2) - F32(1))
+    loss = lambda o: (o * gout).sum()   # noqa: E731
+    pre = PRE
+    if case == "u8_pre":
+        frame = torch.from_numpy(np.random.default_rng(154).integers(0, 256, (N, H, W, C), dtype=np.uint8)).cuda()
+        frame, pre = frame.permute(0, 3, 1, 2), (-127.5, 1.0 / 127.5)
+    else:
+        frame = dev(frames_pm1(N, C, H, W, seed=154))
+    kw = dict(base="affine", upsample=upsample, out_size=(Ho, Wo), pre=pre, post=POST)
+    if case == "broadcast_drift":
+        one = lat[:1].clone()
+        for want_theta in (False, True):
+            leaf = one.detach().requires_grad_(True)
+            th = theta.detach().requires_grad_(want_theta)
+            pw.warp_fused(frame, drift=leaf.expand(N, h, w, 2), theta=th, **kw).backward(gout)
+            ref = FusedBackwardRef(host(frame), host(one.expand(N, h, w, 2)).transpose(0, 3, 1, 2), "affine",
+                                   host(theta), False, upsample, host(gout), "zeros", False, pre, POST)
+            got, want = host(leaf.grad)[0].astype(np.float64), ref.glat64.sum(0)
+            bound = ref.tol.sum(0) + (N - 1) * U * np.abs(ref.glat64).sum(0)   # + autograd's fp32 sum over the items
+            assert (np.abs(got - want) <= bound).all()
+            if want_theta:
+                check_gtheta(host(th.grad), ref)
+        return
+    ref = FusedBackwardRef(host(frame), host(lat).transpose(0, 3, 1, 2), "affine", host(theta), False, upsample,
+                           host(gout), "zeros", False, pre, POST)
+    wants = [(a, b, c) for a in (False, True) for b in (False, True) for c in (False, True) if a or b or c]
+    for want in wants:
+        if case == "u8_pre" and want == (True, False, False):
+            continue                     # a uint8 frame alone asks for no gradient: no backward runs
+        grads, _, kernels = fused_autograd_run(pw, frame, lat, theta, want, loss, **kw)
+        assert kernels and set(kernels) == {"bwd_fused"}, (want, kernels)
+        check_autograd_grads(grads, want, ref, frame, lat, f"{case}, requires_grad {want}")
+
+
+@gpu
+def test_fused_backward_c_entry_edges(pw):
+    """N = 0 and C = 0 leave defined (zero) gradients in NaN-filled buffers; N = 65536 and an output taller than
+    65535 tiles of 16 rows are PWS_EUNSUPPORTED and leave the buffers untouched."""
+    from pwstablenet_b200 import _lib
+    for N, C, base in ((2, 0, "affine"), (0, 3, "none")):      # (an empty theta has no pointer to hand over)
+        frame = torch.zeros((N, C, 5, 6), device="cuda")
+        drift = dev(np.zeros((N, 3, 4, 2), F32))
+        gout = torch.zeros((N, C, 7, 9), device="cuda")
+        rc, gin, glat, gtheta, _ = fused_backward_raw(frame, drift, gout, base, dev(affine_thetas(N, 161)),
+                                                      upsample="aligned")
+        assert rc == _lib.PWS_OK and gin.numel() == 0
+        assert glat.numel() == N * 24 and (glat == 0).all()
+        assert gtheta is None or (gtheta == 0).all()
+    # C = 0 through autograd: the (N, 0, H, W) grad_input torch allocates keeps strides (H*W, H*W, W, 1)
+    f = torch.zeros((2, 0, 5, 6), device="cuda", requires_grad=True)
+    d = torch.zeros((2, 3, 4, 2), device="cuda", requires_grad=True)
+    pw.warp_fused(f, drift=d, upsample="aligned", out_size=(7, 9)).sum().backward()
+    assert f.grad.shape == f.shape and d.grad.shape == d.shape and (d.grad == 0).all()
+    big = 65536
+    rc, gin, glat, gtheta, _ = fused_backward_raw(torch.zeros((big, 1, 1, 1), device="cuda"),
+                                                  torch.zeros((big, 2, 2, 2), device="cuda"),
+                                                  torch.zeros((big, 1, 2, 2), device="cuda"),
+                                                  theta=torch.zeros((big, 2, 3), device="cuda"), base="affine")
+    assert rc == _lib.PWS_EUNSUPPORTED
+    assert all(torch.isnan(t).all() for t in (gin, glat, gtheta))
+    tall = 65535 * 16 + 1
+    rc, gin, glat, _, _ = fused_backward_raw(torch.zeros((1, 1, 2, 2), device="cuda"),
+                                             torch.zeros((1, 2, 1, 2), device="cuda"),
+                                             torch.zeros((1, 1, tall, 1), device="cuda"), upsample="aligned")
+    assert rc == _lib.PWS_EUNSUPPORTED
+    assert torch.isnan(gin).all() and torch.isnan(glat).all()
+
+
+# ---------------------------------------------------------------------------------------------------------------------
 # the coverage table (host-side, no GPU needed)
 # ---------------------------------------------------------------------------------------------------------------------
 def coverage_report():
@@ -799,6 +1320,18 @@ def coverage_report():
         "C = 1..5; " + ", ".join(f"{a} -> {b}" for a, b in FUSED_IO) + "; NaN / inf / out-of-range uint8 stores")
     row("test_fused_u8_fast_path_predicate", "fwd_fused_u8, fwd_fused, compose_map", "noisy", "-",
         "padded batch, lattice one element in (fall back); expanded lattice (fast path)")
+    lines.append("")
+    lines.append("Every float-output call above also runs its backward (bwd_fused) against FusedBackwardRef.")
+    row("test_fused_backward_window_and_scan", "bwd_fused", "rough lattice; affine base on the planar layout", "-",
+        "the census cases below; f32 / bf16 lattices, interleaved, planar, one element in; with and without kGin")
+    row("test_fused_autograd_layouts", "bwd_fused", "affine + drift, half_pixel", "-",
+        "channels-last, channel slice, cropped window frames; channels-last output; grad_output strides 0 / C stride 0")
+    row("test_fused_autograd_routing", "bwd_fused", "affine + drift, none / aligned", "-",
+        "every requires_grad combination, N = 3 distinct thetas; uint8 frame with a pre scale; N-broadcast drift")
+    row("test_fused_backward_c_entry_edges", "-", "-", "-", "N = 0, C = 0 (zeros); N = 65536, > 65535 row tiles")
+    lines += ["", "| backward census case | lattice -> output | tiles and runs |", "|---|---|---|"]
+    for mh, mw, Ho, Wo, up, what in BWD_CASES:
+        lines.append(f"| {what} | {mh}x{mw} -> {Ho}x{Wo} {up} | {census_row(backward_census(mh, mw, Ho, Wo, up))} |")
     return "\n".join(lines)
 
 
