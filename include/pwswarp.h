@@ -27,6 +27,9 @@
  *   - asynchronous on `stream` (a cudaStream_t; NULL = legacy default stream)
  *   - return 0 on success, negative pws_status on failure; the message is in the
  *     thread-local pws_last_error()
+ *   - every tensor argument, the map spec's drift included, must live on the frame's
+ *     device (pws_compose_map: on map_out's device); theta / gtheta are raw pointers
+ *     the library cannot check
  *   - stateless and re-entrant
  */
 #ifndef PWSWARP_H_
@@ -106,6 +109,10 @@ int pws_warp2d_forward(const pws_tensor *in, const pws_tensor *grid, pws_tensor 
  * buffer; it does NOT need to arrive zeroed: the library zero-fills it itself,
  * frame by frame, just ahead of the scatter so the lines are still in L2 when
  * the atomics land (DESIGN.md "backward").  ggrid is fully overwritten.
+ * With C = 0 nothing flows back: gin and ggrid are zero-filled, as ATen returns them.
+ * That takes one memset over each buffer, so ggrid must then be dense in some order of
+ * its dims (interleaved, or the planar-permuted layout); any other layout is
+ * PWS_EUNSUPPORTED.  gin may keep any strides when it is empty (N*C = 0).
  * Accepts every (frame, map) dtype pair pws_warp2d_forward accepts, any strides and C:
  *     frame / gout   map / ggrid     gin
  *     f32            f32             f32
@@ -182,7 +189,8 @@ int pws_warp2d_forward_fused(const pws_tensor *in, const pws_map_spec *spec, pws
  * The map is recomputed with the forward's statements (same taps); go = gout / post_div (a true division, as the forward
  * divides); grad_grid follows ATen's statement order on the pre-scaled taps; fp32 throughout.  Without upsample glattice
  * equals pws_warp2d_backward's grad_grid of the composed map bit for bit; with upsample it is that grad_grid pushed
- * through the upsample's adjoint, summed with atomics (order-dependent in the last bits). */
+ * through the upsample's adjoint, summed with atomics (order-dependent in the last bits).  With C = 0 every output given
+ * is zero-filled. */
 int pws_warp2d_backward_fused(const pws_tensor *gout, const pws_tensor *in, const pws_map_spec *spec,
                               pws_tensor *gin, pws_tensor *glattice, float *gtheta,
                               int padding, int align_corners, void *stream);
@@ -199,6 +207,7 @@ int pws_compose_map(const pws_map_spec *spec, int64_t n, pws_tensor *map_out, vo
  *     outs[k]   = sample((in + pre_add) * pre_mul, grids[k]) * (1 / post_div) + post_add        k < n_stages <= 4
  *     ggrids[k] = d outs[k] / d grids[k] applied to gouts[k]      (entries may be NULL)
  *     gin       = sum_k d outs[k] / d in applied to gouts[k]      (may be NULL; dense NCHW, zero-filled by the library)
+ * With C = 0, gin and every ggrids[k] are zero-filled, under pws_warp2d_backward's layout rule for ggrid.
  * C in {1, 3}, any strides.  `1 / post_div` is the rounded fp32 reciprocal torch's `tensor / scalar` multiplies by, so
  * the results equal the reference's sequence of torch calls bit for bit.  (0, 1, 1, 0) switches the scales off.
  * dtypes (all grids share one dtype; anything else is PWS_EINVAL):

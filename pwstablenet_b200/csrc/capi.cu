@@ -27,6 +27,8 @@ void set_error(const char *fmt, ...)
     va_end(ap);
 }
 
+#define PWS_TRY(expr) do { int rc_ = (expr); if (rc_ != PWS_OK) return rc_; } while (0)
+
 namespace {
 
 int elem_size(int dt)
@@ -53,26 +55,76 @@ int64_t item_span(const pws_tensor *t)
     return s;
 }
 
-int make_view(const pws_tensor *t, const char *what, View *v)
+const char *dtype_name(int dt)
 {
-    if (!t) { set_error("%s: null tensor descriptor", what); return PWS_EINVAL; }
-    if (elem_size(t->dtype) == 0) { set_error("%s: unknown dtype %d", what, t->dtype); return PWS_EINVAL; }
+    static const char *const names[] = {"f32", "f16", "bf16", "f64", "u8", "i32"};
+    return elem_size(dt) ? names[dt] : "?";
+}
+
+// set_error with the argument's name in front: "grad_grid: ..." or, for stage k's tensors, "grad_grid 1: ..."
+int arg_error(int rc, const char *what, int k, const char *fmt, ...)
+{
+    int n = k < 0 ? snprintf(g_err, sizeof(g_err), "%s: ", what) : snprintf(g_err, sizeof(g_err), "%s %d: ", what, k);
+    if (n < 0 || n >= (int)sizeof(g_err)) n = 0;
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(g_err + n, sizeof(g_err) - n, fmt, ap);
+    va_end(ap);
+    return rc;
+}
+
+int make_view(const pws_tensor *t, const char *what, int k, View *v)
+{
+    if (!t) return arg_error(PWS_EINVAL, what, k, "null tensor descriptor");
+    if (elem_size(t->dtype) == 0) return arg_error(PWS_EINVAL, what, k, "unknown dtype %d", t->dtype);
     for (int d = 0; d < 4; ++d) {
-        if (t->size[d] < 0) { set_error("%s: negative size", what); return PWS_EINVAL; }
-        if (t->stride[d] < 0) { set_error("%s: negative strides are not supported", what); return PWS_EUNSUPPORTED; }
-        if (t->size[d] > INT_MAX) { set_error("%s: dimension %d too large", what, d); return PWS_EUNSUPPORTED; }
+        if (t->size[d] < 0) return arg_error(PWS_EINVAL, what, k, "negative size");
+        if (t->stride[d] < 0) return arg_error(PWS_EUNSUPPORTED, what, k, "negative strides are not supported");
+        if (t->size[d] > INT_MAX) return arg_error(PWS_EUNSUPPORTED, what, k, "dimension %d too large", d);
     }
-    if (item_span(t) >= ((int64_t)1 << 31)) {
-        set_error("%s: one batch item spans >= 2^31 elements (32-bit in-frame offsets)", what);
-        return PWS_EUNSUPPORTED;
-    }
+    if (item_span(t) >= ((int64_t)1 << 31))
+        return arg_error(PWS_EUNSUPPORTED, what, k, "one batch item spans >= 2^31 elements (32-bit in-frame offsets)");
     const int64_t numel = t->size[0] * t->size[1] * t->size[2] * t->size[3];
-    if (numel > 0 && !t->data) { set_error("%s: null data pointer", what); return PWS_EINVAL; }
+    if (numel > 0 && !t->data) return arg_error(PWS_EINVAL, what, k, "null data pointer");
     v->p = t->data;
     v->sN = t->stride[0];
     v->s1 = (int32_t)t->stride[1];
     v->s2 = (int32_t)t->stride[2];
     v->s3 = (int32_t)t->stride[3];
+    return PWS_OK;
+}
+
+constexpr int64_t kAny = -1;   // check_arg: any size, dtype or device
+
+// One tensor argument: present, a valid view, sizes (a, b, c, d), `dtype` and memory on device `dev`; kAny skips a check.
+int check_arg(const pws_tensor *t, const char *what, int k, int64_t a, int64_t b, int64_t c, int64_t d, int dtype, int dev,
+              View *v)
+{
+    PWS_TRY(make_view(t, what, k, v));
+    const int64_t want[4] = {a, b, c, d};
+    for (int i = 0; i < 4; ++i)
+        if (want[i] != kAny && t->size[i] != want[i])
+            return arg_error(PWS_EINVAL, what, k, "expected sizes [%lld, %lld, %lld, %lld], got [%lld, %lld, %lld, %lld] "
+                             "(batch/channels or spatial sizes differ from the call's)", (long long)a, (long long)b,
+                             (long long)c, (long long)d, (long long)t->size[0], (long long)t->size[1],
+                             (long long)t->size[2], (long long)t->size[3]);
+    if (dtype != kAny && t->dtype != dtype)
+        return arg_error(PWS_EINVAL, what, k, "expected dtype %s, got %s", dtype_name(dtype), dtype_name(t->dtype));
+    if (dev != kAny && t->device != dev) return arg_error(PWS_EINVAL, what, k, "expected device cuda:%d, got cuda:%d", dev, t->device);
+    return PWS_OK;
+}
+
+// grad_input: the dense (N,C,H,W) buffer the library zero-fills and scatters into, on the frame's device; f32 (16-bit frames
+// accumulate in fp32) or f64 for f64 frames.  An empty buffer (N*C = 0) is dense whatever its strides: torch keeps
+// (H*W, H*W, W, 1) for C = 0.
+int check_gin(const pws_tensor *gin, const pws_tensor *in, View *v)
+{
+    const int64_t Nb = in->size[0], C = in->size[1], H = in->size[2], W = in->size[3];
+    PWS_TRY(check_arg(gin, "grad_input", -1, Nb, C, H, W, in->dtype == PWS_F64 ? PWS_F64 : PWS_F32, in->device, v));
+    const bool dense = Nb * C == 0 || (gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
+                                        (gin->stride[0] == C * H * W || Nb <= 1));
+    if (!dense) return arg_error(PWS_EINVAL, "grad_input", -1, "must be (N,C,H,W)-contiguous (the library zero-fills it)");
+    v->sN = C * H * W;
     return PWS_OK;
 }
 
@@ -88,6 +140,17 @@ int check_modes(int interp, int padding)
         set_error("pwswarp: padding_mode='reflection' is not implemented (zeros and border only)");
         return PWS_EUNSUPPORTED;
     }
+    return PWS_OK;
+}
+
+int check_spatial(const pws_tensor *in)
+{
+    for (int d = 2; d < 4; ++d)
+        if (in->size[d] <= 0) {
+            set_error("grid_sampler(): expected input to have non-empty spatial dimensions, but input has sizes [%lld, %lld, %lld, %lld] with dimension %d being empty",
+                      (long long)in->size[0], (long long)in->size[1], (long long)in->size[2], (long long)in->size[3], d);
+            return PWS_EINVAL;
+        }
     return PWS_OK;
 }
 
@@ -110,32 +173,25 @@ int check_pair(const pws_tensor *in, const pws_tensor *grid)
                   (long long)grid->size[0], (long long)grid->size[1], (long long)grid->size[2], (long long)grid->size[3]);
         return PWS_EINVAL;
     }
-    for (int d = 2; d < 4; ++d)
-        if (in->size[d] <= 0) {
-            set_error("grid_sampler(): expected input to have non-empty spatial dimensions, but input has sizes [%lld, %lld, %lld, %lld] with dimension %d being empty",
-                      (long long)in->size[0], (long long)in->size[1], (long long)in->size[2], (long long)in->size[3], d);
-            return PWS_EINVAL;
-        }
-    return PWS_OK;
+    return check_spatial(in);
 }
 
-int fill_geometry(const pws_tensor *in, const pws_tensor *grid, int padding, int align, Geometry *g)
+// frame: (N, C, H, W) sizes; (Ho, Wo): the output / map size
+Geometry geometry(const int64_t (&frame)[4], int64_t Ho, int64_t Wo, int padding, int align)
 {
-    g->N = (int32_t)in->size[0]; g->C = (int32_t)in->size[1];
-    g->H = (int32_t)in->size[2]; g->W = (int32_t)in->size[3];
-    g->Ho = (int32_t)grid->size[1]; g->Wo = (int32_t)grid->size[2];
-    g->padding = padding; g->align = align ? 1 : 0;
-    return PWS_OK;
+    Geometry g;
+    g.N = (int32_t)frame[0]; g.C = (int32_t)frame[1]; g.H = (int32_t)frame[2]; g.W = (int32_t)frame[3];
+    g.Ho = (int32_t)Ho; g.Wo = (int32_t)Wo;
+    g.padding = padding; g.align = align ? 1 : 0;
+    return g;
 }
 
-int same_shape(const pws_tensor *t, int64_t a, int64_t b, int64_t c, int64_t d, const char *what)
+// Whether a (pre_add, pre_mul, post_div, post_add) scale does anything before and after the sample; post_div must not be 0.
+int scale_flags(float pre_add, float pre_mul, float post_div, float post_add, const char *what, int *has_pre, int *has_post)
 {
-    if (t->size[0] != a || t->size[1] != b || t->size[2] != c || t->size[3] != d) {
-        set_error("%s: expected sizes [%lld, %lld, %lld, %lld], got [%lld, %lld, %lld, %lld]", what,
-                  (long long)a, (long long)b, (long long)c, (long long)d,
-                  (long long)t->size[0], (long long)t->size[1], (long long)t->size[2], (long long)t->size[3]);
-        return PWS_EINVAL;
-    }
+    if (post_div == 0.0f) { set_error("%s: post_div must not be 0", what); return PWS_EINVAL; }
+    *has_pre = !(pre_add == 0.0f && pre_mul == 1.0f);
+    *has_post = !(post_div == 1.0f && post_add == 0.0f);
     return PWS_OK;
 }
 
@@ -150,25 +206,70 @@ struct DeviceGuard {
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
-int finish(const char *what)
+// Runs launch() with `dev` selected (the caller's device is restored after) and reports its launch error as `what`'s.
+template <class Launch>
+int on_device(int dev, const char *what, Launch &&launch)
 {
+    DeviceGuard dg(dev);
+    if (!dg.ok) { set_error("%s: cannot select cuda:%d", what, dev); return PWS_ECUDA; }
+    PWS_TRY(launch());
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { set_error("%s: kernel launch failed: %s", what, cudaGetErrorString(e)); return PWS_ECUDA; }
     return PWS_OK;
 }
 
-}  // namespace
-}  // namespace pws
+// Elements of a buffer that fills its span exactly, with no gap and no overlap, its dims in any stride order (so the
+// planar-permuted maps torch hands over qualify); -1 for any other layout.
+int64_t dense_numel(const pws_tensor *t)
+{
+    int64_t numel = 1, st[4], sz[4];
+    int n = 0;
+    for (int d = 0; d < 4; ++d) {
+        numel *= t->size[d];
+        if (t->size[d] == 1) continue;
+        int i = n++;   // insertion by stride
+        for (; i > 0 && st[i - 1] > t->stride[d]; --i) { st[i] = st[i - 1]; sz[i] = sz[i - 1]; }
+        st[i] = t->stride[d]; sz[i] = t->size[d];
+    }
+    if (numel == 0) return 0;
+    int64_t expected = 1;
+    for (int i = 0; i < n; expected *= sz[i++])
+        if (st[i] != expected) return -1;
+    return numel;
+}
 
-namespace pws {
+// A backward with nothing to scatter (N*C*Ho*Wo == 0): every gradient the caller passed is defined and zero, as ATen
+// returns it.  The buffers are dense (grad_input and glattice by their rules), so each takes one memset over its span.
+int zero_grads(int dev, const char *what, cudaStream_t st, const pws_tensor *gin, const pws_tensor *const *ggrids, int K,
+               bool staged, const pws_tensor *glattice, float *gtheta, int64_t N)
+{
+    if (N == 0) return PWS_OK;
+    for (int k = 0; k < K; ++k)
+        if (ggrids[k] && dense_numel(ggrids[k]) < 0)
+            return arg_error(PWS_EUNSUPPORTED, "grad_grid", staged ? k : -1,
+                             "with C = 0 the library zero-fills it, which needs a buffer without gaps");
+    return on_device(dev, what, [&] {
+        cudaError_t e = cudaSuccess;
+        auto zero = [&](const pws_tensor *t) {
+            if (t && e == cudaSuccess) e = cudaMemsetAsync(t->data, 0, (size_t)dense_numel(t) * elem_size(t->dtype), st);
+        };
+        zero(gin);
+        for (int k = 0; k < K; ++k) zero(ggrids[k]);
+        zero(glattice);
+        if (gtheta && e == cudaSuccess) e = cudaMemsetAsync(gtheta, 0, (size_t)N * 6 * sizeof(float), st);
+        if (e != cudaSuccess) { set_error("%s: cudaMemsetAsync: %s", what, cudaGetErrorString(e)); return (int)PWS_ECUDA; }
+        return (int)PWS_OK;
+    });
+}
+
+}  // namespace
+
 static int make_scale(float pre_add, float pre_mul, float post_div, float post_add, StageScale *sc)
 {
-    if (post_div == 0.0f) { set_error("stages: post_div must not be 0"); return PWS_EINVAL; }
+    PWS_TRY(scale_flags(pre_add, pre_mul, post_div, post_add, "stages", &sc->has_pre, &sc->has_post));
     sc->pre_add = pre_add; sc->pre_mul = pre_mul;
     sc->post_mul = 1.0f / post_div;   // fp32 division: the reciprocal torch's `tensor / scalar` kernel multiplies by
     sc->post_add = post_add;
-    sc->has_pre = !(pre_add == 0.0f && pre_mul == 1.0f);
-    sc->has_post = !(post_div == 1.0f && post_add == 0.0f);
     return PWS_OK;
 }
 
@@ -189,13 +290,31 @@ static int check_stage_dtypes(const pws_tensor *in, const pws_tensor *const *gri
     return PWS_OK;
 }
 
+// The per-stage arguments of warp_stages: K maps of one size, and each stage's output (forward) or grad_output and optional
+// grad_grid (backward; ggrids == nullptr for the forward).
+static int check_stages(const pws_tensor *in, const pws_tensor *const *grids, const pws_tensor *const *io, const char *io_what,
+                        const pws_tensor *const *ggrids, int K, const char *what, StageViews *sv)
+{
+    if (K < 1 || K > kMaxStages) { set_error("%s: n_stages must be 1..%d", what, kMaxStages); return PWS_EINVAL; }
+    PWS_TRY(check_stage_dtypes(in, grids, K, what));
+    const int64_t Nb = in->size[0], Ho = grids[0]->size[1], Wo = grids[0]->size[2];
+    for (int k = 0; k < K; ++k) {
+        PWS_TRY(check_pair(in, grids[k]));
+        PWS_TRY(check_arg(grids[k], "grid", k, Nb, Ho, Wo, 2, kAny, in->device, &sv->map[k]));
+        PWS_TRY(check_arg(io[k], io_what, k, Nb, in->size[1], Ho, Wo, in->dtype, in->device, &sv->io[k]));
+        if (ggrids && ggrids[k]) PWS_TRY(check_arg(ggrids[k], "grad_grid", k, Nb, Ho, Wo, 2, grids[k]->dtype, in->device, &sv->gg[k]));
+    }
+    return PWS_OK;
+}
+
 int launch_forward_fused(const View &in, int in_dtype, const MapSpec &m, const View &out, int out_dtype,
                          const Geometry &g, cudaStream_t st);
 int launch_compose_map(const MapSpec &m, const View &out, int N, int Ho, int Wo, cudaStream_t st);
 int launch_backward_fused(const View &gout, const View &in, int in_dtype, const MapSpec &m, const View &gin, bool want_gin,
                           float *glat, float *gtheta, const Geometry &g, cudaStream_t st);
 
-static int make_spec(const pws_map_spec *spec, int64_t N, int64_t Ho, int64_t Wo, MapSpec *m)
+// dev: the call's device, where the drift must live
+static int make_spec(const pws_map_spec *spec, int64_t N, int64_t Ho, int64_t Wo, int dev, MapSpec *m)
 {
     if (!spec) { set_error("map spec: null"); return PWS_EINVAL; }
     if (spec->base < 0 || spec->base > 2 || spec->upsample < 0 || spec->upsample > 2) { set_error("map spec: bad base/upsample enum"); return PWS_EINVAL; }
@@ -206,11 +325,7 @@ static int make_spec(const pws_map_spec *spec, int64_t N, int64_t Ho, int64_t Wo
         const int dt = spec->drift->dtype;
         if (dt != PWS_F32 && dt != PWS_F16 && dt != PWS_BF16) { set_error("map spec: drift must be f32, f16 or bf16"); return PWS_EUNSUPPORTED; }
         m->drift_dtype = dt;
-        if (spec->drift->size[0] != N || spec->drift->size[1] != spec->map_h || spec->drift->size[2] != spec->map_w || spec->drift->size[3] != 2) {
-            set_error("map spec: drift must have sizes [N, map_h, map_w, 2]"); return PWS_EINVAL;
-        }
-        int rc = make_view(spec->drift, "drift", &m->drift);
-        if (rc != PWS_OK) return rc;
+        PWS_TRY(check_arg(spec->drift, "drift", -1, N, spec->map_h, spec->map_w, 2, kAny, dev, &m->drift));
     } else if (spec->base == PWS_BASE_NONE) { set_error("map spec: no drift and no base"); return PWS_EINVAL; }
     if (spec->base == PWS_BASE_AFFINE && !spec->theta) { set_error("map spec: affine base needs theta"); return PWS_EINVAL; }
     if (spec->upsample == PWS_UP_NONE && (spec->map_h != Ho || spec->map_w != Wo)) {
@@ -218,19 +333,15 @@ static int make_spec(const pws_map_spec *spec, int64_t N, int64_t Ho, int64_t Wo
                   (long long)spec->map_h, (long long)spec->map_w, (long long)Ho, (long long)Wo);
         return PWS_EINVAL;
     }
+    PWS_TRY(scale_flags(spec->pre_add, spec->pre_mul, spec->post_div, spec->post_add, "map spec", &m->has_pre, &m->has_post));
     m->theta = spec->theta; m->base = spec->base; m->base_align = spec->base_align_corners ? 1 : 0;
     m->upsample = spec->upsample; m->mh = (int)spec->map_h; m->mw = (int)spec->map_w;
     m->pre_add = spec->pre_add; m->pre_mul = spec->pre_mul; m->post_div = spec->post_div; m->post_add = spec->post_add;
-    m->has_pre = !(spec->pre_add == 0.0f && spec->pre_mul == 1.0f);
-    m->has_post = !(spec->post_div == 1.0f && spec->post_add == 0.0f);
-    if (spec->post_div == 0.0f) { set_error("map spec: post_div must not be 0"); return PWS_EINVAL; }
     return PWS_OK;
 }
 }  // namespace pws
 
 using namespace pws;
-
-#define PWS_TRY(expr) do { int rc_ = (expr); if (rc_ != PWS_OK) return rc_; } while (0)
 
 extern "C" {
 
@@ -254,21 +365,14 @@ int pws_warp2d_forward(const pws_tensor *in, const pws_tensor *grid, pws_tensor 
 {
     PWS_TRY(check_modes(interp, padding));
     PWS_TRY(check_pair(in, grid));
-    if (!out) { set_error("forward: null output descriptor"); return PWS_EINVAL; }
     Problem pb{};
-    PWS_TRY(make_view(in, "input", &pb.in));
-    PWS_TRY(make_view(grid, "grid", &pb.grid));
-    PWS_TRY(make_view(out, "output", &pb.out));
-    PWS_TRY(same_shape(out, in->size[0], in->size[1], grid->size[1], grid->size[2], "output"));
-    if (out->dtype != in->dtype) { set_error("output: dtype must equal the input's"); return PWS_EINVAL; }
-    if (out->device != in->device) { set_error("output: must be on the input's device"); return PWS_EINVAL; }
-    fill_geometry(in, grid, padding, align_corners, &pb.g);
+    PWS_TRY(make_view(in, "input", -1, &pb.in));
+    PWS_TRY(make_view(grid, "grid", -1, &pb.grid));
+    const Geometry &g = pb.g = geometry(in->size, grid->size[1], grid->size[2], padding, align_corners);
+    PWS_TRY(check_arg(out, "output", -1, g.N, g.C, g.Ho, g.Wo, in->dtype, in->device, &pb.out));
     pb.in_dtype = in->dtype; pb.grid_dtype = grid->dtype;
-    if ((int64_t)pb.g.N * pb.g.C * pb.g.Ho * pb.g.Wo == 0) return PWS_OK;
-    DeviceGuard dg(in->device);
-    if (!dg.ok) { set_error("forward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    PWS_TRY(launch_forward(pb, (cudaStream_t)stream));
-    return finish("forward");
+    if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0) return PWS_OK;
+    return on_device(in->device, "forward", [&] { return launch_forward(pb, (cudaStream_t)stream); });
 }
 
 __attribute__((visibility("default")))
@@ -278,52 +382,19 @@ int pws_warp2d_backward(const pws_tensor *gout, const pws_tensor *in, const pws_
 {
     PWS_TRY(check_modes(interp, padding));
     PWS_TRY(check_pair(in, grid));
-    if (!gout) { set_error("backward: null grad_output descriptor"); return PWS_EINVAL; }
     Problem pb{};
-    PWS_TRY(make_view(in, "input", &pb.in));
-    PWS_TRY(make_view(grid, "grid", &pb.grid));
-    PWS_TRY(make_view(gout, "grad_output", &pb.gout));
-    PWS_TRY(same_shape(gout, in->size[0], in->size[1], grid->size[1], grid->size[2], "grad_output"));
-    if (gout->dtype != in->dtype) { set_error("grad_output: dtype must equal the input's"); return PWS_EINVAL; }
-    if (gout->device != in->device) { set_error("grad_output: must be on the input's device"); return PWS_EINVAL; }
+    PWS_TRY(make_view(in, "input", -1, &pb.in));
+    PWS_TRY(make_view(grid, "grid", -1, &pb.grid));
+    const Geometry &g = pb.g = geometry(in->size, grid->size[1], grid->size[2], padding, align_corners);
+    PWS_TRY(check_arg(gout, "grad_output", -1, g.N, g.C, g.Ho, g.Wo, in->dtype, in->device, &pb.gout));
+    if (gin) PWS_TRY(check_gin(gin, in, &pb.gin));
+    if (ggrid) PWS_TRY(check_arg(ggrid, "grad_grid", -1, g.N, g.Ho, g.Wo, 2, grid->dtype, in->device, &pb.ggrid));
     pb.want_gin = gin != nullptr;
     pb.want_ggrid = ggrid != nullptr;
-    if (gin) {
-        PWS_TRY(make_view(gin, "grad_input", &pb.gin));
-        PWS_TRY(same_shape(gin, in->size[0], in->size[1], in->size[2], in->size[3], "grad_input"));
-        // 16-bit frames: grad_input is an fp32 accumulation buffer that the caller rounds once (see launch_16bit)
-        const bool half_in = in->dtype == PWS_F16 || in->dtype == PWS_BF16;
-        if ((half_in ? gin->dtype != PWS_F32 : gin->dtype != in->dtype) || gin->device != in->device) {
-            set_error(half_in ? "grad_input: 16-bit frames accumulate into an f32 (N,C,H,W) buffer on the input's device"
-                              : "grad_input: dtype/device must equal the input's");
-            return PWS_EINVAL;
-        }
-        const int64_t C = in->size[1], H = in->size[2], W = in->size[3];
-        const bool dense = gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
-                           (gin->stride[0] == C * H * W || in->size[0] <= 1);
-        if (!dense) { set_error("grad_input: must be (N,C,H,W)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
-        pb.gin.sN = C * H * W;
-    }
-    if (ggrid) {
-        PWS_TRY(make_view(ggrid, "grad_grid", &pb.ggrid));
-        PWS_TRY(same_shape(ggrid, grid->size[0], grid->size[1], grid->size[2], 2, "grad_grid"));
-        if (ggrid->dtype != grid->dtype || ggrid->device != in->device) { set_error("grad_grid: dtype/device must equal the grid's"); return PWS_EINVAL; }
-    }
-    fill_geometry(in, grid, padding, align_corners, &pb.g);
     pb.in_dtype = in->dtype; pb.grid_dtype = grid->dtype;
-    DeviceGuard dg(in->device);
-    if (!dg.ok) { set_error("backward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    if (pb.g.N == 0) return PWS_OK;
-    if ((int64_t)pb.g.C * pb.g.Ho * pb.g.Wo == 0) {
-        // nothing scatters; grad_input is still defined (all zeros)
-        if (gin && (int64_t)pb.g.C * pb.g.H * pb.g.W > 0) {
-            cudaError_t e = cudaMemsetAsync(gin->data, 0, (size_t)(in->size[0] * pb.gin.sN * elem_size(gin->dtype)), (cudaStream_t)stream);
-            if (e != cudaSuccess) { set_error("backward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return PWS_ECUDA; }
-        }
-        return PWS_OK;
-    }
-    PWS_TRY(launch_backward(pb, (cudaStream_t)stream));
-    return finish("backward");
+    const cudaStream_t st = (cudaStream_t)stream;
+    if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0) return zero_grads(in->device, "backward", st, gin, &ggrid, 1, false, nullptr, nullptr, g.N);
+    return on_device(in->device, "backward", [&] { return launch_backward(pb, st); });
 }
 
 __attribute__((visibility("default")))
@@ -337,15 +408,10 @@ int pws_warp2d_taps(const pws_tensor *grid, int64_t in_h, int64_t in_w,
     if (grid->size[3] != 2) { set_error("taps: grid must have size 2 in its last dimension"); return PWS_EINVAL; }
     if (in_h <= 0 || in_w <= 0 || in_h > INT_MAX || in_w > INT_MAX) { set_error("taps: bad frame size"); return PWS_EINVAL; }
     View gv;
-    PWS_TRY(make_view(grid, "grid", &gv));
-    Geometry g{};
-    g.N = (int32_t)grid->size[0]; g.C = 1; g.H = (int32_t)in_h; g.W = (int32_t)in_w;
-    g.Ho = (int32_t)grid->size[1]; g.Wo = (int32_t)grid->size[2];
-    g.padding = padding; g.align = align_corners ? 1 : 0;
-    DeviceGuard dg(grid->device);
-    if (!dg.ok) { set_error("taps: cannot select cuda:%d", grid->device); return PWS_ECUDA; }
-    PWS_TRY(launch_taps(gv, g, x0, y0, mask, weights, (cudaStream_t)stream));
-    return finish("taps");
+    PWS_TRY(make_view(grid, "grid", -1, &gv));
+    const int64_t frame[4] = {grid->size[0], 1, in_h, in_w};
+    const Geometry g = geometry(frame, grid->size[1], grid->size[2], padding, align_corners);
+    return on_device(grid->device, "taps", [&] { return launch_taps(gv, g, x0, y0, mask, weights, (cudaStream_t)stream); });
 }
 
 __attribute__((visibility("default")))
@@ -353,24 +419,16 @@ int pws_warp2d_forward_fused(const pws_tensor *in, const pws_map_spec *spec, pws
                              int padding, int align_corners, void *stream)
 {
     PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
-    if (!in || !out) { set_error("fused forward: null tensor descriptor"); return PWS_EINVAL; }
-    for (int d = 2; d < 4; ++d)
-        if (in->size[d] <= 0) { set_error("grid_sampler(): expected input to have non-empty spatial dimensions"); return PWS_EINVAL; }
-    if (out->size[0] != in->size[0] || out->size[1] != in->size[1]) { set_error("fused forward: output batch/channels must equal the input's"); return PWS_EINVAL; }
-    if (out->device != in->device) { set_error("fused forward: output must be on the input's device"); return PWS_EINVAL; }
     View vin, vout;
-    PWS_TRY(make_view(in, "input", &vin));
-    PWS_TRY(make_view(out, "output", &vout));
+    PWS_TRY(make_view(in, "input", -1, &vin));
+    PWS_TRY(check_spatial(in));
+    PWS_TRY(check_arg(out, "output", -1, in->size[0], in->size[1], kAny, kAny, kAny, in->device, &vout));
+    const Geometry g = geometry(in->size, out->size[2], out->size[3], padding, align_corners);
     MapSpec m;
-    PWS_TRY(make_spec(spec, in->size[0], out->size[2], out->size[3], &m));
-    Geometry g{};
-    g.N = (int32_t)in->size[0]; g.C = (int32_t)in->size[1]; g.H = (int32_t)in->size[2]; g.W = (int32_t)in->size[3];
-    g.Ho = (int32_t)out->size[2]; g.Wo = (int32_t)out->size[3]; g.padding = padding; g.align = align_corners ? 1 : 0;
+    PWS_TRY(make_spec(spec, g.N, g.Ho, g.Wo, in->device, &m));
     if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0) return PWS_OK;
-    DeviceGuard dg(in->device);
-    if (!dg.ok) { set_error("fused forward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    PWS_TRY(launch_forward_fused(vin, in->dtype, m, vout, out->dtype, g, (cudaStream_t)stream));
-    return finish("fused forward");
+    return on_device(in->device, "fused forward",
+                     [&] { return launch_forward_fused(vin, in->dtype, m, vout, out->dtype, g, (cudaStream_t)stream); });
 }
 
 __attribute__((visibility("default")))
@@ -379,83 +437,51 @@ int pws_warp2d_backward_fused(const pws_tensor *gout, const pws_tensor *in, cons
                               int padding, int align_corners, void *stream)
 {
     PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
-    if (!in || !gout) { set_error("fused backward: null tensor descriptor"); return PWS_EINVAL; }
-    for (int d = 2; d < 4; ++d)
-        if (in->size[d] <= 0) { set_error("grid_sampler(): expected input to have non-empty spatial dimensions"); return PWS_EINVAL; }
-    if (gout->size[0] != in->size[0] || gout->size[1] != in->size[1]) { set_error("fused backward: grad_output batch/channels must equal the input's"); return PWS_EINVAL; }
-    if (gout->device != in->device) { set_error("fused backward: grad_output must be on the input's device"); return PWS_EINVAL; }
+    View vin, vgout, vgin{}, vglat{};
+    PWS_TRY(make_view(in, "input", -1, &vin));
+    PWS_TRY(check_spatial(in));
     const bool half_in = in->dtype == PWS_F16 || in->dtype == PWS_BF16;
     if (in->dtype != PWS_F32 && in->dtype != PWS_U8 && !half_in) { set_error("fused backward: frames must be f32, f16, bf16 or uint8"); return PWS_EUNSUPPORTED; }
-    if (gout->dtype == PWS_U8) { set_error("fused backward: a uint8 output is not differentiable"); return PWS_EINVAL; }
-    if (gout->dtype != (half_in ? in->dtype : PWS_F32)) {
-        set_error("fused backward: grad_output must be f32 (f32 or uint8 frames) or the frame's 16-bit type (frame %d, grad_output %d)", in->dtype, gout->dtype);
-        return PWS_EINVAL;
-    }
+    if (gout && gout->dtype == PWS_U8) { set_error("fused backward: a uint8 output is not differentiable"); return PWS_EINVAL; }
+    // grad_output has the forward output's dtype: f32 for f32 and uint8 frames, the frame's type for 16-bit frames
+    PWS_TRY(check_arg(gout, "grad_output", -1, in->size[0], in->size[1], kAny, kAny, half_in ? in->dtype : PWS_F32, in->device,
+                      &vgout));
     if (gtheta && (!spec || spec->base != PWS_BASE_AFFINE)) { set_error("fused backward: gtheta needs the affine base"); return PWS_EINVAL; }
     if (gtheta && !glattice) { set_error("fused backward: gtheta needs glattice (the library never allocates)"); return PWS_EINVAL; }
-    View vin, vgout, vgin{}, vglat{};
-    PWS_TRY(make_view(in, "input", &vin));
-    PWS_TRY(make_view(gout, "grad_output", &vgout));
+    const Geometry g = geometry(in->size, gout->size[2], gout->size[3], padding, align_corners);
     MapSpec m;
-    PWS_TRY(make_spec(spec, in->size[0], gout->size[2], gout->size[3], &m));
+    PWS_TRY(make_spec(spec, g.N, g.Ho, g.Wo, in->device, &m));
     if (gin) {
         if (in->dtype == PWS_U8) { set_error("fused backward: a uint8 frame has no gradient (gin must be NULL)"); return PWS_EINVAL; }
-        PWS_TRY(make_view(gin, "grad_input", &vgin));
-        PWS_TRY(same_shape(gin, in->size[0], in->size[1], in->size[2], in->size[3], "grad_input"));
-        const int64_t C = in->size[1], H = in->size[2], W = in->size[3];
-        // an empty buffer (N = 0 or C = 0) is dense whatever its strides: torch keeps (C*H*W, H*W, W, 1) for C = 0
-        const bool dense = gin->dtype == PWS_F32 && (in->size[0] * C == 0 ||
-                           (gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
-                            (gin->stride[0] == C * H * W || in->size[0] <= 1)));
-        if (!dense) { set_error("grad_input: must be f32 (N,C,H,W)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
-        if (gin->device != in->device) { set_error("fused backward: grad_input must be on the input's device"); return PWS_EINVAL; }
-        vgin.sN = C * H * W;
+        PWS_TRY(check_gin(gin, in, &vgin));
     }
     if (glattice) {
-        PWS_TRY(make_view(glattice, "glattice", &vglat));
-        PWS_TRY(same_shape(glattice, in->size[0], spec->map_h, spec->map_w, 2, "glattice"));
-        const int64_t h = spec->map_h, w = spec->map_w;
-        const bool dense = glattice->dtype == PWS_F32 && glattice->stride[3] == 1 && glattice->stride[2] == 2 &&
-                           glattice->stride[1] == 2 * w && (glattice->stride[0] == 2 * h * w || in->size[0] <= 1);
+        PWS_TRY(check_arg(glattice, "glattice", -1, g.N, m.mh, m.mw, 2, PWS_F32, in->device, &vglat));
+        const bool dense = glattice->stride[3] == 1 && glattice->stride[2] == 2 && glattice->stride[1] == 2 * m.mw &&
+                           (glattice->stride[0] == 2 * m.mh * m.mw || g.N <= 1);
         if (!dense) { set_error("glattice: must be f32 (N,map_h,map_w,2)-contiguous (the library zero-fills it)"); return PWS_EINVAL; }
         // every node's (x, y) is stored, reduced into and read back as one 8-byte pair
         if (reinterpret_cast<uintptr_t>(glattice->data) & 7) { set_error("glattice: must be 8-byte aligned (one float2 per node)"); return PWS_EINVAL; }
-        if (glattice->device != in->device) { set_error("fused backward: glattice must be on the input's device"); return PWS_EINVAL; }
     }
-    Geometry g{};
-    g.N = (int32_t)in->size[0]; g.C = (int32_t)in->size[1]; g.H = (int32_t)in->size[2]; g.W = (int32_t)in->size[3];
-    g.Ho = (int32_t)gout->size[2]; g.Wo = (int32_t)gout->size[3]; g.padding = padding; g.align = align_corners ? 1 : 0;
-    DeviceGuard dg(in->device);
-    if (!dg.ok) { set_error("fused backward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    if (g.N == 0) return PWS_OK;
-    if ((int64_t)g.C * g.Ho * g.Wo == 0) {
-        // nothing flows back; the gradients are still defined (all zeros)
-        cudaStream_t st = (cudaStream_t)stream;
-        cudaError_t e = cudaSuccess;
-        if (gin && (int64_t)g.C * g.H * g.W > 0) e = cudaMemsetAsync(gin->data, 0, (size_t)(g.N * vgin.sN * 4), st);
-        if (e == cudaSuccess && glattice) e = cudaMemsetAsync(glattice->data, 0, (size_t)g.N * m.mh * m.mw * 2 * 4, st);
-        if (e == cudaSuccess && gtheta) e = cudaMemsetAsync(gtheta, 0, (size_t)g.N * 6 * 4, st);
-        if (e != cudaSuccess) { set_error("fused backward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return PWS_ECUDA; }
-        return PWS_OK;
-    }
-    PWS_TRY(launch_backward_fused(vgout, vin, in->dtype, m, vgin, gin != nullptr, glattice ? (float *)glattice->data : nullptr,
-                                  gtheta, g, (cudaStream_t)stream));
-    return finish("fused backward");
+    const cudaStream_t st = (cudaStream_t)stream;
+    if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0) return zero_grads(in->device, "fused backward", st, gin, nullptr, 0, false, glattice, gtheta, g.N);
+    return on_device(in->device, "fused backward", [&] {
+        return launch_backward_fused(vgout, vin, in->dtype, m, vgin, gin != nullptr, glattice ? (float *)glattice->data : nullptr,
+                                     gtheta, g, st);
+    });
 }
 
 __attribute__((visibility("default")))
 int pws_compose_map(const pws_map_spec *spec, int64_t n, pws_tensor *map_out, void *stream)
 {
-    if (!map_out) { set_error("compose_map: null output"); return PWS_EINVAL; }
-    if (map_out->dtype != PWS_F32 || map_out->size[3] != 2 || map_out->size[0] != n) { set_error("compose_map: output must be f32 (N,Ho,Wo,2)"); return PWS_EINVAL; }
+    if (n < 0) { set_error("compose_map: negative n"); return PWS_EINVAL; }
     View vout;
-    PWS_TRY(make_view(map_out, "map_out", &vout));
+    PWS_TRY(check_arg(map_out, "output", -1, n, kAny, kAny, 2, PWS_F32, kAny, &vout));
     MapSpec m;
-    PWS_TRY(make_spec(spec, n, map_out->size[1], map_out->size[2], &m));
-    DeviceGuard dg(map_out->device);
-    if (!dg.ok) { set_error("compose_map: cannot select cuda:%d", map_out->device); return PWS_ECUDA; }
-    PWS_TRY(launch_compose_map(m, vout, (int)n, (int)map_out->size[1], (int)map_out->size[2], (cudaStream_t)stream));
-    return finish("compose_map");
+    PWS_TRY(make_spec(spec, n, map_out->size[1], map_out->size[2], map_out->device, &m));
+    return on_device(map_out->device, "compose_map", [&] {
+        return launch_compose_map(m, vout, (int)n, (int)map_out->size[1], (int)map_out->size[2], (cudaStream_t)stream);
+    });
 }
 
 __attribute__((visibility("default")))
@@ -465,30 +491,17 @@ int pws_warp2d_stages_forward(const pws_tensor *in, const pws_tensor *const *gri
 {
     PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
     if (!in || !grids || !outs) { set_error("stages forward: null argument"); return PWS_EINVAL; }
-    if (n_stages < 1 || n_stages > kMaxStages) { set_error("stages forward: n_stages must be 1..%d", kMaxStages); return PWS_EINVAL; }
-    PWS_TRY(check_stage_dtypes(in, grids, n_stages, "stages forward"));
     View vin;
-    PWS_TRY(make_view(in, "input", &vin));
+    PWS_TRY(make_view(in, "input", -1, &vin));
     StageViews sv{};
-    Geometry g{};
-    for (int k = 0; k < n_stages; ++k) {
-        PWS_TRY(check_pair(in, grids[k]));
-        if (!outs[k]) { set_error("stages forward: null output %d", k); return PWS_EINVAL; }
-        if (outs[k]->dtype != in->dtype) { set_error("stages forward: output %d: dtype must equal the input's", k); return PWS_EINVAL; }
-        if (k && (grids[k]->size[1] != grids[0]->size[1] || grids[k]->size[2] != grids[0]->size[2])) { set_error("stages forward: all maps must have the same size"); return PWS_EINVAL; }
-        PWS_TRY(make_view(grids[k], "grid", &sv.map[k]));
-        PWS_TRY(make_view(outs[k], "output", &sv.io[k]));
-        PWS_TRY(same_shape(outs[k], in->size[0], in->size[1], grids[k]->size[1], grids[k]->size[2], "output"));
-        if (outs[k]->device != in->device) { set_error("stages forward: output must be on the input's device"); return PWS_EINVAL; }
-    }
-    fill_geometry(in, grids[0], padding, align_corners, &g);
+    PWS_TRY(check_stages(in, grids, outs, "output", nullptr, n_stages, "stages forward", &sv));
+    const Geometry g = geometry(in->size, grids[0]->size[1], grids[0]->size[2], padding, align_corners);
     StageScale sc;
     PWS_TRY(make_scale(pre_add, pre_mul, post_div, post_add, &sc));
     if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0) return PWS_OK;
-    DeviceGuard dg(in->device);
-    if (!dg.ok) { set_error("stages forward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    PWS_TRY(launch_stages_forward(vin, in->dtype, sv, grids[0]->dtype, n_stages, g, sc, (cudaStream_t)stream));
-    return finish("stages forward");
+    return on_device(in->device, "stages forward", [&] {
+        return launch_stages_forward(vin, in->dtype, sv, grids[0]->dtype, n_stages, g, sc, (cudaStream_t)stream);
+    });
 }
 
 __attribute__((visibility("default")))
@@ -499,56 +512,20 @@ int pws_warp2d_stages_backward(const pws_tensor *const *gouts, const pws_tensor 
 {
     PWS_TRY(check_modes(PWS_INTERP_BILINEAR, padding));
     if (!in || !grids || !gouts || !ggrids) { set_error("stages backward: null argument"); return PWS_EINVAL; }
-    if (n_stages < 1 || n_stages > kMaxStages) { set_error("stages backward: n_stages must be 1..%d", kMaxStages); return PWS_EINVAL; }
-    PWS_TRY(check_stage_dtypes(in, grids, n_stages, "stages backward"));
     View vin, vgin{};
-    PWS_TRY(make_view(in, "input", &vin));
+    PWS_TRY(make_view(in, "input", -1, &vin));
     StageViews sv{};
-    Geometry g{};
-    for (int k = 0; k < n_stages; ++k) {
-        PWS_TRY(check_pair(in, grids[k]));
-        if (!gouts[k]) { set_error("stages backward: null grad_output %d", k); return PWS_EINVAL; }
-        if (gouts[k]->dtype != in->dtype) { set_error("stages backward: grad_output %d: dtype must equal the input's", k); return PWS_EINVAL; }
-        if (gouts[k]->device != in->device) { set_error("stages backward: grad_output %d: must be on the input's device", k); return PWS_EINVAL; }
-        if (k && (grids[k]->size[1] != grids[0]->size[1] || grids[k]->size[2] != grids[0]->size[2])) { set_error("stages backward: all maps must have the same size"); return PWS_EINVAL; }
-        PWS_TRY(make_view(grids[k], "grid", &sv.map[k]));
-        PWS_TRY(make_view(gouts[k], "grad_output", &sv.io[k]));
-        PWS_TRY(same_shape(gouts[k], in->size[0], in->size[1], grids[k]->size[1], grids[k]->size[2], "grad_output"));
-        if (ggrids[k]) {
-            if (ggrids[k]->dtype != grids[k]->dtype) { set_error("stages backward: grad_grid %d: dtype must equal the map's", k); return PWS_EINVAL; }
-            if (ggrids[k]->device != in->device) { set_error("stages backward: grad_grid %d: must be on the input's device", k); return PWS_EINVAL; }
-            PWS_TRY(make_view(ggrids[k], "grad_grid", &sv.gg[k]));
-            PWS_TRY(same_shape(ggrids[k], grids[k]->size[0], grids[k]->size[1], grids[k]->size[2], 2, "grad_grid"));
-        }
-    }
-    if (gin) {
-        PWS_TRY(make_view(gin, "grad_input", &vgin));
-        PWS_TRY(same_shape(gin, in->size[0], in->size[1], in->size[2], in->size[3], "grad_input"));
-        const int64_t C = in->size[1], H = in->size[2], W = in->size[3];
-        const bool dense = gin->dtype == PWS_F32 && gin->stride[3] == 1 && gin->stride[2] == W && gin->stride[1] == H * W &&
-                           (gin->stride[0] == C * H * W || in->size[0] <= 1);
-        if (!dense) {
-            set_error("grad_input: must be f32 (N,C,H,W)-contiguous (the library zero-fills it; 16-bit frames accumulate in fp32)");
-            return PWS_EINVAL;
-        }
-        if (gin->device != in->device) { set_error("stages backward: grad_input must be on the input's device"); return PWS_EINVAL; }
-        vgin.sN = C * H * W;
-    }
-    fill_geometry(in, grids[0], padding, align_corners, &g);
+    PWS_TRY(check_stages(in, grids, gouts, "grad_output", ggrids, n_stages, "stages backward", &sv));
+    if (gin) PWS_TRY(check_gin(gin, in, &vgin));
+    const Geometry g = geometry(in->size, grids[0]->size[1], grids[0]->size[2], padding, align_corners);
     StageScale sc;
     PWS_TRY(make_scale(pre_add, pre_mul, post_div, post_add, &sc));
-    DeviceGuard dg(in->device);
-    if (!dg.ok) { set_error("stages backward: cannot select cuda:%d", in->device); return PWS_ECUDA; }
-    if (g.N == 0) return PWS_OK;
-    if ((int64_t)g.C * g.Ho * g.Wo == 0) {
-        if (gin && (int64_t)g.C * g.H * g.W > 0) {
-            cudaError_t e = cudaMemsetAsync(gin->data, 0, (size_t)(in->size[0] * vgin.sN * 4), (cudaStream_t)stream);
-            if (e != cudaSuccess) { set_error("stages backward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return PWS_ECUDA; }
-        }
-        return PWS_OK;
-    }
-    PWS_TRY(launch_stages_backward(vin, in->dtype, sv, grids[0]->dtype, n_stages, vgin, gin != nullptr, g, sc, (cudaStream_t)stream));
-    return finish("stages backward");
+    const cudaStream_t st = (cudaStream_t)stream;
+    if ((int64_t)g.N * g.C * g.Ho * g.Wo == 0)
+        return zero_grads(in->device, "stages backward", st, gin, ggrids, n_stages, true, nullptr, nullptr, g.N);
+    return on_device(in->device, "stages backward", [&] {
+        return launch_stages_backward(vin, in->dtype, sv, grids[0]->dtype, n_stages, vgin, gin != nullptr, g, sc, st);
+    });
 }
 
 }  // extern "C"
